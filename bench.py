@@ -16,6 +16,9 @@ Prints ONE JSON line (rank 0).  value = device-timed (CUDA events on the launch 
 all state resident in HBM; e2e = the same metric through the public drop-in API the reference's scripts call --
 ``DistrQLearning.learn(num_episodes, ...)`` (main.py:63) -- wall clock, with the per-env hyper-parameter block copied
 host->device and the per-env counters / episode logs copied device->host inside the timed region.
+
+``--dump-outputs DIR`` writes what the headline workload's environments hold after the last timed step (rank 0) as
+float64 ``DIR/<name>.npy`` files, so that two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -31,6 +34,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True                                            # the benchmark leaves the source tree as it found it
 from __graft_entry__ import load_package  # noqa: E402
 
 METRIC = "switch_agent_decisions_per_sec"
@@ -262,6 +266,69 @@ def kernel_counters(workload):
     return None
 
 
+DUMP_ENVS = 8192                                                          # environments whose counters / episode logs are dumped
+DUMP_Q_ENVS = 16                                                          # environments whose Q tables are dumped
+DUMP_Q_BYTES = 40 << 20                                                   # at most this much of Q rows (with the above: < 64 MB)
+
+
+def _sample(n: int, k: int, salt: int) -> np.ndarray:
+    """All of range(n) when n <= k, else k of them drawn with a fixed seed (the same indices in every run), sorted."""
+    if n <= k:
+        return np.arange(n)
+    return np.sort(np.random.default_rng([SEED, salt]).choice(n, k, replace=False))
+
+
+def dump_outputs(out_dir: str, engs) -> None:
+    """``--dump-outputs``: what a caller of the timed path reads back after its last step, one float64 .npy per array.
+
+    env_index          the environments (concatenated over the maps) the per-env arrays cover
+    counters_<field>   [env] the per-env counters (Engine.counters)
+    ep_<field>         [env, ep_cap] the episode log (Engine.episode_log), ep_logged = episodes logged, ep_delays [env, ep_cap, T]
+    q_env, q_key       [row] environment (shared-table mode: map) and state key of a Q row, rows sorted by (q_env, q_key)
+    q_actions          [row] the number of actions of the row's switch
+    q_val              [row, a_max] its action values, 0 beyond q_actions (every value written is finite)
+    """
+    cnt, logs = np.concatenate([eng.counters() for eng in engs]), [eng.episode_log() for eng in engs]
+    envs = _sample(len(cnt), DUMP_ENVS, 0)
+    out = {"env_index": envs}
+    for k in ("decisions", "ticks", "train_ticks", "episodes", "err", "q_rows", "elapsed", "aborted", "forced_stops", "stop_actions",
+              "arrived_trains"):
+        out["counters_" + k] = cnt[k][envs]
+    out["ep_logged"] = np.concatenate([n for n, _, _ in logs])[envs]
+    ep = np.concatenate([log for _, log, _ in logs])[envs]
+    for k in ("cum_reward", "decisions", "arrived", "num_malfunctions", "ticks"):
+        out["ep_" + k] = ep[k]
+    out["ep_delays"] = np.concatenate([d for _, _, d in logs])[envs]
+
+    a_max = max(eng.sizes.a_max for eng in engs)                          # the maps of C3 differ
+
+    def block(owner, eng, keys, vals):
+        tab, NT = eng.map.tab, len(eng.map.trains.targets)
+        n_act = tab.sw_A[tab.port_switch[keys.astype(np.int64) // (NT * 48)]]
+        vals = np.pad(vals, ((0, 0), (0, a_max - vals.shape[1])))
+        return np.full(len(keys), owner), keys, n_act, np.where(np.arange(a_max) < n_act[:, None], vals, 0.0)
+
+    rows = []
+    if engs[0].shared_q:
+        for k, eng in enumerate(engs):
+            q = eng.shared_q_table()
+            rows.append(block(k, eng, np.arange(q.size // q.shape[-1]), q.reshape(-1, q.shape[-1])))
+    else:
+        Bp = engs[0].n_envs
+        for g in _sample(Bp * len(engs), DUMP_Q_ENVS, 1):
+            eng = engs[g // Bp]
+            keys, vals = eng.q_rows(int(g % Bp))
+            order = np.argsort(keys, kind="stable")
+            rows.append(block(g, eng, keys[order], vals[order]))
+    q_env, q_key, q_actions, q_val = (np.concatenate(x) for x in zip(*rows))
+    keep = _sample(len(q_key), DUMP_Q_BYTES // (8 * (3 + q_val.shape[1])), 2)
+    out.update(q_env=q_env[keep], q_key=q_key[keep], q_actions=q_actions[keep], q_val=q_val[keep])
+
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, np.float64))
+
+
 def run_block(cx: Ctx, wl: str, args, steps: int, warmup: int, sampler=None, flush_l2="auto") -> dict:
     """Device-resident arm of one workload: Engine level, CUDA-event timed, one engine per map."""
     torch = cx.torch
@@ -375,6 +442,8 @@ def run_block(cx: Ctx, wl: str, args, steps: int, warmup: int, sampler=None, flu
         sync_ms = float(np.mean([a.elapsed_time(b) for a, b in sync_ev]))
     kern_ms = step_ms / (1 if streams else parts)                         # mean duration of ONE k_run launch (concurrent maps: of the step)
     t1 = totals()
+    if head and args.dump_outputs and cx.rank == 0:
+        dump_outputs(args.dump_outputs, engs)
     q_rows_max, state_mb = 0, 0.0
     variant = engs[0].describe_launch(backend.MODE_LEARN)
     lanes = engs[0].lanes
@@ -546,7 +615,11 @@ def main():
     ap.add_argument("--e2e-episodes", type=int, default=0, help="episodes per env of the end-to-end learn() call (0 = about as many ticks as the timed steps)")
     ap.add_argument("--cpu-seconds", type=float, default=4.0)
     ap.add_argument("--no-cpu", action="store_true")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write what the headline workload's environments hold after the last timed step to DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs dumps the CUDA path's outputs; the reference arm has none")
     global FIXTURE
     FIXTURE = fixture_path(WORKLOADS[args.workload][0])
     if args.impl == "reference":

@@ -587,10 +587,8 @@ class Engine:
             sem = sem.reshape(self.n_envs, self.cfg.dec_cap, NP, 4)[env][:len(dec)]
         return dec, tick, sem
 
-    def export_q(self, env: int, include_init: bool = False, default_q: Optional[float] = None) -> Dict[tuple, List[float]]:
-        """The reference's q_table dict (distr_q.py:42, pickled by :521-523): obs tuple -> list of A floats."""
-        if self.shared_q:
-            return self.export_shared_q(float(self.hparams["default_q"][env]) if default_q is None else default_q)
+    def q_rows(self, env: int):
+        """The rows of env ``env``'s Q hash table in slot order: (uint32[n] state keys, float64[n, a_max] values)."""
         a_max = self.sizes.a_max
         cap = self.cfg.q_cap
         keys = np.zeros(cap, np.uint32)
@@ -598,12 +596,19 @@ class Engine:
         n = C.c_int()
         self._ck(self.lib.sfl_export_q(self.ctx, env, keys.ctypes.data_as(C.POINTER(C.c_uint32)),
                                        vals.ctypes.data_as(C.POINTER(C.c_double)), cap, C.byref(n), self._stream()))
+        return keys[:n.value], vals[:n.value]
+
+    def export_q(self, env: int, include_init: bool = False, default_q: Optional[float] = None) -> Dict[tuple, List[float]]:
+        """The reference's q_table dict (distr_q.py:42, pickled by :521-523): obs tuple -> list of A floats."""
+        if self.shared_q:
+            return self.export_shared_q(float(self.hparams["default_q"][env]) if default_q is None else default_q)
+        keys, vals = self.q_rows(env)
         out = {}
         if include_init:
             out.update(self.map.q_init_rows(float(self.hparams["default_q"][env]) if default_q is None else default_q))
         t = self.map.tab
         NT = len(self.map.trains.targets)
-        for k, v in zip(keys[:n.value], vals[:n.value]):
+        for k, v in zip(keys, vals):
             A = int(t.sw_A[t.port_switch[int(k) // (NT * 48)]])
             out[self.map.key_to_obs(int(k))] = [float(x) for x in v[:A]]
         return out

@@ -15,18 +15,12 @@ def pytest_configure(config):
 
 
 def pytest_collection_modifyitems(config, items):
-    """A plain ``pytest tests`` on a box without a GPU (or without the built library) skips the gpu-marked tests
-    instead of failing them; ``-m gpu`` on the B200 box runs them."""
+    """A plain ``pytest tests`` on a machine without a GPU skips the gpu-marked tests instead of failing them; with a
+    GPU they run, and fail if ``__graft_entry__.build()`` has not built the library."""
     import pytest
     import torch
-    from switchfl_b200 import backend
-    reason = None
     if not torch.cuda.is_available():
-        reason = "needs a CUDA device"
-    elif not os.path.exists(backend.LIB_PATH):
-        reason = "libswitchfl_b200.so is not built"
-    if reason:
-        skip = pytest.mark.skip(reason=reason)
+        skip = pytest.mark.skip(reason="needs a CUDA device")
         for item in items:
             if "gpu" in item.keywords:
                 item.add_marker(skip)

@@ -414,3 +414,31 @@ def test_learn_concurrently_equals_learning_in_turn():
     for x, y in zip(a, b):
         assert np.array_equal(x.metrics["cum_reward"], y.metrics["cum_reward"]) and np.array_equal(x.metrics["delays"], y.metrics["delays"])
         assert x.q_table == y.q_table and len(x.q_table) > 0
+
+
+def test_bench_dump_outputs_are_reproducible_float64_and_what_the_engine_holds():
+    """bench.py --dump-outputs (host build of the kernels): two runs on the same inputs write the same float64 files, and they
+    hold the engine's counters and Q tables."""
+    import bench
+    rm = backend.RailMap(load_golden("c1_synth18")[0])
+    dumps = []
+    for _ in range(2):
+        eng = EmulEngine(rm, n_envs=8, q_cap=1024, ep_cap=4)
+        eng.set_hparams(**bench.HP, seeds=np.arange(8) + bench.SEED, episodes=-1)
+        eng.reset()
+        eng.enable_q_init(True)
+        for _ in range(2):
+            eng.run(backend.MODE_LEARN, 512)
+        with tempfile.TemporaryDirectory() as tmp:
+            bench.dump_outputs(tmp, [eng])
+            dumps.append({f[:-len(".npy")]: np.load(os.path.join(tmp, f)) for f in os.listdir(tmp)})
+    a, b = dumps
+    assert a.keys() == b.keys()
+    for k, v in a.items():
+        assert v.dtype == np.float64 and np.isfinite(v).all() and np.array_equal(v, b[k]), k
+    assert np.array_equal(a["counters_decisions"], eng.counters()["decisions"]) and a["counters_decisions"].min() > 0
+    for env in range(8):
+        mine = a["q_env"] == env
+        q = {rm.key_to_obs(int(k)): [float(x) for x in v[:int(n)]]
+             for k, n, v in zip(a["q_key"][mine], a["q_actions"][mine], a["q_val"][mine])}
+        assert q == eng.export_q(env) and len(q) > 0
