@@ -24,7 +24,7 @@
 extern "C" {
 #endif
 
-#define SFL_ABI_VERSION 6
+#define SFL_ABI_VERSION 7
 
 enum {
   SFL_OK = 0,
@@ -149,7 +149,8 @@ typedef struct sfl_dec_rec {           /* one switch-agent decision (trace)     
   int32_t ep, tick, sw, train;
   uint32_t key;                        /* dense state index (see DESIGN.md)                           */
   int32_t mask, action, next_sw, reward, done;
-  uint64_t arrived;
+  uint64_t arrived;                    /* trains 0..63 at their destination after the decision, bit t = train t       */
+  uint64_t arrived_hi;                 /* trains 64..127 (bit t - 64); 0 when T <= 64                                 */
 } sfl_dec_rec;
 
 /* SFL_MODE_STEP output per environment: what AECEnv.last() returns for the waiting decision (observer.py:246-308)
@@ -162,14 +163,16 @@ typedef struct sfl_step_rec {
   int32_t done;                        /* terminated | truncated << 1                                                 */
   int32_t elapsed;                     /* rail_env._elapsed_steps                                                     */
   int32_t last_next_sw;                /* "next_switch" of the decision just applied, -1 if none                      */
-  uint64_t arrived;                    /* "arrived_trains" as a bit set                                               */
-  int32_t rewards[64];                 /* _cumulative_rewards[sw][train] for every train (switch_env.py:130, 289)     */
+  uint64_t arrived;                    /* "arrived_trains" as a bit set: trains 0..63                                 */
+  int32_t rewards[128];                /* _cumulative_rewards[sw][train] for every train (switch_env.py:130, 289)     */
+  uint64_t arrived_hi;                 /* trains 64..127 of "arrived_trains" (bit t - 64); 0 when T <= 64             */
 } sfl_step_rec;
 
 typedef struct sfl_tick_rec { int32_t pos; int8_t dir, state; int16_t malf; } sfl_tick_rec;
 typedef struct sfl_ep_rec {            /* one finished episode (distr_q.py:360-366)                   */
   double cum_reward; int32_t decisions, arrived, num_malfunctions, ticks;
-  uint64_t arrived_mask;               /* the trains at their destination ("arrived_trains", :345, 371) */
+  uint64_t arrived_mask;               /* the trains at their destination ("arrived_trains", :345, 371): trains 0..63 */
+  uint64_t arrived_mask_hi;            /* trains 64..127 (bit t - 64); 0 when T <= 64                 */
 } sfl_ep_rec;
 
 /* Distance map (flatland DistanceMap as vendored in flatland_patch/distance_map.py:62-167; SURVEY.md row F6 / N1):
@@ -191,7 +194,8 @@ const char *sfl_last_error(void);
  * memory (env: switch_env.py:42-73, learner: distr_q.py:33-57); here PyTorch does, and the library is told how much.  */
 int sfl_query_sizes(const sfl_map_desc *map, const sfl_config *cfg, sfl_sizes *out);
 
-/* replaces ASyncSwitchEnv(rail_env, ...) + DistrQLearning(env, ...)   (main.py:51-60) */
+/* replaces ASyncSwitchEnv(rail_env, ...) + DistrQLearning(env, ...)   (main.py:51-60).  T must be in 1..128;
+ * shared-table mode (sfl_config.shared_q) takes at most 64 trains.                                               */
 int sfl_create(const sfl_map_desc *map, const sfl_config *cfg, int device, void **ctx);
 int sfl_destroy(void *ctx);                       /* env.close() (switch_env.py, called at distr_q.py:241, 379) + garbage collection */
 int sfl_bind(void *ctx, const sfl_buffers *bufs); /* hand over the caller-owned device buffers sized by sfl_query_sizes            */
@@ -202,7 +206,8 @@ int sfl_reset(void *ctx, int keep_q, void *stream);
 
 /* Lanes of a warp that cooperate on one environment (1, 2, 4, 8, 16 or 32; 32/lanes environments share a warp and
  * one instruction stream).  sfl_create picks max(lanes that cover the trains in one pass, lanes that still give the
- * batch ~3.5 warps per SM scheduler); this overrides it.  A scheduling choice only: results do not depend on it.  */
+ * batch ~3.5 warps per SM scheduler); this overrides it.  A scheduling choice only: results do not depend on it.
+ * Maps with more than 64 trains run on 8, 16 or 32 lanes.                                              */
 int sfl_set_lanes(void *ctx, int lanes);
 int sfl_get_lanes(void *ctx);
 /* Warps per CTA of the hot-path kernel: 0 = automatic (4, halved while the launch has fewer than 8 CTAs per SM), or 1, 2,
@@ -217,7 +222,8 @@ int sfl_set_roomy(void *ctx, int roomy);
  * off by default: the production kernels carry no clock reads.                                                       */
 int sfl_set_phase_clock(void *ctx, int on);
 /* Which kernel instantiation and launch configuration sfl_run(mode) would use now (traced != 0: with decision / tick
- * traces), as text: "k_run<G=..,KIND=..,TH=..,SQ=..,ONE=..,ROOMY=..> grid=.. block=.. smem=..".  No counterpart in the
+ * traces), as text: "k_run<G=..,KIND=..,TH=..,SQ=..,ONE=..,ROOMY=..> grid=.. block=.. smem=..", with ",NW=2" after ROOMY
+ * on maps with more than 64 trains (two words per train set).  No counterpart in the
  * reference; it lets the parity tests name -- and force, with sfl_set_lanes / sfl_set_roomy -- exactly the
  * instantiations the benchmark launches.  Needs no bound buffers.                                                  */
 int sfl_describe_launch(void *ctx, int mode, int traced, char *buf, int cap);

@@ -21,7 +21,7 @@ from typing import Dict, List, Optional, Sequence
 
 import numpy as np
 
-from .backend import MODE_GREEDY, MODE_LEARN, Engine, RailMap
+from .backend import MODE_GREEDY, MODE_LEARN, Engine, RailMap, train_set
 
 
 class Discrete:
@@ -212,7 +212,7 @@ class ASyncSwitchEnv:
         for r in self._rec:
             nxt = int(r["last_next_sw"])
             out.append({"next_switch": tuple(int(x) for x in cells[nxt]) if nxt >= 0 else None,
-                        "arrived_trains": [h for h in range(self.rail_map.trains.T) if (int(r["arrived"]) >> h) & 1]})
+                        "arrived_trains": train_set(r["arrived"], r["arrived_hi"], self.rail_map.trains.T)})
         return out
 
     def close(self):
@@ -369,7 +369,7 @@ class DistrQLearning:
                 cum_reward[:, done:done + seg] = log["cum_reward"][:, :seg]
                 arrived[:, done:done + seg] = log["arrived"][:, :seg]
                 num_malf[:, done:done + seg] = log["num_malfunctions"][:, :seg]
-                last_mask = log["arrived_mask"][:, seg - 1].copy()
+                last_mask = log[["arrived_mask", "arrived_mask_hi"]][:, seg - 1].copy()
                 delays[:, done:done + seg] = dl[:, :seg]
                 done += seg
             if cut >= num_episodes:
@@ -388,7 +388,7 @@ class DistrQLearning:
                 np.savez_compressed(os.path.join(out_dir, f"num_malfunctions_checkpoint_{cut + 1}.npz"), x=num_malf[p, :cut])
         self._table_dirty = True
         self._q_stale = True                 # q_table is read back from the device when it is next used
-        at_dest = [[h for h in range(T) if (int(mk) >> h) & 1] for mk in last_mask] if num_episodes else [[] for _ in range(B)]
+        at_dest = [train_set(mk["arrived_mask"], mk["arrived_mask_hi"], T) for mk in last_mask] if num_episodes else [[] for _ in range(B)]
         self.metrics = dict(cum_reward=cum_reward, arrived_trains=arrived, delays=delays, num_malfunctions=num_malf, trains_at_dest=at_dest,
                             cum_reward_exploit=np.array(cum_reward_exploit), arrived_trains_exploit=np.array(arrived_exploit),
                             wall_s=time.time() - t_start)

@@ -18,7 +18,7 @@ from . import railmap
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "csrc", "libswitchfl_b200.so")
 
-ABI_VERSION = 6
+ABI_VERSION = 7
 MODE_LEARN, MODE_GREEDY, MODE_REPLAY, MODE_STEP = 0, 1, 2, 3
 ERR_NO_TRAIN_AT_SWITCH = 1
 ERR_BITS = {1: "no train at active switch (observer.py:294-307)", 2: "infinite distance to target (observer.py:35-36)",
@@ -66,12 +66,21 @@ COUNTERS_DT = np.dtype([("decisions", "u8"), ("ticks", "u8"), ("train_ticks", "u
                         ("forced_stops", "u8"), ("stop_actions", "u8"), ("arrived_trains", "u8"), ("reserved2", "u8"),
                         ("phase_cycles", "u8", (6,))])
 DEC_DT = np.dtype([("ep", "i4"), ("tick", "i4"), ("sw", "i4"), ("train", "i4"), ("key", "u4"), ("mask", "i4"), ("action", "i4"),
-                   ("next_sw", "i4"), ("reward", "i4"), ("done", "i4"), ("arrived", "u8")])
+                   ("next_sw", "i4"), ("reward", "i4"), ("done", "i4"), ("arrived", "u8"), ("arrived_hi", "u8")])
 TICK_DT = np.dtype([("pos", "i4"), ("dir", "i1"), ("state", "i1"), ("malf", "i2")])
 STEP_DT = np.dtype([("pending", "i4"), ("sw", "i4"), ("train", "i4"), ("key", "u4"), ("mask", "i4"), ("done", "i4"), ("elapsed", "i4"),
-                    ("last_next_sw", "i4"), ("arrived", "u8"), ("rewards", "i4", (64,))])
-EP_DT = np.dtype([("cum_reward", "f8"), ("decisions", "i4"), ("arrived", "i4"), ("num_malfunctions", "i4"), ("ticks", "i4"), ("arrived_mask", "u8")])
-assert HPARAMS_DT.itemsize == 80 and COUNTERS_DT.itemsize == 144 and DEC_DT.itemsize == 48 and TICK_DT.itemsize == 8 and EP_DT.itemsize == 32
+                    ("last_next_sw", "i4"), ("arrived", "u8"), ("rewards", "i4", (128,)), ("arrived_hi", "u8")])
+EP_DT = np.dtype([("cum_reward", "f8"), ("decisions", "i4"), ("arrived", "i4"), ("num_malfunctions", "i4"), ("ticks", "i4"), ("arrived_mask", "u8"),
+                  ("arrived_mask_hi", "u8")])
+assert HPARAMS_DT.itemsize == 80 and COUNTERS_DT.itemsize == 144 and DEC_DT.itemsize == 56 and TICK_DT.itemsize == 8 and EP_DT.itemsize == 40
+assert STEP_DT.itemsize == 560
+
+
+def train_set(lo, hi, T: int) -> List[int]:
+    """The trains of a record's two-word train set (``arrived`` / ``arrived_hi``, ``arrived_mask`` / ``arrived_mask_hi``):
+    bit t of ``lo`` is train t, bit t of ``hi`` is train 64 + t; ascending train handles."""
+    lo, hi = int(lo), int(hi)
+    return [h for h in range(T) if ((lo >> h) if h < 64 else (hi >> (h - 64))) & 1]
 
 
 def load_library(path: Optional[str] = None) -> C.CDLL:

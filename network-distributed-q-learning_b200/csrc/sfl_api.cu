@@ -66,6 +66,9 @@ struct DeviceGuard {
 #ifndef SFL_WARPS_PER_CTA
 #define SFL_WARPS_PER_CTA 4
 #endif
+#ifndef SFL_MINB_WIDE
+#define SFL_MINB_WIDE 6                                // CTAs per SM the learn / greedy kernels for more than 64 trains (NW = 2) are
+#endif                                                 // compiled for: 80 registers; at 7 (72) they spill
 #define SFL_CTA_THREADS (32 * SFL_WARPS_PER_CTA)
 #define SFL_SMEM_BUDGET (56u * 1024u)                  // per CTA, so that four CTAs share an SM
 
@@ -104,6 +107,7 @@ SFL_FN void env_init(const InitArgs &ia, int env_id, int lane, int lanes) {
     memset(&z, 0, sizeof(z));
     z.need_reset = 1; z.pending_fin = -1; z.cur_dec = -1; z.q_rows = q_rows; z.cur_train = -1; z.last_next_sw = -1; z.eps_tag = -1;
     *e.h() = z;
+    if (ia.L.T > 64) for (int m = 0; m < 4; m++) ((unsigned long long *)(e.b + sizeof(EnvHdr)))[m] = 0ull;   // word 1 of the train sets
   }
 }
 
@@ -145,11 +149,14 @@ __global__ void __launch_bounds__(SFL_CTA_THREADS) k_init(const __grid_constant_
 // back at the end, so the tick / decision loops touch HBM only for Q rows.
 // ROOMY: compiled for 4 instead of 7 CTAs per SM (about 100 instead of 72 registers, no spills) -- for launches of the
 // large-map kernels that do not fill the SMs anyway (C3: 1024 one-environment warps per map, +10 %).
-template <int G, int KIND, bool TH, bool SQ, bool ONE, bool ROOMY = false>
-__global__ void __launch_bounds__(SFL_CTA_THREADS, TH ? (G == 32 ? 7 : 4) : (ROOMY ? 4 : SFL_MINB_BIG)) k_run(const __grid_constant__ KArgs K) {
+// NW: 64-bit words per train set, 2 for maps with more than 64 trains (tail in HBM, 8 / 16 / 32 lanes, no ONE / ROOMY / SQ);
+// the wide full kernel (traces, replay, step protocol, phase clock) is compiled for 5 CTAs per SM: no spills.
+template <int G, int KIND, bool TH, bool SQ, bool ONE, bool ROOMY = false, int NW = 1>
+__global__ void __launch_bounds__(SFL_CTA_THREADS, NW > 1 ? (KIND == K_FULL ? 5 : SFL_MINB_WIDE) : TH ? (G == 32 ? 7 : 4) : (ROOMY ? 4 : SFL_MINB_BIG))
+k_run(const __grid_constant__ KArgs K) {
   const int slot = threadIdx.x / G;                    // environment slot inside the CTA
   const int env_id = blockIdx.x * (blockDim.x / G) + slot;
-  env_run<G, KIND, TH, SQ, ONE>(K, env_id, (unsigned)slot * K.ra.env_smem, nullptr);
+  env_run<G, KIND, TH, SQ, ONE, NW>(K, env_id, (unsigned)slot * K.ra.env_smem, nullptr);
 }
 
 __global__ void k_sum(const sfl_env_counters *c, int n, unsigned long long *out) {
@@ -229,7 +236,13 @@ template <int G> static run_kernel_t pick_kernel_g(int kind, int th, int sq, int
   return th ? (one ? k_run<G, K_LEARN, true, false, true> : k_run<G, K_LEARN, true, false, false>)
             : (one ? k_run<G, K_LEARN, false, false, true> : k_run<G, K_LEARN, false, false, false>);
 }
-static run_kernel_t pick_kernel(int G, int kind, int th, int sq, int one, int roomy) {
+// more than 64 trains: the tail stays in HBM (choose_hot) and the groups are 8, 16 or 32 lanes wide (sfl_set_lanes)
+template <int G> static run_kernel_t pick_wide_g(int kind) {
+  return kind == K_FULL ? k_run<G, K_FULL, false, false, false, false, 2>
+       : kind == K_GREEDY ? k_run<G, K_GREEDY, false, false, false, false, 2> : k_run<G, K_LEARN, false, false, false, false, 2>;
+}
+static run_kernel_t pick_kernel(int G, int kind, int th, int sq, int one, int roomy, int nw) {
+  if (nw > 1) return G == 8 ? pick_wide_g<8>(kind) : G == 16 ? pick_wide_g<16>(kind) : pick_wide_g<32>(kind);
   switch (G) {
     case 1: return pick_kernel_g<1>(kind, th, sq, one, roomy);
     case 2: return pick_kernel_g<2>(kind, th, sq, one, roomy);
@@ -257,7 +270,7 @@ struct Ctx {
 // ------------------------------------------------------------------------------------------------ launch plan
 // Which k_run instantiation a launch of `kind` uses and its launch configuration -- shared by sfl_run and
 // sfl_describe_launch, so that tests can pin exactly the instantiations the benchmark times.
-struct LaunchPlan { int G, th, one, roomy, threads, grid; size_t smem; };
+struct LaunchPlan { int G, th, one, roomy, nw, threads, grid; size_t smem; };
 static int plan_launch(const Ctx *c, int kind, LaunchPlan *lp) {
   const int G = c->lanes;
   // Warps per CTA: the kernels are compiled for at most SFL_WARPS_PER_CTA; small launches use smaller CTAs so that the
@@ -275,8 +288,9 @@ static int plan_launch(const Ctx *c, int kind, LaunchPlan *lp) {
   if (lp->smem > 227u * 1024u) return fail(SFL_E_ARG, "environment state does not fit shared memory with this many lanes per env: use more lanes%s");
   lp->G = G; lp->threads = threads; lp->grid = (c->cfg.n_envs + envs_per_cta - 1) / envs_per_cta;
   lp->th = (int)c->tail_hot; lp->one = c->L.T <= G && !c->cfg.shared_q && kind != K_FULL;
+  lp->nw = c->L.T > 64 ? 2 : 1;
   int roomy = c->roomy >= 0 ? c->roomy : (warps <= 16L * c->sm_count);                   // one wave even at 4 CTAs per SM
-  lp->roomy = roomy && !lp->th && !c->cfg.shared_q && kind == K_LEARN && G >= 16;        // the only roomy instantiations
+  lp->roomy = roomy && !lp->th && !c->cfg.shared_q && kind == K_LEARN && G >= 16 && lp->nw == 1;   // the only roomy instantiations
   return 0;
 }
 
@@ -284,10 +298,12 @@ static int plan_launch(const Ctx *c, int kind, LaunchPlan *lp) {
 // Shared-memory staging plan for c->lanes lanes per environment: the whole non-Q state (header, train records, pending
 // lists, semaphores, rewards, per-switch counters) when that still leaves room for 16 warps per SM,
 // else only header + train records + pending lists (semaphores, rewards and counters then stay in HBM / L2).
+// More than 64 trains: always the latter -- the whole state fits only for the smallest maps, and the wide kernels are
+// built for the tail in HBM only.
 static int choose_hot(Ctx *c) {
   const unsigned fixed = (unsigned)sizeof(sfl_hparams) + scratch_bytes(c->L.T);
   const unsigned per_warp = 32u / (unsigned)c->lanes;
-  if ((size_t)(c->L.off_q + fixed) * per_warp <= 14u * 1024u) { c->tail_hot = 1; c->hot_bytes = c->L.off_q; }   // >= 16 warps per SM
+  if (c->L.T <= 64 && (size_t)(c->L.off_q + fixed) * per_warp <= 14u * 1024u) { c->tail_hot = 1; c->hot_bytes = c->L.off_q; }   // >= 16 warps per SM
   else { c->tail_hot = 0; c->hot_bytes = c->L.off_pend; }
   c->env_smem = c->hot_bytes + fixed + (c->tail_hot ? 0u : ((unsigned)c->L.NP + 15u) / 16u * 16u);   // + holder bytes of the semaphores
   return (size_t)c->env_smem * per_warp > 227u * 1024u;
@@ -297,7 +313,7 @@ static unsigned align_up(unsigned v, unsigned a) { return (v + a - 1) / a * a; }
 
 static int make_layout(const sfl_map_desc *map, const sfl_config *cfg, Layout *L, int *a_max_out) {
   if (!map || !cfg) return fail(SFL_E_ARG, "null argument%s");
-  if (map->T < 1 || map->T > SFL_MAX_T) return fail(SFL_E_ARG, "T must be in 1..64%s");
+  if (map->T < 1 || map->T > SFL_MAX_T) return fail(SFL_E_ARG, "T must be in 1..128%s");
   if (map->S < 1 || map->S > 4095) return fail(SFL_E_ARG, "S must be in 1..4095%s");
   if (map->NP > 32767) return fail(SFL_E_ARG, "too many ports%s");
   if ((int64_t)(map->H + 2) * (map->W + 2) >= (1 << 28)) return fail(SFL_E_ARG, "grid too large%s");
@@ -310,8 +326,8 @@ static int make_layout(const sfl_map_desc *map, const sfl_config *cfg, Layout *L
   memset(L, 0, sizeof(*L));
   L->T = map->T; L->S = map->S; L->NP = map->NP; L->NT = map->NT; L->a_max = a_max; L->q_cap = cfg->q_cap;
   L->q_stride = 1 + a_max; L->pend_cap = cfg->pend_cap;
-  unsigned o = align_up((unsigned)sizeof(EnvHdr), 16);
   unsigned T = (unsigned)map->T;
+  unsigned o = align_up((unsigned)sizeof(EnvHdr) + (T > 64 ? 4u * 8u : 0u), 16);     // + word 1 of the four train sets
 #define PUT(field, bytes) L->field = o; o = align_up(o + (unsigned)(bytes), 16)
   PUT(off_tra, 16 * T); PUT(off_trb, 16 * T); PUT(off_pend, 8 * T * cfg->pend_cap);
   PUT(off_sem, 16 * (unsigned)map->NP); PUT(off_rewards, 4 * (unsigned)map->S * T); PUT(off_sws, 16 * (unsigned)map->S);
@@ -455,6 +471,7 @@ int sfl_create(const sfl_map_desc *map, const sfl_config *cfg, int device, void 
   Layout L; int a_max;
   int rc = make_layout(map, cfg, &L, &a_max);
   if (rc) return rc;
+  if (cfg->shared_q && map->T > 64) return fail(SFL_E_ARG, "shared-table mode supports at most 64 trains%s");
   const int H = map->H, W = map->W, Hp = H + 2, Wp = W + 2, T = map->T, NT = map->NT, S = map->S, NP = map->NP, NA = map->NA;
   // every transition must lead to a rail cell inside the grid (flatland maps are consistent); the device relies on it
   for (int r = 0; r < H; r++) for (int cc = 0; cc < W; cc++) {
@@ -579,6 +596,7 @@ int sfl_set_lanes(void *ctx, int lanes) {
   Ctx *c = (Ctx *)ctx;
   if (!c) return fail(SFL_E_ARG, "null ctx%s");
   if (lanes != 1 && lanes != 2 && lanes != 4 && lanes != 8 && lanes != 16 && lanes != 32) return fail(SFL_E_ARG, "lanes must be 1, 2, 4, 8, 16 or 32%s");
+  if (c->L.T > 64 && lanes < 8) return fail(SFL_E_ARG, "maps with more than 64 trains run on 8, 16 or 32 lanes%s");
   int old = c->lanes;
   c->lanes = lanes;
   if (choose_hot(c)) { c->lanes = old; choose_hot(c); return fail(SFL_E_ARG, "one warp of environments does not fit shared memory with this few lanes per env%s"); }
@@ -617,8 +635,8 @@ int sfl_describe_launch(void *ctx, int mode, int traced, char *buf, int cap) {
   LaunchPlan lp;
   if (plan_launch(c, kind, &lp)) return SFL_E_ARG;
   static const char *kinds[] = {"learn", "greedy", "full"};
-  snprintf(buf, (size_t)cap, "k_run<G=%d,KIND=%s,TH=%d,SQ=%d,ONE=%d,ROOMY=%d> grid=%d block=%d smem=%zu", lp.G, kinds[kind], lp.th,
-           c->cfg.shared_q ? 1 : 0, lp.one, lp.roomy, lp.grid, lp.threads, lp.smem);
+  snprintf(buf, (size_t)cap, "k_run<G=%d,KIND=%s,TH=%d,SQ=%d,ONE=%d,ROOMY=%d%s> grid=%d block=%d smem=%zu", lp.G, kinds[kind], lp.th,
+           c->cfg.shared_q ? 1 : 0, lp.one, lp.roomy, lp.nw > 1 ? ",NW=2" : "", lp.grid, lp.threads, lp.smem);
   return SFL_OK;
 }
 
@@ -708,7 +726,7 @@ int sfl_run(void *ctx, int mode, int max_ticks, void *stream) {
   if (c->cfg.shared_q && trace) return fail(SFL_E_ARG, "shared-table mode has no trace / step variants%s");
   const int grid = lp.grid, threads = lp.threads;
   const size_t smem = lp.smem;
-  run_kernel_t k = pick_kernel(lp.G, kind, lp.th, c->cfg.shared_q, lp.one, lp.roomy);
+  run_kernel_t k = pick_kernel(lp.G, kind, lp.th, c->cfg.shared_q, lp.one, lp.roomy, lp.nw);
   CU(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   k<<<grid, threads, smem, (cudaStream_t)stream>>>(K);
   CU(cudaGetLastError());
@@ -718,6 +736,10 @@ int sfl_run(void *ctx, int mode, int max_ticks, void *stream) {
     if (c->cfg.shared_q) {
       if (trace) return fail(SFL_E_ARG, "shared-table mode has no trace / step variants%s");
       if (kind == K_GREEDY) env_run<1, K_GREEDY, true, true, false>(K, i, 0u, host_scratch); else env_run<1, K_LEARN, true, true, false>(K, i, 0u, host_scratch);
+    } else if (c->L.T > 64) {
+      if (kind == K_FULL) env_run<1, K_FULL, true, false, false, 2>(K, i, 0u, host_scratch);
+      else if (kind == K_GREEDY) env_run<1, K_GREEDY, true, false, false, 2>(K, i, 0u, host_scratch);
+      else env_run<1, K_LEARN, true, false, false, 2>(K, i, 0u, host_scratch);
     } else if (kind == K_FULL) env_run<1, K_FULL, true, false, false>(K, i, 0u, host_scratch);
     else if (kind == K_GREEDY) env_run<1, K_GREEDY, true, false, false>(K, i, 0u, host_scratch);
     else env_run<1, K_LEARN, true, false, false>(K, i, 0u, host_scratch);

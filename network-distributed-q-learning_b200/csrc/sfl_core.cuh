@@ -50,7 +50,7 @@ enum { A_NOTHING = 0, A_LEFT = 1, A_FWD = 2, A_RIGHT = 3, A_STOP = 4, A_NONE = 0
 enum { ST_WAITING = 0, ST_READY = 1, ST_MALF_OFF = 2, ST_MOVING = 3, ST_STOPPED = 4, ST_MALF = 5, ST_DONE = 6 };
 enum { SEM_IN = 0, SEM_OUT = 1 };
 #define SFL_INF_DIST 0x3FFFFFFF
-#define SFL_MAX_T 64
+#define SFL_MAX_T 128
 #define SFL_PLAN_CAP 4
 
 // ------------------------------------------------------------------------------------------------ lane groups
@@ -102,6 +102,41 @@ SFL_FN double dadd(double a, double b) { volatile double r = a + b; return r; }
 template <class T> SFL_FN T ldg(const T *p) { return *p; }
 #endif
 
+// ------------------------------------------------------------------------------------------------ train sets
+// A set of trains in NW 64-bit words, train t = bit (t & 63) of word (t >> 6): NW = 1 up to 64 trains, NW = 2 up to 128
+// (SFL_MAX_T: the semaphore-holder mirror and the occupancy scratch hold train indices in one byte).  The words are
+// named, never indexed by a runtime value, so that they stay in registers.  With NW = 1 every operation is the plain
+// one-word expression.
+template <int NW> struct TSet {
+  static_assert(NW == 1 || NW == 2, "one or two words of trains");
+  unsigned long long w[NW];
+  SFL_FN void clear() { w[0] = 0ull; if (NW > 1) w[NW - 1] = 0ull; }
+  // or in a group ballot whose bit 0 is train `base` (G divides 64: the chunk lies inside one word)
+  SFL_FN void or_ballot(unsigned b, int base) {
+    if (NW == 1) { w[0] |= (unsigned long long)b << base; return; }
+    const unsigned long long v = (unsigned long long)b << (base & 63);
+    if (base < 64) w[0] |= v; else w[NW - 1] |= v;
+  }
+  SFL_FN unsigned long long test(int t) const {
+    if (NW == 1) return (w[0] >> t) & 1ull;
+    return ((t < 64 ? w[0] : w[NW - 1]) >> (t & 63)) & 1ull;
+  }
+  SFL_FN int any() const { return NW == 1 ? w[0] != 0ull : (w[0] | w[NW - 1]) != 0ull; }
+  SFL_FN int popc() const { return NW == 1 ? popc64(w[0]) : popc64(w[0]) + popc64(w[NW - 1]); }
+  // lowest train of the set, removed from it: word 0 first (train-handle order)
+  SFL_FN int pop() {
+    if (NW == 1 || w[0]) { const int t = ffs64(w[0]); w[0] &= w[0] - 1; return t; }
+    const int t = 64 + ffs64(w[NW - 1]); w[NW - 1] &= w[NW - 1] - 1; return t;
+  }
+  // the set is all of trains 0..T-1
+  SFL_FN int all(int T) const {
+    if (NW == 1) return w[0] == (T >= 64 ? ~0ull : ((1ull << T) - 1ull));
+    return w[0] == ~0ull && w[NW - 1] == (T >= 128 ? ~0ull : ((1ull << (T - 64)) - 1ull));
+  }
+  SFL_FN TSet andnot(const TSet &o) const { TSet r; r.w[0] = w[0] & ~o.w[0]; if (NW > 1) r.w[NW - 1] = w[NW - 1] & ~o.w[NW - 1]; return r; }
+  SFL_FN int operator==(const TSet &o) const { return NW == 1 ? w[0] == o.w[0] : (w[0] == o.w[0]) & (w[NW - 1] == o.w[NW - 1]); }
+};
+
 // ------------------------------------------------------------------------------------------------ device views
 // read-only map table: loads go through the non-coherent path (LDG.CONSTANT, L1-resident across the launch)
 template <class T> struct RO {
@@ -130,7 +165,9 @@ struct Layout {            // byte offsets inside one env block
   unsigned long long env_stride;
 };
 
-struct EnvHdr {            // 128 bytes at the start of every env block
+// The header at the start of every env block.  It holds word 0 of the four train sets; with NW = 2 (T > 64) word 1 of
+// each follows the header (Layout: zero bytes when T <= 64), in the order of the HM_* indices below.
+struct EnvHdr {
   int elapsed, episode, step_counter, num_malf;
   int terminated, truncated, need_reset, halted;
   int err, q_rows, pending_fin, cur_dec;
@@ -156,6 +193,7 @@ struct EnvHdr {            // 128 bytes at the start of every env block
 // and LENGTH of the window, so that extend_semaphores (rail_network.py:229-244: slide the window to start now, keep its
 // length) is one 4-byte store per record and needs no load.
 struct SwS { int ninter, pad; double eps_pow; };
+enum { HM_ACTIVE = 0, HM_MALF = 1, HM_DEST = 2, HM_DONE = 3 };   // the header's train sets: active, malf_prev, at_dest, done
 
 struct RunArgs {           // per-launch arguments
   int mode, max_ticks, n_envs, trace_sem;
@@ -195,6 +233,7 @@ SFL_FN char *hot_ptr(hot_t o) { return o; }
 template <bool TH, bool SQ_ = false> struct EnvT {
   static const bool SQ = SQ_;
   static const bool HOT_TAIL = TH;
+  static const int NW = 1;                 // 64-bit words per train set (EnvW: 2)
   const KArgs *kp;         // the launch's parameter block (methods below read the layout through it)
   hot_t hot;               // staged copy of the first hot_bytes of the env block (the env block itself on the host build)
   char *gb;                // the env block in HBM
@@ -215,7 +254,30 @@ template <bool TH, bool SQ_ = false> struct EnvT {
   SFL_FN int owner(int p) const { return TH ? sem()[p].z : (int)(int8_t)own_ptr()[p]; }
   SFL_FN void sem_put(int p, int4 r) const { sem()[p] = r; if (!TH) own_ptr()[p] = (uint8_t)r.z; }
   SFL_FN void sem_drop(int p) const { sem()[p].z = -1; if (!TH) own_ptr()[p] = 0xFFu; }
+  // header train set m (HM_*): word 0 in EnvHdr, word 1 (EnvW) right after it
+  SFL_FN unsigned long long &hw0(int m) const {
+    EnvHdr *x = h();
+    return m == HM_ACTIVE ? x->active_mask : m == HM_MALF ? x->malf_prev_mask : m == HM_DEST ? x->at_dest_mask : x->done_mask;
+  }
+  SFL_FN unsigned long long *hw1(int m) const { return (unsigned long long *)(hot_ptr(hot) + sizeof(EnvHdr)) + m; }
 };
+// the environment of a map with more than 64 trains: two words per train set.  A type of its own rather than a third
+// template argument of EnvT, so that the types -- and the out-of-line callees named after them -- of the one-word
+// kernels stay exactly what they were
+template <bool TH, bool SQ_ = false> struct EnvW : EnvT<TH, SQ_> { static const int NW = 2; };
+template <bool TH, bool SQ, int NW> struct EnvOf { typedef EnvT<TH, SQ> type; };
+template <bool TH, bool SQ> struct EnvOf<TH, SQ, 2> { typedef EnvW<TH, SQ> type; };
+
+// the header's train sets as TSet<Env::NW>
+template <class Env> SFL_FN TSet<Env::NW> tset(const Env &e, int m) {
+  TSet<Env::NW> s; s.w[0] = e.hw0(m); if (Env::NW > 1) s.w[Env::NW - 1] = *e.hw1(m); return s;
+}
+template <class Env> SFL_FN void tset_put(const Env &e, int m, const TSet<Env::NW> &s) { e.hw0(m) = s.w[0]; if (Env::NW > 1) *e.hw1(m) = s.w[Env::NW - 1]; }
+template <class Env> SFL_FN int tset_any(const Env &e, int m) { return Env::NW == 1 ? e.hw0(m) != 0ull : (e.hw0(m) | *e.hw1(m)) != 0ull; }
+template <class Env> SFL_FN int tset_pop(const Env &e, int m) { TSet<Env::NW> s = tset(e, m); const int t = s.pop(); tset_put(e, m, s); return t; }
+template <class Env> SFL_FN void tset_add(const Env &e, int m, int t) {
+  if (Env::NW > 1 && t >= 64) *e.hw1(m) |= 1ull << (t & 63); else e.hw0(m) |= 1ull << t;
+}
 
 
 
@@ -526,11 +588,11 @@ SFL_FN void finish_decision(SFL_K, Env e, const Hp hp, int env_id) {
   EnvHdr *h = e.h();
   SFL_PHASE_START(h);
   if (mode == SFL_MODE_LEARN || mode == SFL_MODE_REPLAY) {
-    unsigned long long fresh = h->done_mask & ~h->at_dest_mask;
+    TSet<Env::NW> fresh = tset(e, HM_DONE).andnot(tset(e, HM_DEST));
     SFL_NU
-    while (fresh) {
-      int t = ffs64(fresh); fresh &= fresh - 1;
-      h->at_dest_mask |= 1ull << t;
+    while (fresh.any()) {
+      int t = fresh.pop();
+      tset_add(e, HM_DEST, t);
       int4 b = e.trb()[t];
       int n = (b.y >> 16) & 0xFF;
       SFL_NU
@@ -551,7 +613,7 @@ SFL_FN void finish_decision(SFL_K, Env e, const Hp hp, int env_id) {
   if (TRACE) {
     if (c_ra.trace_dec && h->cur_dec >= 0 && h->cur_dec < c_ra.dec_cap) {
       sfl_dec_rec *rec = c_ra.trace_dec + (size_t)env_id * c_ra.dec_cap + h->cur_dec;
-      rec->arrived = h->done_mask;
+      rec->arrived = h->done_mask; rec->arrived_hi = Env::NW > 1 ? *e.hw1(HM_DONE) : 0ull;
       rec->done = h->terminated | (h->truncated << 1);
       if (c_ra.trace_sem_buf) {
         int4 *dst = c_ra.trace_sem_buf + ((size_t)env_id * c_ra.dec_cap + h->cur_dec) * c_L.NP;
@@ -791,6 +853,7 @@ SFL_FN void decide(SFL_K, Env e, const Hp hp, int env_id, int t, const int semb_
         sfl_dec_rec *rec = c_ra.trace_dec + (size_t)env_id * c_ra.dec_cap + h->n_dec_logged;
         rec->ep = h->episode; rec->tick = now; rec->sw = s; rec->train = t; rec->key = key; rec->mask = mask;
         rec->action = action; rec->next_sw = next_switch; rec->reward = reward_in; rec->done = 0; rec->arrived = 0;
+        rec->arrived_hi = 0;
       }
       h->n_dec_logged++;
     }
@@ -832,6 +895,7 @@ SFL_RARE void env_reset(SFL_K, Env e, const Grp<G> &g, int on) {
     h->pending_fin = -1; h->cur_dec = -1; h->ev_cursor = 0; h->active_mask = 0; h->malf_prev_mask = 0; h->at_dest_mask = 0;
     h->eps_tag = -1;
     h->done_mask = 0; h->cum_reward = 0.0;
+    if (Env::NW > 1) { SFL_UA for (int m = 0; m < 4; m++) *e.hw1(m) = 0ull; }
   }
   g.sync();
 }
@@ -839,9 +903,9 @@ SFL_RARE void env_reset(SFL_K, Env e, const Grp<G> &g, int on) {
 // ------------------------------------------------------------------------------------------------ one tick (E5-E7, F2-F5)
 // Group-uniform registers carried across the ticks of a launch (every lane of the group holds the same values);
 // the header copy in shared memory is what the decision phase (first lane) reads and writes.
-struct TickRegs {
+template <int NW> struct TickRegs {
   int elapsed, ended, rng_blk;                 // rng_blk: 16-tick block the cached malfunction bytes belong to (-1: none)
-  unsigned long long active, done;
+  TSet<NW> active, done;
   unsigned ticks, train_ticks;                 // launch-local (max_ticks * T < 2^32), added to the header at the end
 };
 
@@ -863,7 +927,7 @@ SFL_FN int malf_stage2(const Hp hp, int now, int t) {
 template <int G, int KIND, bool ONE, class Env>
 // `live` = this group's environment takes part (not halted, not an idle slot of the last warp); every loop bound and
 // branch that contains a collective is warp-uniform, the per-group work inside is predicated.
-SFL_FN void env_tick(SFL_K, Env e, Scratch sc, const Hp hp, int env_id, const Grp<G> &g, TickRegs &R, const int live) {
+SFL_FN void env_tick(SFL_K, Env e, Scratch sc, const Hp hp, int env_id, const Grp<G> &g, TickRegs<Env::NW> &R, const int live) {
   const bool TRACE = KIND == K_FULL;
   EnvHdr *h = e.h();
   const int Tw = c_L.T;                                                  // warp-uniform loop bound
@@ -936,7 +1000,8 @@ SFL_FN void env_tick(SFL_K, Env e, Scratch sc, const Hp hp, int env_id, const Gr
   if (fresh_rng) R.rng_blk = now >> 4;
   g.sync();
   // ---- phase B: motion check (F3)
-  unsigned long long chain = 0;               // trains whose destination is occupied by a train that is itself moving
+  TSet<Env::NW> chain;                        // trains whose destination is occupied by a train that is itself moving
+  chain.clear();
   SFL_NU
   for (int base = 0; base < (ONE ? 1 : Tw); base += (ONE ? 1 : G)) {
     const int t = base + g.gl;
@@ -957,14 +1022,14 @@ SFL_FN void env_tick(SFL_K, Env e, Scratch sc, const Hp hp, int env_id, const Gr
       sc.occ()[t] = (int8_t)occ; sc.blk()[t] = (uint8_t)blocked;
       follows = !blocked && occ >= 0;
     }
-    chain |= (unsigned long long)g.ballot(follows) << base;
+    chain.or_ballot(g.ballot(follows), base);
   }
   g.sync();
-  if (g.wany(chain != 0)) {                                               // chains: fixed point (monotone)
+  if (g.wany(chain.any())) {                                               // chains: fixed point (monotone)
     SFL_NU
     for (int iter = 0; iter < Tw; iter++) {
       int changed = 0;
-      if (chain) {
+      if (chain.any()) {
         SFL_NU
         for (int t = g.gl, once_ = 1; t < T && (!ONE || once_); t += G, once_ = 0) {
           int occ = sc.occ()[t];
@@ -977,7 +1042,8 @@ SFL_FN void env_tick(SFL_K, Env e, Scratch sc, const Hp hp, int env_id, const Gr
   }
   // ---- phase C: state machine + position update (Appendix B steps 4-5), held-back trains (switch_env.py:353-367),
   //      and _check_active_switch (switch_env.py:427-485), which reads only the train's own new state
-  unsigned long long done_bits = 0, malf_bits = 0, stopped_bits = 0, depart_bits = 0, active = 0;
+  TSet<Env::NW> done_bits, malf_bits, stopped_bits, depart_bits, active;
+  done_bits.clear(); malf_bits.clear(); stopped_bits.clear(); depart_bits.clear(); active.clear();
   SFL_NU
   for (int base = 0; base < (ONE ? 1 : Tw); base += (ONE ? 1 : G)) {
     const int t = base + g.gl;
@@ -1052,58 +1118,57 @@ SFL_FN void env_tick(SFL_K, Env e, Scratch sc, const Hp hp, int env_id, const Gr
       ta.w = mc | (next_port << 16);
       e.tra()[t] = ta;
     }
-    done_bits |= (unsigned long long)g.ballot(f_done) << base;
-    malf_bits |= (unsigned long long)g.ballot(f_malf) << base;
-    stopped_bits |= (unsigned long long)g.ballot(f_stop) << base;
-    depart_bits |= (unsigned long long)g.ballot(f_dep) << base;
-    active |= (unsigned long long)g.ballot(f_act) << base;
+    done_bits.or_ballot(g.ballot(f_done), base);
+    malf_bits.or_ballot(g.ballot(f_malf), base);
+    stopped_bits.or_ballot(g.ballot(f_stop), base);
+    depart_bits.or_ballot(g.ballot(f_dep), base);
+    active.or_ballot(g.ballot(f_act), base);
   }
-  const unsigned long long all_mask = Tw >= 64 ? ~0ull : ((1ull << Tw) - 1ull);
-  const int ended = live && (done_bits == all_mask || now >= c_m.max_episode_steps);   // dones["__all__"] (Appendix B step 6)
-  const unsigned long long prev_done = R.done;
+  const int ended = live && (done_bits.all(Tw) || now >= c_m.max_episode_steps);   // dones["__all__"] (Appendix B step 6)
+  const TSet<Env::NW> prev_done = R.done;
   // ---- phase D2: semaphores of done trains (switch_env.py:370-376); every train counts as done at the end
-  const int release = (done_bits & ~prev_done) || ended;
+  const int release = done_bits.andnot(prev_done).any() || ended;
   if (g.wany(release)) {
     const int NP = release ? c_L.NP : 0;
     SFL_NU
     for (int p = g.gl; p < NP; p += G) {
       int tr = e.owner(p);
-      if (tr >= 0 && (ended || ((done_bits >> tr) & 1))) e.sem_drop(p);
+      if (tr >= 0 && (ended || done_bits.test(tr))) e.sem_drop(p);
     }
   }
   // ---- phase D3: departure bookings (switch_env.py:379-384), train order
-  if (g.wany(depart_bits != 0)) {
+  if (g.wany(depart_bits.any())) {
     g.sync();
-    if (depart_bits && g.gl == 0) {
-      unsigned long long b = depart_bits;
+    if (depart_bits.any() && g.gl == 0) {
+      TSet<Env::NW> b = depart_bits;
       SFL_NU
-      while (b) {
-        int t = ffs64(b); b &= b - 1;
+      while (b.any()) {
+        int t = b.pop();
         int4 tr1 = c_m.train1[t];
         e.sem_put((int)((unsigned)e.tra()[t].w >> 16), make_int4(tr1.x - 2, tr1.w + 2, t, SEM_IN));
       }
     }
   }
   // ---- phase D4: extend_semaphores (rail_network.py:229-244)
-  if (g.wany(stopped_bits != 0)) {
+  if (g.wany(stopped_bits.any())) {
     g.sync();
-    const int NP = stopped_bits ? c_L.NP : 0;
+    const int NP = stopped_bits.any() ? c_L.NP : 0;
     SFL_NU
     for (int p = g.gl; p < NP; p += G) {
       if (Env::HOT_TAIL) {
         int4 r = e.sem()[p];
-        if (r.z >= 0 && ((stopped_bits >> r.z) & 1)) e.sem()[p].x = now;
+        if (r.z >= 0 && stopped_bits.test(r.z)) e.sem()[p].x = now;
       } else {
         const int holder = e.owner(p);                                   // only the records of stopped trains leave shared memory
-        if (holder >= 0 && ((stopped_bits >> holder) & 1)) e.sem()[p].x = now;      // a 4-byte store, no load
+        if (holder >= 0 && stopped_bits.test(holder)) e.sem()[p].x = now;      // a 4-byte store, no load
       }
     }
     g.sync();
-    if (stopped_bits && g.gl == 0) {
-      unsigned long long b = stopped_bits;
+    if (stopped_bits.any() && g.gl == 0) {
+      TSet<Env::NW> b = stopped_bits;
       SFL_NU
-      while (b) {
-        int t = ffs64(b); b &= b - 1;
+      while (b.any()) {
+        int t = b.pop();
         int4 ta = e.tra()[t];
         if (((ta.y >> 8) & 0xFF) == ST_MALF) {
           int port = (int)((unsigned)ta.w >> 16);
@@ -1114,16 +1179,17 @@ SFL_FN void env_tick(SFL_K, Env e, Scratch sc, const Hp hp, int env_id, const Gr
   }
   if (live && g.gl == 0) {
     h->elapsed = now;
-    const unsigned long long new_malf = malf_bits & ~h->malf_prev_mask;
-    if (new_malf) h->num_malf += popc64(new_malf);                       // switch_env.py:399-401
-    if (malf_bits != h->malf_prev_mask) h->malf_prev_mask = malf_bits;
-    if (done_bits != prev_done) h->done_mask = done_bits;
+    const TSet<Env::NW> malf_prev = tset(e, HM_MALF);
+    const TSet<Env::NW> new_malf = malf_bits.andnot(malf_prev);
+    if (new_malf.any()) h->num_malf += new_malf.popc();                  // switch_env.py:399-401
+    if (!(malf_bits == malf_prev)) tset_put(e, HM_MALF, malf_bits);
+    if (!(done_bits == prev_done)) tset_put(e, HM_DONE, done_bits);
     if (ended) h->terminated = 1;
-    if (active) h->active_mask = active;                                 // the queue is empty whenever a tick runs
+    if (active.any()) tset_put(e, HM_ACTIVE, active);                     // the queue is empty whenever a tick runs
     if (TRACE) { if (c_ra.trace_tick) h->n_tick_logged++; }
   }
   R.elapsed = now; R.ended = ended; R.active = active; R.done = done_bits;
-  if (live) { R.ticks++; R.train_ticks += (unsigned)(T - popc64(prev_done)); }
+  if (live) { R.ticks++; R.train_ticks += (unsigned)(T - prev_done.popc()); }
   g.sync();
 }
 
@@ -1132,16 +1198,18 @@ template <class Env>
 SFL_RARE void episode_end(SFL_K, Env e, int env_id) {   // first lane
   EnvHdr *h = e.h();
   if (c_ra.ep_log && h->n_ep_logged < c_ra.ep_cap) {
+    const TSet<Env::NW> done = tset(e, HM_DONE);
     sfl_ep_rec *rec = c_ra.ep_log + (size_t)env_id * c_ra.ep_cap + h->n_ep_logged;
-    rec->cum_reward = h->cum_reward; rec->decisions = h->step_counter; rec->arrived = popc64(h->done_mask);
-    rec->num_malfunctions = h->num_malf; rec->ticks = h->elapsed; rec->arrived_mask = h->done_mask;
+    rec->cum_reward = h->cum_reward; rec->decisions = h->step_counter; rec->arrived = done.popc();
+    rec->num_malfunctions = h->num_malf; rec->ticks = h->elapsed; rec->arrived_mask = done.w[0];
+    rec->arrived_mask_hi = Env::NW > 1 ? done.w[Env::NW - 1] : 0ull;
     if (c_ra.ep_delay) {
       int *d = c_ra.ep_delay + ((size_t)env_id * c_ra.ep_cap + h->n_ep_logged) * c_L.T;
       SFL_NU
       for (int t = 0; t < c_L.T; t++) d[t] = e.trb()[t].z;
     }
   }
-  h->arrived_trains += (unsigned)popc64(h->done_mask);
+  h->arrived_trains += (unsigned)tset(e, HM_DONE).popc();
   h->n_ep_logged++;
   h->episode++;
   h->need_reset = 1;
@@ -1173,9 +1241,10 @@ SFL_FN void step_report(SFL_K, Env e, int env_id, int t) {
   }
   o->done = h->terminated | (h->truncated << 1);
   o->elapsed = h->elapsed; o->last_next_sw = h->last_next_sw; o->arrived = h->done_mask;
+  o->arrived_hi = Env::NW > 1 ? *e.hw1(HM_DONE) : 0ull;
 }
 
-template <int G, int KIND, bool TH, bool SQ, bool ONE>
+template <int G, int KIND, bool TH, bool SQ, bool ONE, int NW = 1>
 SFL_FN void env_run(SFL_K, int env_id, unsigned stage, char *host_scratch) {
   const bool TRACE = KIND == K_FULL;
   const Grp<G> g;
@@ -1183,7 +1252,7 @@ SFL_FN void env_run(SFL_K, int env_id, unsigned stage, char *host_scratch) {
   if (!valid) env_id = 0;
   char *gbase = c_ra.state + (size_t)env_id * c_L.env_stride;
   const unsigned hot_bytes = valid ? c_ra.hot_bytes : 0u;
-  EnvT<TH, SQ> e;
+  typename EnvOf<TH, SQ, NW>::type e;
   Hp hp;
   Scratch sc;
   e.kp = &K; sc.kp = &K;
@@ -1218,12 +1287,12 @@ SFL_FN void env_run(SFL_K, int env_id, unsigned stage, char *host_scratch) {
   sc.base = host_scratch;
 #endif
   EnvHdr *h = e.h();
-  TickRegs R;
-  R.elapsed = 0; R.ended = 0; R.rng_blk = -1; R.active = 0; R.done = 0; R.ticks = 0; R.train_ticks = 0;
+  TickRegs<NW> R;
+  R.elapsed = 0; R.ended = 0; R.rng_blk = -1; R.active.clear(); R.done.clear(); R.ticks = 0; R.train_ticks = 0;
   int need_reset = 0, live = 0;
   if (valid) {
     R.elapsed = h->elapsed; R.ended = h->terminated | h->truncated;
-    R.active = h->active_mask; R.done = h->done_mask;
+    R.active = tset(e, HM_ACTIVE); R.done = tset(e, HM_DONE);
     need_reset = h->need_reset; live = !h->halted;
   }
   const int stepping = TRACE && run_mode<KIND>(K) == SFL_MODE_STEP;
@@ -1239,14 +1308,14 @@ SFL_FN void env_run(SFL_K, int env_id, unsigned stage, char *host_scratch) {
   int any_reset = g.wany(live && need_reset);                             // warp-uniform; can only change in a decision phase
   SFL_NU
   for (int it = 0; it < c_ra.max_ticks; it++) {
-    const int due = live && !paused && (R.active || R.ended);             // something is due before the tick
+    const int due = live && !paused && (R.active.any() || R.ended);             // something is due before the tick
     const unsigned wf = g.wor((live && !paused ? 1u : 0u) | (due ? 2u : 0u));   // one warp-wide OR: anybody running / due
     if (!(wf & 1u)) break;
     if (wf & 2u) {
       if (due && g.gl == 0 && stepping) {
-        if (h->pending_fin >= 0 && (h->active_mask || h->terminated)) finish_decision<KIND>(K, e, hp, env_id);
+        if (h->pending_fin >= 0 && (tset_any(e, HM_ACTIVE) || h->terminated)) finish_decision<KIND>(K, e, hp, env_id);
         int t = -1;
-        if (!(h->terminated || h->truncated) && h->active_mask) { t = ffs64(h->active_mask); h->active_mask &= h->active_mask - 1; }
+        if (!(h->terminated || h->truncated) && tset_any(e, HM_ACTIVE)) t = tset_pop(e, HM_ACTIVE);
         step_report(K, e, env_id, t);
         if (h->terminated || h->truncated) episode_end(K, e, env_id);
       } else if (SQ && !stepping) {
@@ -1256,9 +1325,9 @@ SFL_FN void env_run(SFL_K, int env_id, unsigned stage, char *host_scratch) {
         SFL_NU
         while (g.wany(more)) {
           if (more && g.gl == 0) {
-            if (h->pending_fin >= 0 && (h->active_mask || h->terminated)) finish_decision<KIND>(K, e, hp, env_id);
-            h->dec_go = !(h->terminated || h->truncated || !h->active_mask);
-            if (h->dec_go) { h->dec_t = ffs64(h->active_mask); h->active_mask &= h->active_mask - 1; }
+            if (h->pending_fin >= 0 && (tset_any(e, HM_ACTIVE) || h->terminated)) finish_decision<KIND>(K, e, hp, env_id);
+            h->dec_go = !(h->terminated || h->truncated || !tset_any(e, HM_ACTIVE));
+            if (h->dec_go) h->dec_t = tset_pop(e, HM_ACTIVE);
           }
           g.sync();
           if (more) more = h->dec_go;
@@ -1270,16 +1339,15 @@ SFL_FN void env_run(SFL_K, int env_id, unsigned stage, char *host_scratch) {
       } else if (due && g.gl == 0) {
         SFL_NU
         for (;;) {                                                        // agent_iter: FIFO in train-handle order
-          if (h->pending_fin >= 0 && (h->active_mask || h->terminated)) finish_decision<KIND>(K, e, hp, env_id);
-          if (h->terminated || h->truncated || !h->active_mask) break;
-          int t = ffs64(h->active_mask);
-          h->active_mask &= h->active_mask - 1;
+          if (h->pending_fin >= 0 && (tset_any(e, HM_ACTIVE) || h->terminated)) finish_decision<KIND>(K, e, hp, env_id);
+          if (h->terminated || h->truncated || !tset_any(e, HM_ACTIVE)) break;
+          const int t = tset_pop(e, HM_ACTIVE);
           decide<KIND>(K, e, hp, env_id, t);
         }
         if (h->terminated || h->truncated) episode_end(K, e, env_id);
       }
       g.sync();
-      if (due) { need_reset = h->need_reset; R.active = 0; if (stepping) paused = h->cur_train >= 0; }
+      if (due) { need_reset = h->need_reset; R.active.clear(); if (stepping) paused = h->cur_train >= 0; }
       any_reset = g.wany(live && need_reset);
     }
     if (any_reset) {
@@ -1288,7 +1356,7 @@ SFL_FN void env_run(SFL_K, int env_id, unsigned stage, char *host_scratch) {
       if (on && g.gl == 0) SFL_PHASE_START(h);
       env_reset<G>(K, e, g, on);
       if (on && g.gl == 0) SFL_PHASE_MARK(h, PH_RESET);
-      if (on) { need_reset = 0; R.elapsed = 0; R.ended = 0; R.rng_blk = -1; R.active = 0; R.done = 0; }
+      if (on) { need_reset = 0; R.elapsed = 0; R.ended = 0; R.rng_blk = -1; R.active.clear(); R.done.clear(); }
       any_reset = 0;
     }
     if (live && !paused && g.gl == 0) SFL_PHASE_START(h);

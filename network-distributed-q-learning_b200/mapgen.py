@@ -410,6 +410,13 @@ def c4_fixture() -> dict:
                         max_duration=15, name="c4_rail100_t50")
 
 
+def t100_fixture() -> dict:
+    """The reference's 100-train evaluation (plot.ipynb "100_agents_challenge") on the C4 rail network: the map of
+    ``c4_fixture`` with 100 trains on its timetable.  Generated from its seed, never stored."""
+    return rail_fixture(100, 100, 0, n_rings=3, n_lines=20, cross_every=8, num_cities=25, malfunction_rate=0.01, min_duration=5,
+                        max_duration=15, name="rail100_t100")
+
+
 def offmap_malfunction_fixture() -> dict:
     """The 7x7 loop + chord map with two trains that share their entry cell (opposite headings): with injected
     malfunctions it exercises flatland's MALFUNCTION_OFF_MAP -> STOPPED transition onto an occupied cell (row F4)."""

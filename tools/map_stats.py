@@ -6,6 +6,7 @@ generator parameters can be tuned on the GPU-less box.  The numbers to compare a
 curves (BASELINE.md: about 5.8 of 15 trains arrive at episode 0 with epsilon 0.5, about 14.7 of 15 once trained).
 
     python tools/map_stats.py tests/golden/c4_synth100_t50.fixture.npz [--envs 8] [--episodes 3]
+    python tools/map_stats.py mapgen.t100_fixture                # a map generated from its seed by a mapgen function
 """
 from __future__ import annotations
 
@@ -61,12 +62,13 @@ def stats(fx: dict, n_envs: int = 8, n_ep: int = 3, seed0: int = 450565, q_cap: 
 
 def main():
     ap = argparse.ArgumentParser()
-    ap.add_argument("fixture", nargs="+")
+    ap.add_argument("fixture", nargs="+", help="fixture .npz, or mapgen.<function> for a generated map")
     ap.add_argument("--envs", type=int, default=8)
     ap.add_argument("--episodes", type=int, default=3)
     args = ap.parse_args()
     for path in args.fixture:
-        s = stats(mapgen.load_fixture(path), args.envs, args.episodes)
+        fx = getattr(mapgen, path[len("mapgen."):])() if path.startswith("mapgen.") else mapgen.load_fixture(path)
+        s = stats(fx, args.envs, args.episodes)
         print({k: (round(v, 3) if isinstance(v, float) else v) for k, v in s.items()})
 
 
