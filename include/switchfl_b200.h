@@ -24,7 +24,7 @@
 extern "C" {
 #endif
 
-#define SFL_ABI_VERSION 7
+#define SFL_ABI_VERSION 8
 
 enum {
   SFL_OK = 0,
@@ -49,7 +49,7 @@ enum {
 
 /* run modes (sfl_run) */
 enum {
-  SFL_MODE_LEARN = 0,    /* distr_q.py:296-366  epsilon-greedy + Q-update (Philox instead of PCG64)  */
+  SFL_MODE_LEARN = 0,    /* distr_q.py:296-366  epsilon-greedy + Q-update (Philox, or the reference's PCG64: sfl_config.rng) */
   SFL_MODE_GREEDY = 1,   /* distr_q.py:195-224  test(): max_action only, no update                   */
   SFL_MODE_REPLAY = 2,   /* learn() with the actions (and malfunction events) of a recorded trace; an action
                             with bit 6 set was an exploit choice: the row is looked up (inserted) and the
@@ -91,7 +91,25 @@ typedef struct sfl_config {
   int32_t shared_q;             /* 1: shared-table mode (extension, no counterpart in the reference): every environment
                                    of this context reads ONE dense Q table and accumulates its TD steps into a delta
                                    buffer; sfl_shared_q_apply folds the mean step into the table (see DESIGN.md)  */
+  int32_t rng;                  /* epsilon-greedy stream of SFL_MODE_LEARN: SFL_RNG_PHILOX (0) or SFL_RNG_REFERENCE (1)      */
 } sfl_config;
+
+/* sfl_config.rng.
+ * SFL_RNG_PHILOX: counter-based Philox4x32-10 draws (DESIGN.md section 4); the specialised learn kernels.
+ * SFL_RNG_REFERENCE: the reference learner's own numpy stream, so that a seeded learn() makes the reference's decisions.
+ *   distr_q.py:269 creates rng = np.random.default_rng(seed) at the start of learn(); per decision (:315-317)
+ *     if rng.random() < epsilon * epsilon_decay_rate ** n:      n = interactions of the deciding switch
+ *         action_space.seed(int(rng.integers(0, 2**31 - 1)))  then  action = action_space.sample(mask)
+ *   i.e. Generator(PCG64(SeedSequence(sd))).choice(where(mask)).  Here: per environment one PCG64 generator (SeedSequence
+ *   seeding, XSL-RR output, random() = (next_uint64 >> 11) * 2^-53, integers() = Lemire's method on 32-bit draws with
+ *   the carried half-word), seeded from sfl_hparams.seed by every sfl_reset that does not keep the interaction counters
+ *   (keep bit 1 clear: the start of a learn() call) and continued by every other reset; consumed by SFL_MODE_LEARN only,
+ *   one random() per decision, exploit included.  The comparison with epsilon is exact (the power is recomputed when the
+ *   draw is within rounding of it); decisions equal the reference's when lr_decay_rate == 1 (else Q-values agree to
+ *   1e-12 relative, and so do decisions unless a tie is that close).  Learn runs use the full kernel; a bound
+ *   malfunction schedule (ev_cap > 0) replaces the Philox malfunction draws in learn mode too.  Not with shared_q.
+ *   The stream's state takes 48 bytes of every env block, after the header; with SFL_RNG_PHILOX it takes none.      */
+enum { SFL_RNG_PHILOX = 0, SFL_RNG_REFERENCE = 1 };
 
 /* DistrQLearning.__init__ arguments (distr_q.py:32) + MalfunctionParameters (main.py:28-33), per env */
 typedef struct sfl_hparams {
@@ -120,6 +138,8 @@ typedef struct sfl_sizes {
   uint64_t shared_c_bytes;      /*   ... x a_max int32 (number of TD steps)                           */
   int32_t q_stride;             /* doubles per Q row (1 key slot + A_max)                             */
   int32_t a_max;
+  uint64_t rng_offset;          /* SFL_RNG_REFERENCE: byte offset of the stream's state in an env block: uint64 state_hi,
+                                   state_lo, inc_hi, inc_lo, uint32 has_uint32, uinteger (numpy's PCG64 state); 0 otherwise */
 } sfl_sizes;
 
 typedef struct sfl_buffers {    /* all device pointers; optional ones may be NULL                     */
@@ -187,6 +207,19 @@ int sfl_distance_map(const uint16_t *grid, int32_t H, int32_t W, const int32_t *
  * {q, lr, reward, gamma, max_next, bootstrap (0: the train stayed at the same switch, :444-447)}; out[i] = new Q(s, a). */
 int sfl_kat_q_update(const double *operands, int32_t n, double *out, int device);
 
+/* Known-answer hooks of SFL_RNG_REFERENCE, evaluated ON THE DEVICE with the kernel's own functions.
+ * sfl_kat_pcg64: n generators, gens[6 g ..] = {state_hi, state_lo, inc_hi, inc_lo, has_uint32, uinteger}, or -- when inc_lo is
+ * even (a PCG64 increment is odd) -- the generator np.random.default_rng(state_lo); then n_codes draws each, codes[g n_codes + k]:
+ *   0                     random()                                     -> the double's bits
+ *   1 .. 2^32             integers(0, code)                            -> the value
+ *   2^63 | mask           one exploring decision (distr_q.py:316-317)  -> the action: the integers(0, 2**31 - 1)-th seed's
+ *                         Generator(PCG64(SeedSequence(sd))).choice over the set bits of mask
+ * out[(12 + n_codes) g ..] = the 6 words after seeding, the n_codes results, the 6 words of the final state.
+ * sfl_kat_explore: rows {u, epsilon, decay, n, running product of the decay over n interactions}; out[i] = 1 iff the
+ * kernel explores, i.e. u < epsilon * decay ** n as the reference evaluates it (distr_q.py:315).                      */
+int sfl_kat_pcg64(const uint64_t *gens, const uint64_t *codes, int32_t n, int32_t n_codes, uint64_t *out, int device);
+int sfl_kat_explore(const double *rows, int32_t n, int32_t *out, int device);
+
 int sfl_abi_version(void);
 const char *sfl_last_error(void);
 
@@ -195,13 +228,15 @@ const char *sfl_last_error(void);
 int sfl_query_sizes(const sfl_map_desc *map, const sfl_config *cfg, sfl_sizes *out);
 
 /* replaces ASyncSwitchEnv(rail_env, ...) + DistrQLearning(env, ...)   (main.py:51-60).  T must be in 1..128;
- * shared-table mode (sfl_config.shared_q) takes at most 64 trains.                                               */
+ * shared-table mode (sfl_config.shared_q) takes at most 64 trains and not SFL_RNG_REFERENCE (the reference has no shared
+ * table, and its learner one stream).                                                                              */
 int sfl_create(const sfl_map_desc *map, const sfl_config *cfg, int device, void **ctx);
 int sfl_destroy(void *ctx);                       /* env.close() (switch_env.py, called at distr_q.py:241, 379) + garbage collection */
 int sfl_bind(void *ctx, const sfl_buffers *bufs); /* hand over the caller-owned device buffers sized by sfl_query_sizes            */
 
 /* zero state + mark every env "needs reset"; the first sfl_run performs env.reset (switch_env.py:93-158)
- * on the device.  keep_q != 0 keeps Q tables and interaction counters (a new learn()/test() call).     */
+ * on the device.  keep bit 0 keeps the Q tables, bit 1 the per-switch interaction counters (and, with SFL_RNG_REFERENCE,
+ * continues the random stream; without bit 1 every environment's stream restarts from sfl_hparams.seed).              */
 int sfl_reset(void *ctx, int keep_q, void *stream);
 
 /* Lanes of a warp that cooperate on one environment (1, 2, 4, 8, 16 or 32; 32/lanes environments share a warp and
@@ -223,7 +258,7 @@ int sfl_set_roomy(void *ctx, int roomy);
 int sfl_set_phase_clock(void *ctx, int on);
 /* Which kernel instantiation and launch configuration sfl_run(mode) would use now (traced != 0: with decision / tick
  * traces), as text: "k_run<G=..,KIND=..,TH=..,SQ=..,ONE=..,ROOMY=..> grid=.. block=.. smem=..", with ",NW=2" after ROOMY
- * on maps with more than 64 trains (two words per train set).  No counterpart in the
+ * on maps with more than 64 trains (two words per train set); learn with SFL_RNG_REFERENCE is KIND=full.  No counterpart in the
  * reference; it lets the parity tests name -- and force, with sfl_set_lanes / sfl_set_roomy -- exactly the
  * instantiations the benchmark launches.  Needs no bound buffers.                                                  */
 int sfl_describe_launch(void *ctx, int mode, int traced, char *buf, int cap);

@@ -18,8 +18,10 @@ from . import railmap
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "csrc", "libswitchfl_b200.so")
 
-ABI_VERSION = 7
+ABI_VERSION = 8
 MODE_LEARN, MODE_GREEDY, MODE_REPLAY, MODE_STEP = 0, 1, 2, 3
+RNG_PHILOX, RNG_REFERENCE = 0, 1
+RNG_NAMES = {"philox": RNG_PHILOX, "reference": RNG_REFERENCE}
 ERR_NO_TRAIN_AT_SWITCH = 1
 ERR_BITS = {1: "no train at active switch (observer.py:294-307)", 2: "infinite distance to target (observer.py:35-36)",
             4: "per-env Q table full (raise q_cap)", 8: "pending-update list full (raise pend_cap)",
@@ -42,14 +44,14 @@ class MapDesc(C.Structure):
 
 class Config(C.Structure):
     _fields_ = [(n, C.c_int32) for n in ("n_envs", "q_cap", "pend_cap", "max_steps", "dec_cap", "tick_cap", "ep_cap",
-                                         "act_cap", "ev_cap", "trace_sem", "shared_q")]
+                                         "act_cap", "ev_cap", "trace_sem", "shared_q", "rng")]
 
 
 class Sizes(C.Structure):
     _fields_ = [(n, C.c_uint64) for n in ("state_bytes", "env_stride", "hparams_bytes", "trace_dec_bytes", "trace_tick_bytes",
                                           "trace_sem_bytes", "ep_log_bytes", "ep_delay_bytes", "replay_act_bytes",
                                           "replay_ev_bytes", "counters_bytes", "step_out_bytes", "shared_q_bytes", "shared_d_bytes",
-                                          "shared_c_bytes")] + [("q_stride", C.c_int32), ("a_max", C.c_int32)]
+                                          "shared_c_bytes")] + [("q_stride", C.c_int32), ("a_max", C.c_int32), ("rng_offset", C.c_uint64)]
 
 
 class Buffers(C.Structure):
@@ -110,6 +112,8 @@ def load_library(path: Optional[str] = None) -> C.CDLL:
     lib.sfl_shared_q_apply.argtypes = [C.c_void_p, C.c_void_p]
     lib.sfl_shared_q_apply_to.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
     lib.sfl_kat_q_update.argtypes = [C.POINTER(C.c_double), C.c_int32, C.POINTER(C.c_double), C.c_int]
+    lib.sfl_kat_pcg64.argtypes = [C.POINTER(C.c_uint64), C.POINTER(C.c_uint64), C.c_int32, C.c_int32, C.POINTER(C.c_uint64), C.c_int]
+    lib.sfl_kat_explore.argtypes = [C.POINTER(C.c_double), C.c_int32, C.POINTER(C.c_int32), C.c_int]
     lib.sfl_distance_map.argtypes = [_u16p, C.c_int32, C.c_int32, _i32p, C.c_int32, _i32p, C.c_int]
     if lib.sfl_abi_version() != ABI_VERSION:
         raise RuntimeError("switchfl_b200 ABI version mismatch")
@@ -139,6 +143,40 @@ def device_q_update(rows: Sequence[Sequence[float]], device: int = 0, lib: Optio
     if rc != 0:
         raise RuntimeError(f"switchfl_b200 error {rc}: {lib.sfl_last_error().decode()}")
     return out
+
+
+def device_pcg64(gens, codes, device: int = 0, lib: Optional[C.CDLL] = None):
+    """``sfl_kat_pcg64``: the device's copy of the reference's random stream (SFL_RNG_REFERENCE).  ``gens``: rows of
+    (state_hi, state_lo, inc_hi, inc_lo, has_uint32, uinteger), or (0, seed, 0, 0, 0, 0) for ``np.random.default_rng(seed)``;
+    ``codes[g]``: the draws of generator g (0: random(), 1..2^32: integers(0, code), 2^63 | mask: one exploring decision).
+    Returns (states after seeding [n, 6], results [n, n_codes] as uint64, final states [n, 6])."""
+    lib = lib or load_library()
+    g = np.ascontiguousarray(np.asarray(gens, dtype=object).astype(np.uint64)).reshape(-1, 6)
+    c = np.ascontiguousarray(np.asarray(codes, dtype=object).astype(np.uint64)).reshape(len(g), -1)
+    out = np.zeros((len(g), 12 + c.shape[1]), np.uint64)
+    u64p = C.POINTER(C.c_uint64)
+    rc = lib.sfl_kat_pcg64(g.ctypes.data_as(u64p), c.ctypes.data_as(u64p), len(g), c.shape[1], out.ctypes.data_as(u64p), int(device))
+    if rc != 0:
+        raise RuntimeError(f"switchfl_b200 error {rc}: {lib.sfl_last_error().decode()}")
+    return out[:, :6], out[:, 6:6 + c.shape[1]], out[:, 6 + c.shape[1]:]
+
+
+def device_explore(rows, device: int = 0, lib: Optional[C.CDLL] = None) -> np.ndarray:
+    """``sfl_kat_explore``: the kernel's epsilon test on rows of (u, epsilon, decay, n, running product of the decay)."""
+    lib = lib or load_library()
+    a = np.ascontiguousarray(rows, np.float64).reshape(-1, 5)
+    out = np.zeros(len(a), np.int32)
+    rc = lib.sfl_kat_explore(a.ctypes.data_as(C.POINTER(C.c_double)), len(a), out.ctypes.data_as(C.POINTER(C.c_int32)), int(device))
+    if rc != 0:
+        raise RuntimeError(f"switchfl_b200 error {rc}: {lib.sfl_last_error().decode()}")
+    return out.astype(bool)
+
+
+def pcg64_state(words) -> dict:
+    """numpy's ``bit_generator.state`` of a PCG64 from the kernel's words (state_hi, state_lo, inc_hi, inc_lo, has_uint32, uinteger)."""
+    w = [int(x) for x in words]
+    return {"bit_generator": "PCG64", "state": {"state": (w[0] << 64) | w[1], "inc": (w[2] << 64) | w[3]},
+            "has_uint32": w[4], "uinteger": w[5]}
 
 
 def side_ok(engine) -> bool:
@@ -253,8 +291,15 @@ class Engine:
     def __init__(self, rail_map: RailMap, n_envs: int, device: str = "cuda:0", q_cap: int = 1024, pend_cap: int = 8,
                  max_steps: int = 100_000, dec_cap: int = 0, tick_cap: int = 0, ep_cap: int = 64, act_cap: int = 0,
                  ev_cap: int = 0, trace_sem: bool = False, lanes: Optional[int] = None, shared_q: bool = False,
-                 cta_warps: Optional[int] = None, roomy: Optional[bool] = None, phase_clock: bool = False, bind: bool = True):
-        """``bind=False`` creates the context only (no device buffers): enough for ``describe_launch``."""
+                 cta_warps: Optional[int] = None, roomy: Optional[bool] = None, phase_clock: bool = False, bind: bool = True,
+                 rng: str = "philox"):
+        """``bind=False`` creates the context only (no device buffers): enough for ``describe_launch``.
+        ``rng``: the epsilon-greedy stream of learn mode -- "philox" (the specialised learn kernels) or "reference" (numpy's
+        PCG64 stream of the reference learner, seeded per environment from its seed at every reset that restarts the
+        interaction counters: a seeded learn() makes the reference's decisions; runs on the full kernel)."""
+        if rng not in RNG_NAMES:
+            raise ValueError(f"rng must be one of {sorted(RNG_NAMES)}, not {rng!r}")
+        self.rng = rng
         import torch
         self.torch = torch
         self.map = rail_map
@@ -262,7 +307,7 @@ class Engine:
         self.lib, self.device, dev_index = self._open(device)
         self.cfg = Config(n_envs=self.n_envs, q_cap=q_cap, pend_cap=pend_cap, max_steps=max_steps, dec_cap=dec_cap,
                           tick_cap=tick_cap, ep_cap=ep_cap, act_cap=act_cap, ev_cap=ev_cap, trace_sem=int(trace_sem),
-                          shared_q=int(shared_q))
+                          shared_q=int(shared_q), rng=RNG_NAMES[rng])
         self.shared_q = bool(shared_q)
         self.sizes = Sizes()
         self._ck(self.lib.sfl_query_sizes(C.byref(rail_map.desc), C.byref(self.cfg), C.byref(self.sizes)))
@@ -559,6 +604,20 @@ class Engine:
         return self._download("step_out", self.n_envs * STEP_DT.itemsize).view(STEP_DT).copy()
 
     # ------------------------------------------------------------------ results
+    def rng_state(self, env: Optional[int] = None):
+        """The reference stream's state of every environment (or of ``env``) in numpy's ``bit_generator.state`` layout:
+        ``np.random.Generator(np.random.PCG64())`` with this state continues where the environment's learner stands."""
+        if self.rng != "reference":
+            raise RuntimeError('rng_state() needs Engine(rng="reference")')
+        off, stride = int(self.sizes.rng_offset), int(self.sizes.env_stride)
+        envs = range(self.n_envs) if env is None else [int(env)]
+        out = []
+        for i in envs:
+            raw = self.buf["state"][i * stride + off:i * stride + off + 48].cpu().numpy()
+            w = raw[:32].view(np.uint64)
+            out.append(pcg64_state([w[0], w[1], w[2], w[3], *raw[32:40].view(np.uint32)]))
+        return out if env is None else out[0]
+
     def total_decisions(self):
         d, t = C.c_uint64(), C.c_uint64()
         self._ck(self.lib.sfl_total_decisions(self.ctx, C.byref(d), C.byref(t), self._stream()))

@@ -7,9 +7,10 @@
 ``config.ini`` keeps the reference's sections and keys (hyperparam_tuning.py:51-78): MISC{random_seed, out_dir,
 checkpoint_freq, exploit_freq}, ENV{width, height, max_num_cities, max_rails_between_cities, max_rail_pairs_in_city,
 number_of_agents, malfunction_rate, min_duration, max_duration}, MODEL{gamma, epsilon, epsilon_decay_rate, lr,
-lr_decay_rate, default_q, num_episodes}.  Three optional keys are new: ENV.fixture (a map fixture .npz recorded from
-flatland, see tools/record_flatland_fixture.py), MISC.n_envs (lockstep replicas with seeds random_seed + i) and
-MISC.q_cap (Q hash rows per environment; default: sized from the map, see ``default_q_cap``).
+lr_decay_rate, default_q, num_episodes}.  Four optional keys are new: ENV.fixture (a map fixture .npz recorded from
+flatland, see tools/record_flatland_fixture.py), MISC.n_envs (lockstep replicas with seeds random_seed + i),
+MISC.q_cap (Q hash rows per environment; default: sized from the map, see ``default_q_cap``) and MISC.rng (``philox``,
+the default, or ``reference``: the reference's own numpy epsilon-greedy stream, see ``ASyncSwitchEnv``).
 Without ENV.fixture the map comes from the synthetic generator with the same size / train count / seed, because
 flatland's sparse_rail_generator cannot run here (mapgen.py).
 """
@@ -53,7 +54,7 @@ def default_device() -> str:
 
 
 def launch_experiment(config_path: str, device: Optional[str] = None, q_cap: Optional[int] = None, env_cls=ASyncSwitchEnv,
-                      _engine_kwargs=None) -> DistrQLearning:
+                      _engine_kwargs=None, rng: Optional[str] = None) -> DistrQLearning:
     """main.py:13-78."""
     start_time = time.time()
     device = device or default_device()
@@ -67,8 +68,9 @@ def launch_experiment(config_path: str, device: Optional[str] = None, q_cap: Opt
     rail_env = RailEnv(fixture_from_env_section(dict(envs), seed), malfunction_generator=mf)
     if q_cap is None and misc.get("q_cap"):
         q_cap = int(misc["q_cap"])
+    rng = rng or misc.get("rng", "philox")
     env = env_cls(rail_env, render_mode=None, max_steps=100_000, n_envs=int(misc.get("n_envs", 1)), device=device, q_cap=q_cap,
-                  _engine_kwargs=_engine_kwargs)
+                  rng=rng, _engine_kwargs=_engine_kwargs)
     model = DistrQLearning(env=env, gamma=float(mdl["gamma"]), epsilon=float(mdl["epsilon"]),
                            epsilon_decay_rate=float(mdl["epsilon_decay_rate"]), lr=float(mdl["lr"]),
                            lr_decay_rate=float(mdl["lr_decay_rate"]), default_q=float(mdl["default_q"]), seed=seed)
@@ -92,10 +94,13 @@ def launch_experiment(config_path: str, device: Optional[str] = None, q_cap: Opt
 
 def launch_grid(hyperparams: Dict[str, Sequence[float]], random_seeds: Sequence[int], out_dir: str, env_section: Dict[str, object],
                 num_episodes: int, checkpoint_freq: int, exploit_freq: Optional[int], gamma: float = 1.0, default_q: float = 0.0,
-                device: Optional[str] = None, q_cap: Optional[int] = None, env_cls=ASyncSwitchEnv, _engine_kwargs=None) -> List[str]:
+                device: Optional[str] = None, q_cap: Optional[int] = None, env_cls=ASyncSwitchEnv, _engine_kwargs=None,
+                rng: str = "philox") -> List[str]:
     """hyperparam_tuning.py:42-91: every (grid point, seed) pair gets ``out_dir/exp_i/seed_j/`` with its config.ini
     and the reference's output files.  One seed = one map (the generators are seeded with it), so each seed is ONE
-    batched engine whose environments are the grid points; under torchrun the seeds are sharded over the ranks."""
+    batched engine whose environments are the grid points; under torchrun the seeds are sharded over the ranks.
+    With ``rng="reference"`` every environment learns on the reference's stream of its seed: environment i of a seed is
+    the reference's main.py run for that (grid point, seed)."""
     names = list(hyperparams)
     points = [dict(zip(names, v)) for v in product(*[hyperparams[n] for n in names])]
     rank, world_size, _ = sharding.world()
@@ -109,7 +114,7 @@ def launch_grid(hyperparams: Dict[str, Sequence[float]], random_seeds: Sequence[
         mf = ParamMalfunctionGen(MalfunctionParameters(float(env_section.get("malfunction_rate", 0.0)),
                                                        int(env_section.get("min_duration", 0)), int(env_section.get("max_duration", 0))))
         env = env_cls(RailEnv(fx, malfunction_generator=mf), render_mode=None, max_steps=100_000, n_envs=len(points),
-                      device=device, q_cap=q_cap, _engine_kwargs=_engine_kwargs)
+                      device=device, q_cap=q_cap, rng=rng, _engine_kwargs=_engine_kwargs)
         col = lambda k, d: np.array([p.get(k, d) for p in points], np.float64)
         model = DistrQLearning(env=env, gamma=gamma, epsilon=col("epsilon", 0.4), epsilon_decay_rate=col("epsilon_decay_rate", 0.0),
                                lr=col("lr", 0.4), lr_decay_rate=col("lr_decay_rate", 0.0), default_q=default_q,
@@ -124,6 +129,8 @@ def launch_grid(hyperparams: Dict[str, Sequence[float]], random_seeds: Sequence[
             config = configparser.ConfigParser()
             config["MISC"] = {"random_seed": str(seed), "out_dir": exp_dir, "checkpoint_freq": str(checkpoint_freq),
                               "exploit_freq": str(exploit_freq)}
+            if rng != "philox":
+                config["MISC"]["rng"] = rng
             config["ENV"] = {k: str(v) for k, v in env_section.items()}
             config["MODEL"] = {"gamma": str(gamma), **{k: str(params[k]) for k in names}, "default_q": str(default_q),
                                "num_episodes": str(num_episodes)}
@@ -174,8 +181,10 @@ def main(argv=None):
     ap.add_argument("-c", "--config", type=str, help="Config file path", required=True)
     ap.add_argument("--device", default=None, help="default: cuda:<LOCAL_RANK>")
     ap.add_argument("--q-cap", type=int, default=None, help="Q hash rows per environment (default: MISC.q_cap, else sized from the map)")
+    ap.add_argument("--rng", choices=("philox", "reference"), default=None,
+                    help="epsilon-greedy stream of learn(): philox, or the reference's own numpy stream (default: MISC.rng, else philox)")
     args = ap.parse_args(argv)
-    launch_experiment(args.config, device=args.device, q_cap=args.q_cap)
+    launch_experiment(args.config, device=args.device, q_cap=args.q_cap, rng=args.rng)
 
 
 if __name__ == "__main__":

@@ -73,7 +73,7 @@ struct DeviceGuard {
 #define SFL_SMEM_BUDGET (56u * 1024u)                  // per CTA, so that four CTAs share an SM
 
 // ------------------------------------------------------------------------------------------------ kernels
-struct InitArgs { Layout L; char *state; int n_envs, keep_q, keep_ninter, pad; };
+struct InitArgs { Layout L; char *state; const sfl_hparams *hp; int n_envs, keep_q, keep_ninter, pad; };
 
 struct InitEnv {          // the env block in HBM, no staging
   const Layout *L;
@@ -108,6 +108,8 @@ SFL_FN void env_init(const InitArgs &ia, int env_id, int lane, int lanes) {
     z.need_reset = 1; z.pending_fin = -1; z.cur_dec = -1; z.q_rows = q_rows; z.cur_train = -1; z.last_next_sw = -1; z.eps_tag = -1;
     *e.h() = z;
     if (ia.L.T > 64) for (int m = 0; m < 4; m++) ((unsigned long long *)(e.b + sizeof(EnvHdr)))[m] = 0ull;   // word 1 of the train sets
+    // the reference's stream restarts with the interaction counters: np.random.default_rng(seed) at the start of learn() (distr_q.py:269)
+    if (ia.L.off_rng && !ia.keep_ninter) *(Pcg *)(e.b + ia.L.off_rng) = pcg_seed(ia.hp[env_id].seed);
   }
 }
 
@@ -131,7 +133,35 @@ SFL_FN void q_reinit_slot(const ReinitArgs &a, int env, int slot) {
   row[1 + (qi & 15)] = (qi & 16) ? 1000.0 : 500.0;
 }
 
+// known-answer hooks of the reference's stream: the kernel's own PCG64 / SeedSequence / epsilon functions on caller operands
+SFL_FN void pcg_words(const Pcg &g, uint64_t *o) { o[0] = g.s_hi; o[1] = g.s_lo; o[2] = g.i_hi; o[3] = g.i_lo; o[4] = g.has32; o[5] = g.u32; }
+SFL_FN void kat_pcg64_one(const uint64_t *gen, const uint64_t *codes, int n_codes, uint64_t *out) {
+  Pcg g;
+  if (gen[3] & 1ull) { g.s_hi = gen[0]; g.s_lo = gen[1]; g.i_hi = gen[2]; g.i_lo = gen[3]; g.has32 = (unsigned)gen[4]; g.u32 = (unsigned)gen[5]; g.pad0 = g.pad1 = 0u; }
+  else g = pcg_seed(gen[1]);
+  pcg_words(g, out);
+  for (int k = 0; k < n_codes; k++) {
+    const uint64_t c = codes[k];
+    uint64_t r;
+    if (!c) { const double d = pcg_double(g); memcpy(&r, &d, 8); }
+    else if (c >> 63) r = (uint64_t)pcg_explore_action(g, (int)(c & 0xFFFFull));
+    else r = pcg_bounded(g, c);
+    out[6 + k] = r;
+  }
+  pcg_words(g, out + 6 + n_codes);
+}
+SFL_FN int kat_explore_one(const double *r) { return eps_explore(r[0], r[1], r[2], (int)r[3], r[4]); }
+
 #ifndef SFL_HOST_EMUL
+__global__ void k_kat_pcg64(const uint64_t *gens, const uint64_t *codes, int n, int n_codes, uint64_t *out) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < n) kat_pcg64_one(gens + 6 * (size_t)i, codes + (size_t)i * n_codes, n_codes, out + (size_t)i * (12 + n_codes));
+}
+__global__ void k_kat_explore(const double *rows, int n, int *out) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < n) out[i] = kat_explore_one(rows + 5 * (size_t)i);
+}
+
 __global__ void __launch_bounds__(256) k_q_reinit(const __grid_constant__ ReinitArgs a) {
   const size_t n = (size_t)a.n_envs * a.L.q_cap;
   for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x)
@@ -150,9 +180,10 @@ __global__ void __launch_bounds__(SFL_CTA_THREADS) k_init(const __grid_constant_
 // ROOMY: compiled for 4 instead of 7 CTAs per SM (about 100 instead of 72 registers, no spills) -- for launches of the
 // large-map kernels that do not fill the SMs anyway (C3: 1024 one-environment warps per map, +10 %).
 // NW: 64-bit words per train set, 2 for maps with more than 64 trains (tail in HBM, 8 / 16 / 32 lanes, no ONE / ROOMY / SQ);
-// the wide full kernel (traces, replay, step protocol, phase clock) is compiled for 5 CTAs per SM: no spills.
+// The full kernels (traces, replay, step protocol, phase clock, learning on the reference's stream) are compiled for at most
+// 5 CTAs per SM: no spills.
 template <int G, int KIND, bool TH, bool SQ, bool ONE, bool ROOMY = false, int NW = 1>
-__global__ void __launch_bounds__(SFL_CTA_THREADS, NW > 1 ? (KIND == K_FULL ? 5 : SFL_MINB_WIDE) : TH ? (G == 32 ? 7 : 4) : (ROOMY ? 4 : SFL_MINB_BIG))
+__global__ void __launch_bounds__(SFL_CTA_THREADS, KIND == K_FULL ? (TH && G != 32 ? 4 : 5) : NW > 1 ? SFL_MINB_WIDE : TH ? (G == 32 ? 7 : 4) : (ROOMY ? 4 : SFL_MINB_BIG))
 k_run(const __grid_constant__ KArgs K) {
   const int slot = threadIdx.x / G;                    // environment slot inside the CTA
   const int env_id = blockIdx.x * (blockDim.x / G) + slot;
@@ -323,11 +354,14 @@ static int make_layout(const sfl_map_desc *map, const sfl_config *cfg, Layout *L
   for (int s = 0; s < map->S; s++) { if (map->sw_A[s] > a_max) a_max = map->sw_A[s]; if (map->sw_P[s] > 4) return fail(SFL_E_ARG, "P > 4%s"); }
   if (a_max > 15) return fail(SFL_E_ARG, "A > 15%s");
   if ((uint64_t)map->NP * map->NT * 48ull >= 0xFFFFFFFFull) return fail(SFL_E_ARG, "state index does not fit 32 bits%s");
+  if (cfg->rng != SFL_RNG_PHILOX && cfg->rng != SFL_RNG_REFERENCE) return fail(SFL_E_ARG, "rng must be SFL_RNG_PHILOX (0) or SFL_RNG_REFERENCE (1)%s");
   memset(L, 0, sizeof(*L));
   L->T = map->T; L->S = map->S; L->NP = map->NP; L->NT = map->NT; L->a_max = a_max; L->q_cap = cfg->q_cap;
   L->q_stride = 1 + a_max; L->pend_cap = cfg->pend_cap;
   unsigned T = (unsigned)map->T;
-  unsigned o = align_up((unsigned)sizeof(EnvHdr) + (T > 64 ? 4u * 8u : 0u), 16);     // + word 1 of the four train sets
+  unsigned o = (unsigned)sizeof(EnvHdr) + (T > 64 ? 4u * 8u : 0u);                   // + word 1 of the four train sets
+  if (cfg->rng == SFL_RNG_REFERENCE) { L->off_rng = o; o += SFL_PCG_BYTES; }          // + the reference's stream (none with Philox)
+  o = align_up(o, 16);
 #define PUT(field, bytes) L->field = o; o = align_up(o + (unsigned)(bytes), 16)
   PUT(off_tra, 16 * T); PUT(off_trb, 16 * T); PUT(off_pend, 8 * T * cfg->pend_cap);
   PUT(off_sem, 16 * (unsigned)map->NP); PUT(off_rewards, 4 * (unsigned)map->S * T); PUT(off_sws, 16 * (unsigned)map->S);
@@ -423,6 +457,59 @@ int sfl_kat_q_update(const double *operands, int32_t n, double *out, int device)
 #endif
 }
 
+// copy in, run the known-answer kernel, copy out (the host build runs the same functions in a loop)
+#ifndef SFL_HOST_EMUL
+struct KatBufs {
+  void *p[3] = {nullptr, nullptr, nullptr};
+  ~KatBufs() { for (void *q : p) cudaFree(q); }
+};
+#endif
+
+int sfl_kat_pcg64(const uint64_t *gens, const uint64_t *codes, int32_t n, int32_t n_codes, uint64_t *out, int device) {
+  if (!gens || !out || n < 0 || n_codes < 0 || (n_codes && !codes)) return fail(SFL_E_ARG, "bad argument%s");
+  for (size_t i = 0; i < (size_t)n * n_codes; i++)
+    if (!(codes[i] >> 63) && codes[i] > 0x100000000ull) return fail(SFL_E_ARG, "a bounded draw's range must be at most 2^32%s");
+  if (!n) return SFL_OK;
+  const size_t gb = (size_t)n * 48, cb = (size_t)n * n_codes * 8 + 8, ob = (size_t)n * (12 + n_codes) * 8;
+#ifndef SFL_HOST_EMUL
+  int ndev = 0;
+  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) return fail(SFL_E_CUDA, "no CUDA device: this library has no CPU path%s");
+  DeviceGuard guard(device);
+  KatBufs b;
+  CU(cudaMalloc(&b.p[0], gb)); CU(cudaMalloc(&b.p[1], cb)); CU(cudaMalloc(&b.p[2], ob));
+  CU(cudaMemcpy(b.p[0], gens, gb, cudaMemcpyHostToDevice));
+  if (n_codes) CU(cudaMemcpy(b.p[1], codes, cb - 8, cudaMemcpyHostToDevice));
+  k_kat_pcg64<<<(n + 127) / 128, 128>>>((const uint64_t *)b.p[0], (const uint64_t *)b.p[1], n, n_codes, (uint64_t *)b.p[2]);
+  CU(cudaGetLastError());
+  CU(cudaMemcpy(out, b.p[2], ob, cudaMemcpyDeviceToHost));
+#else
+  (void)device; (void)gb; (void)cb; (void)ob;
+  for (int i = 0; i < n; i++) kat_pcg64_one(gens + 6 * (size_t)i, codes + (size_t)i * n_codes, n_codes, out + (size_t)i * (12 + n_codes));
+#endif
+  return SFL_OK;
+}
+
+int sfl_kat_explore(const double *rows, int32_t n, int32_t *out, int device) {
+  if (!rows || !out || n < 0) return fail(SFL_E_ARG, "bad argument%s");
+  for (int i = 0; i < n; i++) if (!(rows[5 * i + 3] >= 0.0 && rows[5 * i + 3] < 2147483648.0)) return fail(SFL_E_ARG, "n must be in 0..2^31-1%s");
+  if (!n) return SFL_OK;
+#ifndef SFL_HOST_EMUL
+  int ndev = 0;
+  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) return fail(SFL_E_CUDA, "no CUDA device: this library has no CPU path%s");
+  DeviceGuard guard(device);
+  KatBufs b;
+  CU(cudaMalloc(&b.p[0], (size_t)n * 40)); CU(cudaMalloc(&b.p[1], (size_t)n * 4));
+  CU(cudaMemcpy(b.p[0], rows, (size_t)n * 40, cudaMemcpyHostToDevice));
+  k_kat_explore<<<(n + 127) / 128, 128>>>((const double *)b.p[0], n, (int *)b.p[1]);
+  CU(cudaGetLastError());
+  CU(cudaMemcpy(out, b.p[1], (size_t)n * 4, cudaMemcpyDeviceToHost));
+#else
+  (void)device;
+  for (int i = 0; i < n; i++) out[i] = kat_explore_one(rows + 5 * (size_t)i);
+#endif
+  return SFL_OK;
+}
+
 int sfl_query_sizes(const sfl_map_desc *map, const sfl_config *cfg, sfl_sizes *out) {
   Layout L; int a_max;
   int rc = make_layout(map, cfg, &L, &a_max);
@@ -445,6 +532,7 @@ int sfl_query_sizes(const sfl_map_desc *map, const sfl_config *cfg, sfl_sizes *o
   out->replay_ev_bytes = B * (uint64_t)cfg->ev_cap * 12ull;
   out->q_stride = L.q_stride;
   out->a_max = a_max;
+  out->rng_offset = L.off_rng;
   return SFL_OK;
 }
 
@@ -472,6 +560,8 @@ int sfl_create(const sfl_map_desc *map, const sfl_config *cfg, int device, void 
   int rc = make_layout(map, cfg, &L, &a_max);
   if (rc) return rc;
   if (cfg->shared_q && map->T > 64) return fail(SFL_E_ARG, "shared-table mode supports at most 64 trains%s");
+  if (cfg->shared_q && cfg->rng == SFL_RNG_REFERENCE)
+    return fail(SFL_E_ARG, "the reference's random stream (SFL_RNG_REFERENCE) has no shared-table mode: the reference keeps one table and one stream per learner%s");
   const int H = map->H, W = map->W, Hp = H + 2, Wp = W + 2, T = map->T, NT = map->NT, S = map->S, NP = map->NP, NA = map->NA;
   // every transition must lead to a rail cell inside the grid (flatland maps are consistent); the device relies on it
   for (int r = 0; r < H; r++) for (int cc = 0; cc < W; cc++) {
@@ -630,7 +720,7 @@ int sfl_set_phase_clock(void *ctx, int on) {
 int sfl_describe_launch(void *ctx, int mode, int traced, char *buf, int cap) {
   Ctx *c = (Ctx *)ctx;
   if (!c || !buf || cap < 1) return fail(SFL_E_ARG, "null argument%s");
-  const int trace = traced || mode == SFL_MODE_STEP || mode == SFL_MODE_REPLAY || c->phase_clock;
+  const int trace = traced || mode == SFL_MODE_STEP || mode == SFL_MODE_REPLAY || c->phase_clock || (mode == SFL_MODE_LEARN && c->cfg.rng);
   const int kind = trace ? K_FULL : (mode == SFL_MODE_GREEDY ? K_GREEDY : K_LEARN);
   LaunchPlan lp;
   if (plan_launch(c, kind, &lp)) return SFL_E_ARG;
@@ -650,7 +740,7 @@ int sfl_reset(void *ctx, int keep, void *stream) {
   if (!c) return fail(SFL_E_ARG, "null ctx%s");
   if (!c->bound) return fail(SFL_E_STATE, "sfl_bind first%s");
   DeviceGuard dg(c->device);
-  InitArgs ia; ia.L = c->L; ia.state = (char *)c->bufs.state; ia.n_envs = c->cfg.n_envs; ia.keep_q = keep & 1; ia.keep_ninter = (keep >> 1) & 1; ia.pad = 0;
+  InitArgs ia; ia.L = c->L; ia.state = (char *)c->bufs.state; ia.hp = (const sfl_hparams *)c->bufs.hparams; ia.n_envs = c->cfg.n_envs; ia.keep_q = keep & 1; ia.keep_ninter = (keep >> 1) & 1; ia.pad = 0;
   CK(dev_zero(c->bufs.counters, (size_t)c->cfg.n_envs * sizeof(sfl_env_counters), stream));
 #ifndef SFL_HOST_EMUL
   int grid = (c->cfg.n_envs + SFL_WARPS_PER_CTA - 1) / SFL_WARPS_PER_CTA;
@@ -715,10 +805,13 @@ int sfl_run(void *ctx, int mode, int max_ticks, void *stream) {
   ra.step_out = (sfl_step_rec *)c->bufs.step_out;
   if (c->cfg.shared_q) { ra.sq_q = (double *)c->bufs.shared_q; ra.sq_d = (long long *)c->bufs.shared_d; ra.sq_c = (int *)c->bufs.shared_c; }
   // recorded malfunction events replace the Philox draws in replay mode, and in greedy / step mode when a schedule was bound (ev_cap > 0)
-  ra.replay_ev = (mode != SFL_MODE_LEARN && c->cfg.ev_cap > 0) ? (const int *)c->bufs.replay_ev : nullptr;
-  // learn and greedy without traces run the two specialised kernels; replay, step and traced runs the full one
+  // -- and in learn mode with the reference's stream, whose learn runs use the full kernel
+  const int ref_learn = mode == SFL_MODE_LEARN && c->cfg.rng == SFL_RNG_REFERENCE;
+  ra.replay_ev = ((mode != SFL_MODE_LEARN || ref_learn) && c->cfg.ev_cap > 0) ? (const int *)c->bufs.replay_ev : nullptr;
+  // learn and greedy without traces run the two specialised kernels; replay, step, traced runs and learning on the
+  // reference's stream the full one
   ra.phase_clock = c->phase_clock;
-  const int trace = ra.trace_dec || ra.trace_tick || mode == SFL_MODE_STEP || mode == SFL_MODE_REPLAY || c->phase_clock;
+  const int trace = ra.trace_dec || ra.trace_tick || mode == SFL_MODE_STEP || mode == SFL_MODE_REPLAY || c->phase_clock || ref_learn;
   const int kind = trace ? K_FULL : (mode == SFL_MODE_GREEDY ? K_GREEDY : K_LEARN);
 #ifndef SFL_HOST_EMUL
   LaunchPlan lp;

@@ -83,6 +83,8 @@ SFL_FN int ffs64(unsigned long long v) { return __ffsll((long long)v) - 1; }
 SFL_FN int popc32(unsigned v) { return __popc(v); }
 SFL_FN double dmul(double a, double b) { return __dmul_rn(a, b); }
 SFL_FN double dadd(double a, double b) { return __dadd_rn(a, b); }
+SFL_FN double dfma(double a, double b, double c) { return __fma_rn(a, b, c); }
+SFL_FN unsigned long long mulhi64(unsigned long long a, unsigned long long b) { return __umul64hi(a, b); }
 template <class T> SFL_FN T ldg(const T *p) { return __ldg(p); }
 #else
 template <int G> struct Grp {
@@ -99,6 +101,8 @@ SFL_FN int ffs64(unsigned long long v) { return __builtin_ffsll((long long)v) - 
 SFL_FN int popc32(unsigned v) { return __builtin_popcount(v); }
 SFL_FN double dmul(double a, double b) { volatile double r = a * b; return r; }
 SFL_FN double dadd(double a, double b) { volatile double r = a + b; return r; }
+SFL_FN double dfma(double a, double b, double c) { return fma(a, b, c); }
+SFL_FN unsigned long long mulhi64(unsigned long long a, unsigned long long b) { return (unsigned long long)(((unsigned __int128)a * b) >> 64); }
 template <class T> SFL_FN T ldg(const T *p) { return *p; }
 #endif
 
@@ -161,7 +165,8 @@ struct DevMap {            // map constants (device pointers)
 
 struct Layout {            // byte offsets inside one env block
   int T, S, NP, NT, a_max, q_cap, q_stride, pend_cap;
-  unsigned off_tra, off_trb, off_pend, off_sem, off_rewards, off_sws, off_q, pad;
+  unsigned off_tra, off_trb, off_pend, off_sem, off_rewards, off_sws, off_q;
+  unsigned off_rng;          // the reference's random stream (Pcg, SFL_RNG_REFERENCE), right after the header; 0: Philox
   unsigned long long env_stride;
 };
 
@@ -338,6 +343,122 @@ SFL_FN U4 philox4x32(unsigned c0, unsigned c1, unsigned c2, unsigned c3, unsigne
   }
   U4 r = {c0, c1, c2, c3};
   return r;
+}
+
+// ------------------------------------------------------------------------------------------------ the reference's stream
+// SFL_RNG_REFERENCE: numpy's Generator(PCG64) exactly as distr_q.py draws from it -- rng = np.random.default_rng(seed) at
+// the start of learn() (:269); per decision rng.random() < epsilon; on exploration Discrete.seed(int(rng.integers(0,
+// 2**31 - 1))) and Discrete.sample(mask) = Generator(PCG64(SeedSequence(sd))).choice(where(mask)) (:315-317).  Integer
+// arithmetic only (numpy's bit_generator.pyx, _pcg64.pyx, pcg64.h, distributions.c).
+struct Pcg {                 // numpy's pcg64_state: 128-bit state and increment, the carried half-word of next_uint32
+  unsigned long long s_hi, s_lo, i_hi, i_lo;
+  unsigned has32, u32, pad0, pad1;
+};
+#define SFL_PCG_BYTES 48
+
+SFL_FN void pcg_step(Pcg &g) {        // state = state * 0x2360ED051FC65DA44385DF649FCCF645 + inc  (mod 2^128)
+  const unsigned long long M_HI = 0x2360ED051FC65DA4ull, M_LO = 0x4385DF649FCCF645ull;
+  const unsigned long long lo = g.s_lo * M_LO;
+  const unsigned long long hi = mulhi64(g.s_lo, M_LO) + g.s_lo * M_HI + g.s_hi * M_LO;
+  g.s_lo = lo + g.i_lo;
+  g.s_hi = hi + g.i_hi + (g.s_lo < lo ? 1ull : 0ull);
+}
+SFL_FN unsigned long long pcg_next64(Pcg &g) {     // step, then XSL-RR of the new state
+  pcg_step(g);
+  const unsigned long long x = g.s_hi ^ g.s_lo;
+  const unsigned r = (unsigned)(g.s_hi >> 58);
+  return (x >> r) | (x << ((64u - r) & 63u));
+}
+SFL_FN double pcg_double(Pcg &g) { return (double)(pcg_next64(g) >> 11) * (1.0 / 9007199254740992.0); }   // random()
+SFL_FN unsigned pcg_next32(Pcg &g) {             // a 64-bit draw serves two calls: low half now, high half carried
+  if (g.has32) { g.has32 = 0; return g.u32; }
+  const unsigned long long v = pcg_next64(g);
+  g.has32 = 1; g.u32 = (unsigned)(v >> 32);
+  return (unsigned)v;
+}
+// Generator.integers(0, ex) for 1 <= ex <= 2^32: random_bounded_uint64_fill, Lemire's method on 32-bit draws
+SFL_FN unsigned pcg_bounded(Pcg &g, unsigned long long ex) {
+  if (ex <= 1ull) return 0u;                     // one value: no draw
+  if (ex == 0x100000000ull) return pcg_next32(g);
+  const unsigned e = (unsigned)ex;
+  unsigned long long m = (unsigned long long)pcg_next32(g) * e;
+  if ((unsigned)m < e) {
+    const unsigned threshold = (0u - e) % e;     // (2^32 - ex) mod ex
+    SFL_NU
+    while ((unsigned)m < threshold) m = (unsigned long long)pcg_next32(g) * e;
+  }
+  return (unsigned)(m >> 32);
+}
+// PCG64(SeedSequence(seed)) = np.random.default_rng(seed): the seed's little-endian 32-bit words (one below 2^32) hashed into
+// a 4-word pool, cross-mixed, expanded to 8 words = 4 uint64 {initstate hi, lo, initseq hi, lo}; then pcg's srandom
+SFL_FN unsigned ss_hashmix(unsigned v, unsigned &hc) { v ^= hc; hc *= 0x931e8875u; v *= hc; return v ^ (v >> 16); }
+SFL_FN unsigned ss_mix(unsigned x, unsigned y) { const unsigned r = 0xca01f9ddu * x - 0x4973f715u * y; return r ^ (r >> 16); }
+SFL_FN Pcg pcg_seed(unsigned long long seed) {
+  unsigned hc = 0x43b0d7e5u, pool[4], w[8];
+  pool[0] = ss_hashmix((unsigned)seed, hc);
+  pool[1] = ss_hashmix((unsigned)(seed >> 32), hc);   // a seed below 2^32 has one word: the pool is padded with 0 alike
+  pool[2] = ss_hashmix(0u, hc);
+  pool[3] = ss_hashmix(0u, hc);
+  SFL_UA
+  for (int s = 0; s < 4; s++) {
+    SFL_UA
+    for (int d = 0; d < 4; d++) if (s != d) pool[d] = ss_mix(pool[d], ss_hashmix(pool[s], hc));
+  }
+  hc = 0x8b51f9ddu;
+  SFL_UA
+  for (int i = 0; i < 8; i++) { unsigned v = pool[i & 3] ^ hc; hc *= 0x58f38dedu; v *= hc; w[i] = v ^ (v >> 16); }
+  const unsigned long long v0 = w[0] | (unsigned long long)w[1] << 32, v1 = w[2] | (unsigned long long)w[3] << 32;
+  const unsigned long long v2 = w[4] | (unsigned long long)w[5] << 32, v3 = w[6] | (unsigned long long)w[7] << 32;
+  Pcg g;
+  g.s_hi = 0ull; g.s_lo = 0ull; g.i_hi = (v2 << 1) | (v3 >> 63); g.i_lo = (v3 << 1) | 1ull;     // inc = initseq << 1 | 1
+  g.has32 = 0u; g.u32 = 0u; g.pad0 = 0u; g.pad1 = 0u;
+  pcg_step(g);
+  const unsigned long long lo = g.s_lo + v1;                                                     // state += initstate
+  g.s_hi += v0 + (lo < v1 ? 1ull : 0ull); g.s_lo = lo;
+  pcg_step(g);
+  return g;
+}
+
+// decay ** n rounded to nearest: binary exponentiation in double-double (relative error about 2^-100 for n < 2^31, far
+// inside half an ulp), the pair rounded by its renormalisation.  The pairs are kept scaled by exact powers of two (2^-er,
+// 2^-eb) so that their low words never go subnormal; decay is in [0, 1].
+SFL_FN void dd_mul(double &ah, double &al, double bh, double bl) {
+  const double p = dmul(ah, bh);
+  const double t = dadd(dfma(ah, bh, -p), dadd(dmul(ah, bl), dmul(al, bh)));
+  const double s = dadd(p, t);
+  al = dadd(t, -dadd(s, -p)); ah = s;
+}
+SFL_FN void dd_rescale(double &h, double &l, long long &e) {
+  if (h < 0x1p-400 && e < 4000) { h = dmul(h, 0x1p400); l = dmul(l, 0x1p400); e += 400; }
+}
+SFL_FN double pow_dd(double b, int n) {
+  if (b == 0.0) return n == 0 ? 1.0 : 0.0;
+  double rh = 1.0, rl = 0.0, bh = b, bl = 0.0;
+  long long er = 0, eb = 0;
+  SFL_NU
+  for (; n > 0; n >>= 1) {
+    if (n & 1) { dd_mul(rh, rl, bh, bl); er += eb; dd_rescale(rh, rl, er); }
+    if (n > 1) { dd_mul(bh, bl, bh, bl); eb = eb < 4000 ? 2 * eb : eb; dd_rescale(bh, bl, eb); }
+  }
+  return er >= 4000 ? 0.0 : ldexp(rh, -(int)er);
+}
+// distr_q.py:315 `rng.random() < epsilon * epsilon_decay_rate ** n`.  eps_pow is the kernel's running product of the decay
+// (SwS.eps_pow: one rounding per interaction, relative error below (n + 1) 2^-53; pow's is below one ulp): only a draw
+// inside that margin of the product recomputes the power exactly -- practically never, but it makes the comparison exact.
+SFL_FN int eps_explore(double u, double epsilon, double decay, int n, double eps_pow) {
+  const double eps = dmul(epsilon, eps_pow);
+  const double tol = dadd(dmul(eps, (double)(n + 4) * 0x1p-52), 0x1p-1000);
+  const double gap = dadd(u, -eps);
+  if (gap > tol || -gap > tol) return u < eps;
+  return u < dmul(epsilon, pow_dd(decay, n));
+}
+// the exploring branch (distr_q.py:316-317): a new generator from the learner's stream, its choice among the allowed actions
+SFL_FN int pcg_explore_action(Pcg &g, int mask) {
+  Pcg x = pcg_seed(pcg_bounded(g, 0x7FFFFFFFull));
+  unsigned mm = (unsigned)mask;
+  SFL_NU
+  for (unsigned pick = pcg_bounded(x, (unsigned long long)popc32(mm)); pick > 0; pick--) mm &= mm - 1;
+  return ffs64(mm);
 }
 
 // ------------------------------------------------------------------------------------------------ F1
@@ -706,7 +827,11 @@ SFL_FN void decide(SFL_K, Env e, const Hp hp, int env_id, int t, const int semb_
   const int s_early = tb.y & 0xFFFF;
   const int reward_in = e.rewards()[s_early * c_L.T + t];                         // last(): _cumulative_rewards[agent][train]
   double eps_pow = 1.0;
-  if (mode == SFL_MODE_LEARN) eps_pow = e.sws()[s_early].eps_pow;
+  int ninter = 0;
+  if (mode == SFL_MODE_LEARN) {
+    eps_pow = e.sws()[s_early].eps_pow;
+    if (KIND == K_FULL && c_L.off_rng) ninter = e.sws()[s_early].ninter;
+  }
   int2 pend0 = make_int2(0, -1);
   if (learning && ((tb.y >> 16) & 0xFF)) pend0 = e.pend()[t * c_L.pend_cap];
   const Obs ob = observe(K, e, t, now, ta, tb, semb_pre);
@@ -740,6 +865,12 @@ SFL_FN void decide(SFL_K, Env e, const Hp hp, int env_id, int t, const int semb_
       my_row = q_row(K, e, hp, key);
       if (max_action(my_row, A, mask) != action) h->err |= SFL_ERR_REPLAY_DIVERGED;
     }
+  } else if (KIND == K_FULL && mode == SFL_MODE_LEARN && c_L.off_rng) {
+    // the reference's stream: one random() per decision, exploit included; the exploring branch draws its seed from it
+    Pcg *gp = (Pcg *)(hot_ptr(e.hot) + c_L.off_rng);
+    Pcg g = *gp;
+    if (eps_explore(pcg_double(g), hp->epsilon, hp->epsilon_decay_rate, ninter, eps_pow)) action = pcg_explore_action(g, mask);
+    *gp = g;
   } else if (mode == SFL_MODE_LEARN) {
     double eps = dmul(hp->epsilon, eps_pow);
     // one Philox4x32-10 block per PAIR of decisions: counter (step_counter >> 1, episode, 0x5F1, 0), key = env seed; the
@@ -933,7 +1064,7 @@ SFL_FN void env_tick(SFL_K, Env e, Scratch sc, const Hp hp, int env_id, const Gr
   const int Tw = c_L.T;                                                  // warp-uniform loop bound
   const int T = live ? Tw : 0;
   const int now = R.elapsed + 1;                                         // flatland: _elapsed_steps += 1 first
-  const int replay_ev = KIND != K_LEARN && c_ra.replay_ev != 0;          // recorded events never replace the draws in learn mode
+  const int replay_ev = KIND != K_LEARN && c_ra.replay_ev != 0;          // never in the learn kernel (sfl_run binds events for learn only with the reference stream)
   const unsigned thr = live ? hp->malf_threshold : 0u;
   if (replay_ev) {
     SFL_NU
