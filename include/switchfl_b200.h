@@ -24,7 +24,7 @@
 extern "C" {
 #endif
 
-#define SFL_ABI_VERSION 8
+#define SFL_ABI_VERSION 9
 
 enum {
   SFL_OK = 0,
@@ -92,6 +92,7 @@ typedef struct sfl_config {
                                    of this context reads ONE dense Q table and accumulates its TD steps into a delta
                                    buffer; sfl_shared_q_apply folds the mean step into the table (see DESIGN.md)  */
   int32_t rng;                  /* epsilon-greedy stream of SFL_MODE_LEARN: SFL_RNG_PHILOX (0) or SFL_RNG_REFERENCE (1)      */
+  int32_t malf_rng;             /* malfunction draws: SFL_MALF_PHILOX (0) or SFL_MALF_REFERENCE (1)                           */
 } sfl_config;
 
 /* sfl_config.rng.
@@ -111,10 +112,22 @@ typedef struct sfl_config {
  *   The stream's state takes 48 bytes of every env block, after the header; with SFL_RNG_PHILOX it takes none.      */
 enum { SFL_RNG_PHILOX = 0, SFL_RNG_REFERENCE = 1 };
 
+/* sfl_config.malf_rng.
+ * SFL_MALF_PHILOX: the two-stage Philox malfunction draw (sfl_hparams.malf_threshold, DESIGN.md section 4), unless a
+ *   schedule is bound (ev_cap > 0: replay, greedy and step mode, and learn mode with SFL_RNG_REFERENCE).
+ * SFL_MALF_REFERENCE: flatland's own stream, so that a seeded run has the reference's malfunctions.  rail_env.reset
+ *   (random_seed=seed) creates np_random = np.random.RandomState(seed) at every episode (switch_env.py:99); each tick
+ *   1 .. max_episode_steps, for every train in handle order, ParamMalfunctionGen draws rand() < 1 - exp(-rate) and, on a
+ *   hit, randint(min_duration, max_duration + 1) + 1 steps.  No draw depends on the actions, so the schedule is a function
+ *   of (seed, rate, min, max, T, max_episode_steps), the same in every episode.  sfl_malf_schedule writes it into replay_ev;
+ *   every mode then applies it (learn mode on the full kernel), an event only while the train's counter is 0.  Needs
+ *   ev_cap >= 1; not with shared_q.                                                                                    */
+enum { SFL_MALF_PHILOX = 0, SFL_MALF_REFERENCE = 1 };
+
 /* DistrQLearning.__init__ arguments (distr_q.py:32) + MalfunctionParameters (main.py:28-33), per env */
 typedef struct sfl_hparams {
   double gamma, epsilon, epsilon_decay_rate, lr, lr_decay_rate, default_q;
-  uint64_t seed;                /* Philox key                                                         */
+  uint64_t seed;                /* Philox key; the reference's seed (SFL_RNG_REFERENCE, SFL_MALF_REFERENCE) */
   uint32_t malf_threshold;      /* floor((1 - exp(-rate)) * 2^32), 0 = no malfunctions                */
   int32_t malf_min, malf_max;   /* duration = min + U{0..max-min} + 1                                 */
   int32_t episodes;             /* halt after this many episodes since sfl_reset (<0: never)          */
@@ -220,6 +233,16 @@ int sfl_kat_q_update(const double *operands, int32_t n, double *out, int device)
 int sfl_kat_pcg64(const uint64_t *gens, const uint64_t *codes, int32_t n, int32_t n_codes, uint64_t *out, int device);
 int sfl_kat_explore(const double *rows, int32_t n, int32_t *out, int device);
 
+/* SFL_MALF_REFERENCE: flatland's malfunction schedule of every environment, generated ON THE DEVICE (numpy's MT19937:
+ * init_genrand, twist, tempering; rand() from two words; legacy randint by masked rejection on 32-bit words) into the
+ * bound replay_ev: the events (tick, train, duration) drawn for ticks 1 .. max_episode_steps in tick order, -1 after the
+ * last.  Seed, min_duration and max_duration come from the bound sfl_hparams (seed.. malf_max; malf_threshold is not
+ * used); hit_below[n_envs] (host) = ceil(p * 2^53) with p = 1 - exp(-rate) (0 for rate <= 0), so that a draw hits iff its
+ * 53-bit integer k < hit_below.  *max_events = the largest number of events of an environment.  SFL_E_ARG for a seed
+ * RandomState refuses (not below 2^32) or min_duration > max_duration; SFL_E_NOMEM when a schedule has more than ev_cap
+ * events (nothing is truncated).  Synchronises `stream`.                                                            */
+int sfl_malf_schedule(void *ctx, const uint64_t *hit_below, int32_t *max_events, void *stream);
+
 int sfl_abi_version(void);
 const char *sfl_last_error(void);
 
@@ -228,8 +251,8 @@ const char *sfl_last_error(void);
 int sfl_query_sizes(const sfl_map_desc *map, const sfl_config *cfg, sfl_sizes *out);
 
 /* replaces ASyncSwitchEnv(rail_env, ...) + DistrQLearning(env, ...)   (main.py:51-60).  T must be in 1..128;
- * shared-table mode (sfl_config.shared_q) takes at most 64 trains and not SFL_RNG_REFERENCE (the reference has no shared
- * table, and its learner one stream).                                                                              */
+ * shared-table mode (sfl_config.shared_q) takes at most 64 trains and neither SFL_RNG_REFERENCE nor SFL_MALF_REFERENCE
+ * (the reference has no shared table, and its learner one stream).  SFL_MALF_REFERENCE needs ev_cap >= 1.            */
 int sfl_create(const sfl_map_desc *map, const sfl_config *cfg, int device, void **ctx);
 int sfl_destroy(void *ctx);                       /* env.close() (switch_env.py, called at distr_q.py:241, 379) + garbage collection */
 int sfl_bind(void *ctx, const sfl_buffers *bufs); /* hand over the caller-owned device buffers sized by sfl_query_sizes            */
@@ -258,7 +281,7 @@ int sfl_set_roomy(void *ctx, int roomy);
 int sfl_set_phase_clock(void *ctx, int on);
 /* Which kernel instantiation and launch configuration sfl_run(mode) would use now (traced != 0: with decision / tick
  * traces), as text: "k_run<G=..,KIND=..,TH=..,SQ=..,ONE=..,ROOMY=..> grid=.. block=.. smem=..", with ",NW=2" after ROOMY
- * on maps with more than 64 trains (two words per train set); learn with SFL_RNG_REFERENCE is KIND=full.  No counterpart in the
+ * on maps with more than 64 trains (two words per train set); learn with SFL_RNG_REFERENCE or SFL_MALF_REFERENCE is KIND=full.  No counterpart in the
  * reference; it lets the parity tests name -- and force, with sfl_set_lanes / sfl_set_roomy -- exactly the
  * instantiations the benchmark launches.  Needs no bound buffers.                                                  */
 int sfl_describe_launch(void *ctx, int mode, int traced, char *buf, int cap);

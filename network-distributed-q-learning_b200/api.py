@@ -101,20 +101,24 @@ class ASyncSwitchEnv:
 
     def __init__(self, rail_env: RailEnv, max_steps: int = 200, render_mode=None, observer=None, seed=None,
                  n_envs: int = 1, device: str = "cuda:0", q_cap: Optional[int] = None, ep_cap: int = 128, shared_q: bool = False,
-                 phase_timers: bool = False, rng: str = "philox", _engine_kwargs=None):
+                 phase_timers: bool = False, rng: str = "philox", malfunction_rng: str = "philox", _engine_kwargs=None):
         """``phase_timers``: run the instrumented kernel (per-phase cycle counters, a few per cent slower) so that all seven
         wall-clock accumulators of switch_env.py:67-73 are filled; without it the fused kernel books its whole time on
         ``step_time`` (and resets on ``reset_total_time``).
         ``rng="reference"``: learn() draws its epsilon-greedy choices from the reference's own numpy stream
         (``np.random.default_rng(seed)`` per learn() call, distr_q.py:269, 315-317), so environment i with seed s makes the
-        decisions of the reference's learn() with seed s (malfunction-free maps; flatland's malfunction RNG is not
-        reproduced).  "philox" (default): the faster counter-based stream."""
+        decisions of the reference's learn() with seed s -- on maps with malfunctions together with
+        ``malfunction_rng="reference"``.  "philox" (default): the faster counter-based stream.
+        ``malfunction_rng="reference"``: the malfunctions come from flatland's own stream, ``np.random.RandomState(seed)``
+        created by every episode's ``rail_env.reset(random_seed=seed)`` (switch_env.py:99): environment i with seed s has
+        the malfunctions of the reference's episodes with seed s, in learn(), test() and the AEC protocol (whose
+        ``reset()`` then needs an explicit seed).  "philox" (default): the counter-based draws."""
         self.rail_env = rail_env
         self.max_steps = max_steps
         self.render_mode = render_mode
         self.seed = seed
         self.n_envs = int(n_envs)
-        kw = dict(act_cap=1, shared_q=shared_q, phase_clock=bool(phase_timers), rng=rng)
+        kw = dict(act_cap=1, shared_q=shared_q, phase_clock=bool(phase_timers), rng=rng, malfunction_rng=malfunction_rng)
         kw.update(_engine_kwargs or {})
         self.rail_map = RailMap(rail_env.fixture, device_bfs=self.engine_cls.bfs_device(device))
         self.possible_agents = self.rail_map.tab.switch_names()          # switch_env.py:51-52
@@ -151,6 +155,9 @@ class ASyncSwitchEnv:
     # ``view`` (0) and need n_envs == 1 for ``step``.
     def reset(self, seed=None, options=None):
         eng = self.engine
+        if seed is None and eng.malfunction_rng == "reference":
+            # the reference would continue flatland's stream (or seed it from entropy), which this mode does not model
+            raise ValueError('reset() with malfunction_rng="reference" needs an explicit seed: reset(seed=...)')
         if seed is not None:
             self.seed = seed
         base = 0 if self.seed is None else int(self.seed)

@@ -18,10 +18,12 @@ from . import railmap
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "csrc", "libswitchfl_b200.so")
 
-ABI_VERSION = 8
+ABI_VERSION = 9
 MODE_LEARN, MODE_GREEDY, MODE_REPLAY, MODE_STEP = 0, 1, 2, 3
 RNG_PHILOX, RNG_REFERENCE = 0, 1
 RNG_NAMES = {"philox": RNG_PHILOX, "reference": RNG_REFERENCE}
+MALF_PHILOX, MALF_REFERENCE = 0, 1
+MALF_NAMES = {"philox": MALF_PHILOX, "reference": MALF_REFERENCE}
 ERR_NO_TRAIN_AT_SWITCH = 1
 ERR_BITS = {1: "no train at active switch (observer.py:294-307)", 2: "infinite distance to target (observer.py:35-36)",
             4: "per-env Q table full (raise q_cap)", 8: "pending-update list full (raise pend_cap)",
@@ -44,7 +46,7 @@ class MapDesc(C.Structure):
 
 class Config(C.Structure):
     _fields_ = [(n, C.c_int32) for n in ("n_envs", "q_cap", "pend_cap", "max_steps", "dec_cap", "tick_cap", "ep_cap",
-                                         "act_cap", "ev_cap", "trace_sem", "shared_q", "rng")]
+                                         "act_cap", "ev_cap", "trace_sem", "shared_q", "rng", "malf_rng")]
 
 
 class Sizes(C.Structure):
@@ -114,6 +116,7 @@ def load_library(path: Optional[str] = None) -> C.CDLL:
     lib.sfl_kat_q_update.argtypes = [C.POINTER(C.c_double), C.c_int32, C.POINTER(C.c_double), C.c_int]
     lib.sfl_kat_pcg64.argtypes = [C.POINTER(C.c_uint64), C.POINTER(C.c_uint64), C.c_int32, C.c_int32, C.POINTER(C.c_uint64), C.c_int]
     lib.sfl_kat_explore.argtypes = [C.POINTER(C.c_double), C.c_int32, C.POINTER(C.c_int32), C.c_int]
+    lib.sfl_malf_schedule.argtypes = [C.c_void_p, C.POINTER(C.c_uint64), C.POINTER(C.c_int32), C.c_void_p]
     lib.sfl_distance_map.argtypes = [_u16p, C.c_int32, C.c_int32, _i32p, C.c_int32, _i32p, C.c_int]
     if lib.sfl_abi_version() != ABI_VERSION:
         raise RuntimeError("switchfl_b200 ABI version mismatch")
@@ -189,6 +192,25 @@ def malf_threshold(rate: float) -> int:
     if rate <= 0:
         return 0
     return min(int((1.0 - math.exp(-rate)) * 4294967296.0), 0xFFFFFFFF)
+
+
+def malf_prob(rate: float) -> float:
+    """flatland's malfunction probability per (train, tick), computed as ParamMalfunctionGen.prob does."""
+    return 0.0 if rate <= 0 else 1.0 - math.exp(-rate)
+
+
+def malf_hit_below(rate: float) -> int:
+    """ceil(p * 2^53) for p = malf_prob(rate): a draw rand() = k * 2^-53 hits iff the integer k is below it
+    (SFL_MALF_REFERENCE)."""
+    return math.ceil(malf_prob(rate) * 2.0 ** 53)
+
+
+def reference_ev_cap(fixture: dict) -> int:
+    """Events per environment that flatland's malfunction schedule of this map fits in: the mean of the binomial
+    T * max_episode_steps draws plus a wide margin (16 standard deviations + 64), at most one per draw."""
+    n = len(fixture["init_dir"]) * int(fixture["max_episode_steps"])
+    p = malf_prob(float(fixture["malfunction_rate"]))
+    return max(1, min(n, int(math.ceil(n * p + 16.0 * math.sqrt(n * p * (1.0 - p)))) + 64))
 
 
 def malf_thr2(threshold: int) -> int:
@@ -292,14 +314,23 @@ class Engine:
                  max_steps: int = 100_000, dec_cap: int = 0, tick_cap: int = 0, ep_cap: int = 64, act_cap: int = 0,
                  ev_cap: int = 0, trace_sem: bool = False, lanes: Optional[int] = None, shared_q: bool = False,
                  cta_warps: Optional[int] = None, roomy: Optional[bool] = None, phase_clock: bool = False, bind: bool = True,
-                 rng: str = "philox"):
+                 rng: str = "philox", malfunction_rng: str = "philox"):
         """``bind=False`` creates the context only (no device buffers): enough for ``describe_launch``.
         ``rng``: the epsilon-greedy stream of learn mode -- "philox" (the specialised learn kernels) or "reference" (numpy's
         PCG64 stream of the reference learner, seeded per environment from its seed at every reset that restarts the
-        interaction counters: a seeded learn() makes the reference's decisions; runs on the full kernel)."""
+        interaction counters: a seeded learn() makes the reference's decisions; runs on the full kernel).
+        ``malfunction_rng``: "philox" (the counter-based draws) or "reference" (flatland's ``RandomState(seed)`` stream:
+        every environment's malfunction schedule is generated on the device from its seed, rate and durations by
+        ``reset()``, and applied in every mode; learn runs on the full kernel).  With "reference" and ``ev_cap=0`` the
+        schedule's capacity is sized from the fixture (``reference_ev_cap``)."""
         if rng not in RNG_NAMES:
             raise ValueError(f"rng must be one of {sorted(RNG_NAMES)}, not {rng!r}")
+        if malfunction_rng not in MALF_NAMES:
+            raise ValueError(f"malfunction_rng must be one of {sorted(MALF_NAMES)}, not {malfunction_rng!r}")
         self.rng = rng
+        self.malfunction_rng = malfunction_rng
+        if malfunction_rng == "reference" and not ev_cap:
+            ev_cap = reference_ev_cap(rail_map.fixture)
         import torch
         self.torch = torch
         self.map = rail_map
@@ -307,7 +338,7 @@ class Engine:
         self.lib, self.device, dev_index = self._open(device)
         self.cfg = Config(n_envs=self.n_envs, q_cap=q_cap, pend_cap=pend_cap, max_steps=max_steps, dec_cap=dec_cap,
                           tick_cap=tick_cap, ep_cap=ep_cap, act_cap=act_cap, ev_cap=ev_cap, trace_sem=int(trace_sem),
-                          shared_q=int(shared_q), rng=RNG_NAMES[rng])
+                          shared_q=int(shared_q), rng=RNG_NAMES[rng], malf_rng=MALF_NAMES[malfunction_rng])
         self.shared_q = bool(shared_q)
         self.sizes = Sizes()
         self._ck(self.lib.sfl_query_sizes(C.byref(rail_map.desc), C.byref(self.cfg), C.byref(self.sizes)))
@@ -323,6 +354,9 @@ class Engine:
             self._ck(self.lib.sfl_set_phase_clock(self.ctx, 1))
         self.phase_clock = bool(phase_clock)
         self.hparams = np.zeros(self.n_envs, HPARAMS_DT)
+        self.malfunction_rate = float(rail_map.fixture["malfunction_rate"])
+        self._malf_key = None                             # (seeds, rate, min, max) of the generated schedules
+        self.max_malfunction_events = 0                   # events of the longest generated schedule
         self._pinned = {}
         self._pinned_ev = {}
         self.buf = {}
@@ -419,6 +453,7 @@ class Engine:
             hp[k] = v
         hp["seed"] = np.arange(self.n_envs, dtype=np.uint64) if seeds is None else np.asarray(seeds, np.uint64)
         rate = fx["malfunction_rate"] if malfunction_rate is None else malfunction_rate
+        self.malfunction_rate = float(rate)
         hp["malf_threshold"] = malf_threshold(float(rate))
         hp["malf_thr2"] = malf_thr2(int(hp["malf_threshold"][0]))
         hp["malf_min"] = fx["min_duration"] if min_duration is None else min_duration
@@ -426,7 +461,36 @@ class Engine:
         self._upload("hparams", hp)
 
     def reset(self, keep_q: bool = False, keep_interactions: bool = False):
+        """``malfunction_rng="reference"``: first (re)generates the malfunction schedules when the seeds, the rate or the
+        durations changed since they were last generated -- every path (learn(), learn_chunk(), test(), the AEC reset)
+        goes through here."""
+        if self.malfunction_rng == "reference":
+            self._malf_generate()
         self._ck(self.lib.sfl_reset(self.ctx, int(keep_q) | (int(keep_interactions) << 1), self._stream()))
+
+    def _malf_generate(self):
+        hp = self.hparams
+        key = (hp["seed"].tobytes(), self.malfunction_rate, hp["malf_min"].tobytes(), hp["malf_max"].tobytes())
+        if key == self._malf_key:
+            return
+        hit = np.full(self.n_envs, malf_hit_below(self.malfunction_rate), np.uint64)
+        n = C.c_int32()
+        self._malf_key = None
+        rc = self.lib.sfl_malf_schedule(self.ctx, hit.ctypes.data_as(C.POINTER(C.c_uint64)), C.byref(n), self._stream())
+        self.max_malfunction_events = n.value             # also when the schedules do not fit: the ev_cap they need
+        self._ck(rc)
+        self._malf_key = key
+
+    def malfunction_schedule(self, env: int) -> np.ndarray:
+        """``malfunction_rng="reference"``: environment ``env``'s schedule, int32 rows (tick, train, duration) in tick order --
+        every malfunction flatland draws for ticks 1 .. max_episode_steps; one is applied when the train's counter is 0."""
+        if self.malfunction_rng != "reference":
+            raise RuntimeError('malfunction_schedule() needs Engine(malfunction_rng="reference")')
+        self._malf_generate()
+        cap = self.cfg.ev_cap
+        ev = self.buf["replay_ev"][int(env) * cap * 12:(int(env) + 1) * cap * 12].cpu().numpy().view(np.int32).reshape(cap, 3)
+        end = np.nonzero(ev[:, 0] < 0)[0]
+        return ev[:int(end[0]) if len(end) else cap].copy()
 
     @property
     def lanes(self) -> int:
@@ -455,13 +519,16 @@ class Engine:
         self._ck(self.lib.sfl_run(self.ctx, int(mode), int(max_ticks), self._stream()))
 
     def set_replay(self, actions: Optional[Sequence[Sequence[int]]], events: Optional[Sequence[np.ndarray]] = None):
-        """actions[i]: the recorded action stream of env i; events[i]: int array [(tick, train, duration)]."""
+        """actions[i]: the recorded action stream of env i; events[i]: int array [(tick, train, duration)].  With
+        ``malfunction_rng="reference"`` the schedule comes from the seeds alone: ``events`` must be None."""
+        if self.malfunction_rng == "reference" and events is not None:
+            raise ValueError('set_replay(events=...) with malfunction_rng="reference": the schedule is generated from the seeds')
         if actions is not None:
             a = np.full((self.n_envs, self.cfg.act_cap), -1, np.int8)
             for i, s in enumerate(actions):
                 a[i, :len(s)] = s
             self._upload("replay_act", a)
-        if self.cfg.ev_cap:
+        if self.cfg.ev_cap and self.malfunction_rng != "reference":
             ev = np.full((self.n_envs, self.cfg.ev_cap, 3), -1, np.int32)
             for i, e in enumerate(events or []):
                 e = np.asarray(e, np.int32).reshape(-1, 3)

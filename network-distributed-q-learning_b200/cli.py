@@ -7,10 +7,11 @@
 ``config.ini`` keeps the reference's sections and keys (hyperparam_tuning.py:51-78): MISC{random_seed, out_dir,
 checkpoint_freq, exploit_freq}, ENV{width, height, max_num_cities, max_rails_between_cities, max_rail_pairs_in_city,
 number_of_agents, malfunction_rate, min_duration, max_duration}, MODEL{gamma, epsilon, epsilon_decay_rate, lr,
-lr_decay_rate, default_q, num_episodes}.  Four optional keys are new: ENV.fixture (a map fixture .npz recorded from
+lr_decay_rate, default_q, num_episodes}.  Five optional keys are new: ENV.fixture (a map fixture .npz recorded from
 flatland, see tools/record_flatland_fixture.py), MISC.n_envs (lockstep replicas with seeds random_seed + i),
-MISC.q_cap (Q hash rows per environment; default: sized from the map, see ``default_q_cap``) and MISC.rng (``philox``,
-the default, or ``reference``: the reference's own numpy epsilon-greedy stream, see ``ASyncSwitchEnv``).
+MISC.q_cap (Q hash rows per environment; default: sized from the map, see ``default_q_cap``), MISC.rng (``philox``,
+the default, or ``reference``: the reference's own numpy epsilon-greedy stream, see ``ASyncSwitchEnv``) and
+MISC.malfunction_rng (``philox``, the default, or ``reference``: flatland's own malfunction stream of the seed).
 Without ENV.fixture the map comes from the synthetic generator with the same size / train count / seed, because
 flatland's sparse_rail_generator cannot run here (mapgen.py).
 """
@@ -54,7 +55,7 @@ def default_device() -> str:
 
 
 def launch_experiment(config_path: str, device: Optional[str] = None, q_cap: Optional[int] = None, env_cls=ASyncSwitchEnv,
-                      _engine_kwargs=None, rng: Optional[str] = None) -> DistrQLearning:
+                      _engine_kwargs=None, rng: Optional[str] = None, malfunction_rng: Optional[str] = None) -> DistrQLearning:
     """main.py:13-78."""
     start_time = time.time()
     device = device or default_device()
@@ -69,8 +70,9 @@ def launch_experiment(config_path: str, device: Optional[str] = None, q_cap: Opt
     if q_cap is None and misc.get("q_cap"):
         q_cap = int(misc["q_cap"])
     rng = rng or misc.get("rng", "philox")
+    malfunction_rng = malfunction_rng or misc.get("malfunction_rng", "philox")
     env = env_cls(rail_env, render_mode=None, max_steps=100_000, n_envs=int(misc.get("n_envs", 1)), device=device, q_cap=q_cap,
-                  rng=rng, _engine_kwargs=_engine_kwargs)
+                  rng=rng, malfunction_rng=malfunction_rng, _engine_kwargs=_engine_kwargs)
     model = DistrQLearning(env=env, gamma=float(mdl["gamma"]), epsilon=float(mdl["epsilon"]),
                            epsilon_decay_rate=float(mdl["epsilon_decay_rate"]), lr=float(mdl["lr"]),
                            lr_decay_rate=float(mdl["lr_decay_rate"]), default_q=float(mdl["default_q"]), seed=seed)
@@ -95,12 +97,13 @@ def launch_experiment(config_path: str, device: Optional[str] = None, q_cap: Opt
 def launch_grid(hyperparams: Dict[str, Sequence[float]], random_seeds: Sequence[int], out_dir: str, env_section: Dict[str, object],
                 num_episodes: int, checkpoint_freq: int, exploit_freq: Optional[int], gamma: float = 1.0, default_q: float = 0.0,
                 device: Optional[str] = None, q_cap: Optional[int] = None, env_cls=ASyncSwitchEnv, _engine_kwargs=None,
-                rng: str = "philox") -> List[str]:
+                rng: str = "philox", malfunction_rng: str = "philox") -> List[str]:
     """hyperparam_tuning.py:42-91: every (grid point, seed) pair gets ``out_dir/exp_i/seed_j/`` with its config.ini
     and the reference's output files.  One seed = one map (the generators are seeded with it), so each seed is ONE
     batched engine whose environments are the grid points; under torchrun the seeds are sharded over the ranks.
     With ``rng="reference"`` every environment learns on the reference's stream of its seed: environment i of a seed is
-    the reference's main.py run for that (grid point, seed)."""
+    the reference's main.py run for that (grid point, seed) -- on maps with malfunctions together with
+    ``malfunction_rng="reference"`` (flatland's own malfunction stream of the seed)."""
     names = list(hyperparams)
     points = [dict(zip(names, v)) for v in product(*[hyperparams[n] for n in names])]
     rank, world_size, _ = sharding.world()
@@ -114,7 +117,7 @@ def launch_grid(hyperparams: Dict[str, Sequence[float]], random_seeds: Sequence[
         mf = ParamMalfunctionGen(MalfunctionParameters(float(env_section.get("malfunction_rate", 0.0)),
                                                        int(env_section.get("min_duration", 0)), int(env_section.get("max_duration", 0))))
         env = env_cls(RailEnv(fx, malfunction_generator=mf), render_mode=None, max_steps=100_000, n_envs=len(points),
-                      device=device, q_cap=q_cap, rng=rng, _engine_kwargs=_engine_kwargs)
+                      device=device, q_cap=q_cap, rng=rng, malfunction_rng=malfunction_rng, _engine_kwargs=_engine_kwargs)
         col = lambda k, d: np.array([p.get(k, d) for p in points], np.float64)
         model = DistrQLearning(env=env, gamma=gamma, epsilon=col("epsilon", 0.4), epsilon_decay_rate=col("epsilon_decay_rate", 0.0),
                                lr=col("lr", 0.4), lr_decay_rate=col("lr_decay_rate", 0.0), default_q=default_q,
@@ -131,6 +134,8 @@ def launch_grid(hyperparams: Dict[str, Sequence[float]], random_seeds: Sequence[
                               "exploit_freq": str(exploit_freq)}
             if rng != "philox":
                 config["MISC"]["rng"] = rng
+            if malfunction_rng != "philox":
+                config["MISC"]["malfunction_rng"] = malfunction_rng
             config["ENV"] = {k: str(v) for k, v in env_section.items()}
             config["MODEL"] = {"gamma": str(gamma), **{k: str(params[k]) for k in names}, "default_q": str(default_q),
                                "num_episodes": str(num_episodes)}
@@ -183,8 +188,10 @@ def main(argv=None):
     ap.add_argument("--q-cap", type=int, default=None, help="Q hash rows per environment (default: MISC.q_cap, else sized from the map)")
     ap.add_argument("--rng", choices=("philox", "reference"), default=None,
                     help="epsilon-greedy stream of learn(): philox, or the reference's own numpy stream (default: MISC.rng, else philox)")
+    ap.add_argument("--malfunction-rng", choices=("philox", "reference"), default=None,
+                    help="malfunction draws: philox, or flatland's own numpy stream of the seed (default: MISC.malfunction_rng, else philox)")
     args = ap.parse_args(argv)
-    launch_experiment(args.config, device=args.device, q_cap=args.q_cap, rng=args.rng)
+    launch_experiment(args.config, device=args.device, q_cap=args.q_cap, rng=args.rng, malfunction_rng=args.malfunction_rng)
 
 
 if __name__ == "__main__":

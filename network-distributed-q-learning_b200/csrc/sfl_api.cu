@@ -152,6 +152,21 @@ SFL_FN void kat_pcg64_one(const uint64_t *gen, const uint64_t *codes, int n_code
 }
 SFL_FN int kat_explore_one(const double *r) { return eps_explore(r[0], r[1], r[2], (int)r[3], r[4]); }
 
+// flatland's malfunction schedule of every environment (SFL_MALF_REFERENCE): one group per environment, its MT19937 state
+// (2 x 624 words) in shared memory.  result[0]: the largest event count, result[1]: 1 = a seed RandomState refuses,
+// 2 = min_duration > max_duration with malfunctions on (randint(min, max + 1) refuses)
+struct MalfArgs { const sfl_hparams *hp; const unsigned long long *hit_below; int *ev; int *result; int n_envs, T, steps, ev_cap; };
+template <int G> SFL_FN void malf_env(const MalfArgs &a, int env, unsigned *mt, const Grp<G> &g, int &max_n, int &flags) {
+  const sfl_hparams &h = a.hp[env];
+  const unsigned long long hit = a.hit_below[env];
+  if (hit && h.malf_min > h.malf_max) { flags |= 2; return; }
+  const int n = malf_schedule_env(h.seed, hit, h.malf_min, h.malf_max, a.T, a.steps, a.ev + (size_t)env * a.ev_cap * 3, a.ev_cap,
+                                  mt, mt + SFL_MT_N, g);
+  if (n < 0) flags |= 1;
+  else if (n > max_n) max_n = n;
+}
+#define SFL_MALF_WARPS 4
+
 #ifndef SFL_HOST_EMUL
 __global__ void k_kat_pcg64(const uint64_t *gens, const uint64_t *codes, int n, int n_codes, uint64_t *out) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
@@ -160,6 +175,16 @@ __global__ void k_kat_pcg64(const uint64_t *gens, const uint64_t *codes, int n, 
 __global__ void k_kat_explore(const double *rows, int n, int *out) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i < n) out[i] = kat_explore_one(rows + 5 * (size_t)i);
+}
+
+__global__ void __launch_bounds__(32 * SFL_MALF_WARPS) k_malf_schedule(const __grid_constant__ MalfArgs a) {
+  __shared__ unsigned s_mt[SFL_MALF_WARPS][2 * SFL_MT_N];
+  const int w = threadIdx.x >> 5, env = blockIdx.x * SFL_MALF_WARPS + w;
+  if (env >= a.n_envs) return;                         // warp-uniform
+  const Grp<32> g;
+  int max_n = 0, flags = 0;
+  malf_env(a, env, s_mt[w], g, max_n, flags);
+  if (g.gl == 0) { if (max_n) atomicMax(&a.result[0], max_n); if (flags) atomicOr(&a.result[1], flags); }
 }
 
 __global__ void __launch_bounds__(256) k_q_reinit(const __grid_constant__ ReinitArgs a) {
@@ -296,6 +321,7 @@ struct Ctx {
   unsigned hot_bytes, env_smem, tail_hot;
   void *blob;          // device block holding every map table
   void *sum_buf;       // 2 x u64
+  void *malf_buf;      // SFL_MALF_REFERENCE: n_envs x u64 hit_below, then the 2 x i32 result of k_malf_schedule
 };
 
 // ------------------------------------------------------------------------------------------------ launch plan
@@ -355,6 +381,8 @@ static int make_layout(const sfl_map_desc *map, const sfl_config *cfg, Layout *L
   if (a_max > 15) return fail(SFL_E_ARG, "A > 15%s");
   if ((uint64_t)map->NP * map->NT * 48ull >= 0xFFFFFFFFull) return fail(SFL_E_ARG, "state index does not fit 32 bits%s");
   if (cfg->rng != SFL_RNG_PHILOX && cfg->rng != SFL_RNG_REFERENCE) return fail(SFL_E_ARG, "rng must be SFL_RNG_PHILOX (0) or SFL_RNG_REFERENCE (1)%s");
+  if (cfg->malf_rng != SFL_MALF_PHILOX && cfg->malf_rng != SFL_MALF_REFERENCE)
+    return fail(SFL_E_ARG, "malf_rng must be SFL_MALF_PHILOX (0) or SFL_MALF_REFERENCE (1)%s");
   memset(L, 0, sizeof(*L));
   L->T = map->T; L->S = map->S; L->NP = map->NP; L->NT = map->NT; L->a_max = a_max; L->q_cap = cfg->q_cap;
   L->q_stride = 1 + a_max; L->pend_cap = cfg->pend_cap;
@@ -562,6 +590,10 @@ int sfl_create(const sfl_map_desc *map, const sfl_config *cfg, int device, void 
   if (cfg->shared_q && map->T > 64) return fail(SFL_E_ARG, "shared-table mode supports at most 64 trains%s");
   if (cfg->shared_q && cfg->rng == SFL_RNG_REFERENCE)
     return fail(SFL_E_ARG, "the reference's random stream (SFL_RNG_REFERENCE) has no shared-table mode: the reference keeps one table and one stream per learner%s");
+  if (cfg->malf_rng == SFL_MALF_REFERENCE && cfg->shared_q)
+    return fail(SFL_E_ARG, "flatland's malfunction stream (SFL_MALF_REFERENCE) has no shared-table mode%s");
+  if (cfg->malf_rng == SFL_MALF_REFERENCE && cfg->ev_cap < 1)
+    return fail(SFL_E_ARG, "flatland's malfunction stream (SFL_MALF_REFERENCE) needs ev_cap >= 1: the schedule goes to replay_ev%s");
   const int H = map->H, W = map->W, Hp = H + 2, Wp = W + 2, T = map->T, NT = map->NT, S = map->S, NP = map->NP, NA = map->NA;
   // every transition must lead to a rail cell inside the grid (flatland maps are consistent); the device relies on it
   for (int r = 0; r < H; r++) for (int cc = 0; cc < W; cc++) {
@@ -583,7 +615,7 @@ int sfl_create(const sfl_map_desc *map, const sfl_config *cfg, int device, void 
   DeviceGuard dg(device);
   Ctx *c = new (std::nothrow) Ctx();
   if (!c) return fail(SFL_E_NOMEM, "host alloc%s");
-  c->L = L; c->cfg = *cfg; c->bound = 0; c->device = device; c->q_init_on = 0; c->cta_warps = 0; c->roomy = -1; c->phase_clock = 0; c->blob = nullptr; c->sum_buf = nullptr; c->sm_count = sm_count;
+  c->L = L; c->cfg = *cfg; c->bound = 0; c->device = device; c->q_init_on = 0; c->cta_warps = 0; c->roomy = -1; c->phase_clock = 0; c->blob = nullptr; c->sum_buf = nullptr; c->malf_buf = nullptr; c->sm_count = sm_count;
   memset(&c->bufs, 0, sizeof(c->bufs));
   auto pcell = [&](int cell) { return cell < 0 ? -1 : (cell / W + 1) * Wp + (cell % W + 1); };
   // ---- pack every table into one host image, 16-byte aligned sections
@@ -627,7 +659,10 @@ int sfl_create(const sfl_map_desc *map, const sfl_config *cfg, int device, void 
     dist[((size_t)k * Hp * Wp + (r + 1) * Wp + cc + 1) * 4 + d] = map->dist[(((size_t)k * H + r) * W + cc) * 4 + d];
   int8_t *qi = (int8_t *)&img[o_qi];
   for (int i = 0; i < NP * NT; i++) qi[i] = map->qinit_act[i] < 0 ? (int8_t)-1 : (int8_t)(map->qinit_act[i] | (map->qinit_final[i] ? 16 : 0));
-  if (dev_alloc(&c->blob, img.size()) || dev_alloc(&c->sum_buf, 16)) { sfl_destroy(c); return fail(SFL_E_CUDA, "device alloc of map constants failed%s"); }
+  if (dev_alloc(&c->blob, img.size()) || dev_alloc(&c->sum_buf, 16) ||
+      (cfg->malf_rng == SFL_MALF_REFERENCE && dev_alloc(&c->malf_buf, (size_t)cfg->n_envs * 8 + 8))) {
+    sfl_destroy(c); return fail(SFL_E_CUDA, "device alloc of map constants failed%s");
+  }
   if (h2d(c->blob, img.data(), img.size(), nullptr)) { sfl_destroy(c); return fail(SFL_E_CUDA, "upload of map constants failed%s"); }
 #ifndef SFL_HOST_EMUL
   if (cudaDeviceSynchronize() != cudaSuccess) { sfl_destroy(c); return fail(SFL_E_CUDA, "upload of map constants failed%s"); }
@@ -666,6 +701,7 @@ int sfl_destroy(void *ctx) {
   DeviceGuard dg(c->device);
   if (c->blob) dev_free(c->blob);
   if (c->sum_buf) dev_free(c->sum_buf);
+  if (c->malf_buf) dev_free(c->malf_buf);
   delete c;
   return SFL_OK;
 }
@@ -720,7 +756,8 @@ int sfl_set_phase_clock(void *ctx, int on) {
 int sfl_describe_launch(void *ctx, int mode, int traced, char *buf, int cap) {
   Ctx *c = (Ctx *)ctx;
   if (!c || !buf || cap < 1) return fail(SFL_E_ARG, "null argument%s");
-  const int trace = traced || mode == SFL_MODE_STEP || mode == SFL_MODE_REPLAY || c->phase_clock || (mode == SFL_MODE_LEARN && c->cfg.rng);
+  const int trace = traced || mode == SFL_MODE_STEP || mode == SFL_MODE_REPLAY || c->phase_clock ||
+                    (mode == SFL_MODE_LEARN && (c->cfg.rng || c->cfg.malf_rng));
   const int kind = trace ? K_FULL : (mode == SFL_MODE_GREEDY ? K_GREEDY : K_LEARN);
   LaunchPlan lp;
   if (plan_launch(c, kind, &lp)) return SFL_E_ARG;
@@ -805,11 +842,11 @@ int sfl_run(void *ctx, int mode, int max_ticks, void *stream) {
   ra.step_out = (sfl_step_rec *)c->bufs.step_out;
   if (c->cfg.shared_q) { ra.sq_q = (double *)c->bufs.shared_q; ra.sq_d = (long long *)c->bufs.shared_d; ra.sq_c = (int *)c->bufs.shared_c; }
   // recorded malfunction events replace the Philox draws in replay mode, and in greedy / step mode when a schedule was bound (ev_cap > 0)
-  // -- and in learn mode with the reference's stream, whose learn runs use the full kernel
-  const int ref_learn = mode == SFL_MODE_LEARN && c->cfg.rng == SFL_RNG_REFERENCE;
+  // -- and in learn mode with the reference's stream or flatland's malfunction schedule, whose learn runs use the full kernel
+  const int ref_learn = mode == SFL_MODE_LEARN && (c->cfg.rng == SFL_RNG_REFERENCE || c->cfg.malf_rng == SFL_MALF_REFERENCE);
   ra.replay_ev = ((mode != SFL_MODE_LEARN || ref_learn) && c->cfg.ev_cap > 0) ? (const int *)c->bufs.replay_ev : nullptr;
   // learn and greedy without traces run the two specialised kernels; replay, step, traced runs and learning on the
-  // reference's stream the full one
+  // reference's streams the full one
   ra.phase_clock = c->phase_clock;
   const int trace = ra.trace_dec || ra.trace_tick || mode == SFL_MODE_STEP || mode == SFL_MODE_REPLAY || c->phase_clock || ref_learn;
   const int kind = trace ? K_FULL : (mode == SFL_MODE_GREEDY ? K_GREEDY : K_LEARN);
@@ -838,6 +875,39 @@ int sfl_run(void *ctx, int mode, int max_ticks, void *stream) {
     else env_run<1, K_LEARN, true, false, false>(K, i, 0u, host_scratch);
   }
 #endif
+  return SFL_OK;
+}
+
+int sfl_malf_schedule(void *ctx, const uint64_t *hit_below, int32_t *max_events, void *stream) {
+  Ctx *c = (Ctx *)ctx;
+  if (!c || !hit_below || !max_events) return fail(SFL_E_ARG, "null argument%s");
+  if (c->cfg.malf_rng != SFL_MALF_REFERENCE) return fail(SFL_E_STATE, "the context was not created with SFL_MALF_REFERENCE%s");
+  if (!c->bound || !c->bufs.replay_ev) return fail(SFL_E_STATE, "sfl_bind first, with replay_ev%s");
+  const int n = c->cfg.n_envs;
+  for (int i = 0; i < n; i++) if (hit_below[i] > (1ull << 53)) return fail(SFL_E_ARG, "hit_below must be at most 2^53%s");
+  DeviceGuard dg(c->device);
+  MalfArgs a;
+  a.hp = (const sfl_hparams *)c->bufs.hparams; a.hit_below = (const unsigned long long *)c->malf_buf; a.ev = (int *)c->bufs.replay_ev;
+  a.result = (int *)((char *)c->malf_buf + (size_t)n * 8); a.n_envs = n; a.T = c->L.T; a.steps = c->m.max_episode_steps; a.ev_cap = c->cfg.ev_cap;
+  int res[2] = {0, 0};
+  CK(h2d(c->malf_buf, hit_below, (size_t)n * 8, stream));
+#ifndef SFL_HOST_EMUL
+  CK(dev_zero(a.result, 8, stream));
+  k_malf_schedule<<<(n + SFL_MALF_WARPS - 1) / SFL_MALF_WARPS, 32 * SFL_MALF_WARPS, 0, (cudaStream_t)stream>>>(a);
+  CU(cudaGetLastError());
+  CK(d2h(res, a.result, 8, stream));
+#else
+  static thread_local unsigned mt[2 * SFL_MT_N];
+  for (int i = 0; i < n; i++) malf_env(a, i, mt, Grp<1>(), res[0], res[1]);
+#endif
+  *max_events = res[0];
+  if (res[1] & 1) return fail(SFL_E_ARG, "Seed must be between 0 and 2**32 - 1%s");
+  if (res[1] & 2) return fail(SFL_E_ARG, "min_duration > max_duration: randint(min_duration, max_duration + 1) has low >= high%s");
+  if (res[0] > c->cfg.ev_cap) {
+    char detail[96];
+    snprintf(detail, sizeof(detail), "%d events, ev_cap is %d", res[0], c->cfg.ev_cap);
+    return fail(SFL_E_NOMEM, "the malfunction schedule does not fit replay_ev: %s", detail);
+  }
   return SFL_OK;
 }
 

@@ -461,6 +461,91 @@ SFL_FN int pcg_explore_action(Pcg &g, int mask) {
   return ffs64(mm);
 }
 
+// ------------------------------------------------------------------------------------------------ flatland's malfunction stream
+// SFL_MALF_REFERENCE: numpy's legacy RandomState (MT19937) exactly as flatland draws from it.  rail_env.reset(random_seed=
+// seed) creates np_random = RandomState(seed) at every episode (switch_env.py:99); every tick 1 .. max_episode_steps, for
+// every train in handle order, ParamMalfunctionGen.generate draws rand() < 1 - exp(-rate) and, on a hit, randint(min,
+// max + 1) + 1 steps (SURVEY.md Appendix B, F5).  No draw depends on the actions: the schedule is a function of (seed, rate,
+// min, max, T, max_episode_steps), the same in every episode.  Integer arithmetic only (numpy's mt19937.c, _mt19937.pyx
+// _legacy_seeding, distributions.c random_bounded_uint64_fill).  The 624 state words and their tempered outputs live in
+// memory shared by the G lanes of a group: the group twists together, and every lane walks the same draws (broadcast reads).
+#define SFL_MT_N 624
+#define SFL_MT_M 397
+SFL_FN unsigned mt_temper(unsigned y) {
+  y ^= y >> 11;
+  y ^= (y << 7) & 0x9D2C5680u;
+  y ^= (y << 15) & 0xEFC60000u;
+  return y ^ (y >> 18);
+}
+// RandomState(seed): init_genrand; numpy accepts only 0 <= seed < 2^32 (returns 0 for any other seed).  The one place that
+// turns a seed into the generator's key.
+template <int G> SFL_FN int mt_seed(unsigned *key, unsigned long long seed, const Grp<G> &g) {
+  if (seed >> 32) return 0;
+  if (g.gl == 0) {
+    unsigned s = (unsigned)seed;
+    SFL_NU
+    for (int i = 0; i < SFL_MT_N; i++) { key[i] = s; s = 1812433253u * (s ^ (s >> 30)) + (unsigned)(i + 1); }
+  }
+  g.sync();
+  return 1;
+}
+// mt19937_gen, G words at a time: new key[i] needs old key[i], old key[i + 1] (new key[0] for i = N - 1) and key[i + M]
+// (old) below N - M, key[i - (N - M)] (new: an earlier chunk) from there on -- all read before the chunk writes.  Then
+// every word is tempered into out[].
+template <int G> SFL_FN void mt_twist(unsigned *key, unsigned *out, const Grp<G> &g) {
+  SFL_NU
+  for (int base = 0; base < SFL_MT_N; base += G) {
+    const int i = base + g.gl;
+    unsigned v = 0u;
+    if (i < SFL_MT_N) {
+      const unsigned y = (key[i] & 0x80000000u) | (key[i + 1 == SFL_MT_N ? 0 : i + 1] & 0x7FFFFFFFu);
+      v = key[i < SFL_MT_N - SFL_MT_M ? i + SFL_MT_M : i - (SFL_MT_N - SFL_MT_M)] ^ (y >> 1) ^ ((0u - (y & 1u)) & 0x9908B0DFu);
+    }
+    g.sync();
+    if (i < SFL_MT_N) key[i] = v;
+    g.sync();
+  }
+  for (int i = g.gl; i < SFL_MT_N; i += G) out[i] = mt_temper(key[i]);
+  g.sync();
+}
+template <int G> SFL_FN unsigned mt_next(unsigned *key, unsigned *out, int &pos, const Grp<G> &g) {
+  if (pos == SFL_MT_N) { mt_twist(key, out, g); pos = 0; }
+  return out[pos++];
+}
+// RandomState.randint(lo, lo + rng + 1) - lo: masked rejection on 32-bit words, mask = the smallest 2^k - 1 >= rng; rng = 0
+// consumes no word
+template <int G> SFL_FN unsigned mt_masked(unsigned *key, unsigned *out, int &pos, const Grp<G> &g, unsigned rng) {
+  if (!rng) return 0u;
+  unsigned mask = rng;
+  mask |= mask >> 1; mask |= mask >> 2; mask |= mask >> 4; mask |= mask >> 8; mask |= mask >> 16;
+  unsigned v;
+  SFL_NU
+  do v = mt_next(key, out, pos, g) & mask; while (v > rng);
+  return v;
+}
+// One environment's schedule: every drawn event (tick, train, duration) in tick order into ev[0 .. ev_cap), -1 after the
+// last when there is room.  rand() = ((a >> 5) 2^26 + (b >> 6)) 2^-53 < p is compared in the integers: k < hit_below =
+// ceil(p 2^53).  Returns the number of events (also those beyond ev_cap), or -1 for a seed RandomState refuses.
+template <int G> SFL_FN int malf_schedule_env(unsigned long long seed, unsigned long long hit_below, int lo, int hi, int T, int steps,
+                                              int *ev, int ev_cap, unsigned *key, unsigned *out, const Grp<G> &g) {
+  if (!mt_seed(key, seed, g)) return -1;
+  int n = 0, pos = SFL_MT_N;
+  const unsigned rng = (unsigned)hi - (unsigned)lo;
+  SFL_NU
+  for (int tick = 1; hit_below && tick <= steps; tick++) {
+    SFL_NU
+    for (int t = 0; t < T; t++) {
+      const unsigned a = mt_next(key, out, pos, g), b = mt_next(key, out, pos, g);
+      if ((((unsigned long long)(a >> 5) << 26) | (b >> 6)) >= hit_below) continue;
+      const int dur = lo + (int)mt_masked(key, out, pos, g, rng) + 1;
+      if (g.gl == 0 && n < ev_cap) { ev[3 * n] = tick; ev[3 * n + 1] = t; ev[3 * n + 2] = dur; }
+      n++;
+    }
+  }
+  if (g.gl == 0 && n < ev_cap) ev[3 * n] = -1;
+  return n;
+}
+
 // ------------------------------------------------------------------------------------------------ F1
 // flatland rail.check_action_on_agent (SURVEY.md Appendix B; called switch_env.py:325,450,545, reward_func.py:49)
 // through the per-(cell, heading) move table built in sfl_create: entry bits [3a, 3a+3) = valid | new heading << 1
