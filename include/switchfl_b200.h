@@ -24,7 +24,7 @@
 extern "C" {
 #endif
 
-#define SFL_ABI_VERSION 9
+#define SFL_ABI_VERSION 10
 
 enum {
   SFL_OK = 0,
@@ -93,6 +93,8 @@ typedef struct sfl_config {
                                    buffer; sfl_shared_q_apply folds the mean step into the table (see DESIGN.md)  */
   int32_t rng;                  /* epsilon-greedy stream of SFL_MODE_LEARN: SFL_RNG_PHILOX (0) or SFL_RNG_REFERENCE (1)      */
   int32_t malf_rng;             /* malfunction draws: SFL_MALF_PHILOX (0) or SFL_MALF_REFERENCE (1)                           */
+  int32_t eval_q;               /* 1: evaluation context -- greedy runs on ONE read-only Q table (sfl_set_eval_table) shared by
+                                   every environment; no per-environment tables.  0: today's layout                       */
 } sfl_config;
 
 /* sfl_config.rng.
@@ -124,6 +126,17 @@ enum { SFL_RNG_PHILOX = 0, SFL_RNG_REFERENCE = 1 };
  *   ev_cap >= 1; not with shared_q.                                                                                    */
 enum { SFL_MALF_PHILOX = 0, SFL_MALF_REFERENCE = 1 };
 
+/* sfl_config.eval_q: evaluating one learned policy on many environments (eval.py:31-97 runs test() ten times).
+ * Greedy rollouts never change a decision by writing: the only write test() makes is the insert-on-lookup of a default
+ * row (distr_q.py:482 -> :56-57), and a missing row and a fresh default row give the same max_action.  So an evaluation
+ * context keeps no per-environment Q region (env_stride ends after the per-switch records) and q_cap is the capacity of
+ * ONE open-addressing table (same row format, hash and probing as the private tables) in the caller-owned buffer
+ * sfl_buffers.eval_q (sfl_sizes.eval_q_bytes), filled by sfl_set_eval_table.  The greedy kernel probes it through the
+ * non-coherent path and never inserts: a miss reads as the default row (default_q x A).  The table is not mutated and
+ * q_rows stays 0; lazy Q-init (sfl_enable_q_init) does not apply -- put the optimistic rows into the table.
+ * sfl_run accepts SFL_MODE_GREEDY only, without traces or the phase clock.  Not with shared_q or SFL_RNG_REFERENCE
+ * (a greedy run draws no epsilon); SFL_MALF_REFERENCE is allowed (flatland's malfunctions of every seed).               */
+
 /* DistrQLearning.__init__ arguments (distr_q.py:32) + MalfunctionParameters (main.py:28-33), per env */
 typedef struct sfl_hparams {
   double gamma, epsilon, epsilon_decay_rate, lr, lr_decay_rate, default_q;
@@ -153,6 +166,7 @@ typedef struct sfl_sizes {
   int32_t a_max;
   uint64_t rng_offset;          /* SFL_RNG_REFERENCE: byte offset of the stream's state in an env block: uint64 state_hi,
                                    state_lo, inc_hi, inc_lo, uint32 has_uint32, uinteger (numpy's PCG64 state); 0 otherwise */
+  uint64_t eval_q_bytes;        /* sfl_config.eval_q: q_cap rows x q_stride doubles (the evaluation table); 0 otherwise     */
 } sfl_sizes;
 
 typedef struct sfl_buffers {    /* all device pointers; optional ones may be NULL                     */
@@ -162,6 +176,7 @@ typedef struct sfl_buffers {    /* all device pointers; optional ones may be NUL
   void *replay_act; void *replay_ev;
   void *step_out;
   void *shared_q; void *shared_d; void *shared_c;    /* shared-table mode; shared_d / shared_c may be all-reduced (sum) by the caller */
+  void *eval_q;                                      /* sfl_config.eval_q: the evaluation table (eval_q_bytes); mandatory there */
 } sfl_buffers;
 
 typedef struct sfl_env_counters {      /* written by sfl_run for every env                            */
@@ -281,7 +296,8 @@ int sfl_set_roomy(void *ctx, int roomy);
 int sfl_set_phase_clock(void *ctx, int on);
 /* Which kernel instantiation and launch configuration sfl_run(mode) would use now (traced != 0: with decision / tick
  * traces), as text: "k_run<G=..,KIND=..,TH=..,SQ=..,ONE=..,ROOMY=..> grid=.. block=.. smem=..", with ",NW=2" after ROOMY
- * on maps with more than 64 trains (two words per train set); learn with SFL_RNG_REFERENCE or SFL_MALF_REFERENCE is KIND=full.  No counterpart in the
+ * on maps with more than 64 trains (two words per train set); learn with SFL_RNG_REFERENCE or SFL_MALF_REFERENCE is KIND=full.  Evaluation
+ * contexts (sfl_config.eval_q) name their kernel "k_eval<G=..,KIND=greedy,TH=..,SQ=0,ONE=..,ROOMY=0[,NW=2],EVQ=1> ...".  No counterpart in the
  * reference; it lets the parity tests name -- and force, with sfl_set_lanes / sfl_set_roomy -- exactly the
  * instantiations the benchmark launches.  Needs no bound buffers.                                                  */
 int sfl_describe_launch(void *ctx, int mode, int traced, char *buf, int cap);
@@ -315,6 +331,10 @@ int sfl_total_decisions(void *ctx, uint64_t *decisions, uint64_t *ticks, void *s
 int sfl_export_q(void *ctx, int env, uint32_t *keys_host, double *vals_host, int cap_rows, int *n_rows, void *stream);
 /* Q-table import (distr_q.py:510-527 load) */
 int sfl_import_q(void *ctx, int env, const uint32_t *keys_host, const double *vals_host, int n_rows, void *stream);
+/* sfl_config.eval_q: fill the bound evaluation table with n_rows (key, A_max values) rows -- the hash image sfl_import_q
+ * builds, once, uploaded into sfl_buffers.eval_q; a repeated key overwrites its row.  SFL_E_NOMEM when n_rows >= q_cap.
+ * Synchronises `stream`.  Export / import of per-environment rows do not exist in these contexts.                    */
+int sfl_set_eval_table(void *ctx, const uint32_t *keys_host, const double *vals_host, int n_rows, void *stream);
 
 #ifdef __cplusplus
 }

@@ -462,6 +462,60 @@ class DistrQLearning:
         self._q_stale = True                 # test() inserts rows (App. A #15)
         return float(cum[p]), int(arr[p]), list(delays[p])
 
+    # ------------------------------------------------------------------ evaluation on one read-only table (extension)
+    def evaluate(self, q_table: Optional[Dict[tuple, List[float]]] = None, n_runs: Optional[int] = None,
+                 seeds: Optional[Sequence[int]] = None, out_dir: Optional[str] = None):
+        """Greedy rollouts of one table -- what eval.py does with ``load()`` + ``test()`` ten times -- on as many environments
+        as wanted: one episode per environment of an evaluation engine on the same map (``Engine(eval_q=True)``), every
+        environment reading the one read-only table.  ``q_table``: default ``self.q_table`` (with the optimistic rows when
+        this learner was q-initialised).  ``seeds``: one per run; default ``seed + i`` for ``n_runs`` runs (default: as many
+        as this learner has environments), the seeds ``test()`` gives its environments.
+
+        Decisions and metrics equal ``load()`` + ``test()``; the one difference is that the table is not mutated: ``test()``
+        inserts a default row at every lookup that misses (distr_q.py:482 -> :56-57), which never changes a decision.
+        This learner's engine and tables are not touched.  Returns (cum_reward[n], arrived[n], delays[n, T],
+        num_malfunctions[n], the arrived trains of every run); ``out_dir``: also writes them to ``eval_batched.npz``."""
+        env = self.env
+        q = self.q_table if q_table is None else q_table
+        if seeds is None:
+            n = env.n_envs if n_runs is None else int(n_runs)
+            seeds = np.arange(n, dtype=np.uint64) + np.uint64(self.seed)
+        seeds = np.asarray(seeds, np.uint64).reshape(-1)
+        if n_runs is not None and len(seeds) != int(n_runs):
+            raise ValueError(f"{len(seeds)} seeds for {n_runs} runs")
+        n, T = len(seeds), env.rail_map.trains.T
+        cap = 1024
+        while cap < 2 * len(q) + 2:                                       # load factor at most one half
+            cap *= 2
+        learner = env.engine
+        eng = env.engine_cls(env.rail_map, n_envs=n, device=learner.device, q_cap=cap, max_steps=env.max_steps, ep_cap=1,
+                             eval_q=True, malfunction_rng=learner.malfunction_rng)
+        try:
+            eng.set_hparams(default_q=self._default_q_of(self.primary_env), seeds=seeds, episodes=1)
+            eng.reset()
+            eng.set_eval_table(q)
+            t0 = time.time()
+            while True:
+                eng.run(MODE_GREEDY, self.ticks_per_launch)
+                c = eng.counters()
+                if c["err"].any():
+                    eng.check_errors()
+                if (c["halted"] == 1).all():
+                    break
+            self.eval_time = time.time() - t0
+            _, log, dl = eng.episode_log()
+        finally:
+            eng.close()
+        cum, arr = log["cum_reward"][:, 0].copy(), log["arrived"][:, 0].copy()
+        delays, malf = dl[:, 0].astype(np.float64), log["num_malfunctions"][:, 0].copy()
+        at_dest = [train_set(r["arrived_mask"], r["arrived_mask_hi"], T) for r in log[:, 0]]
+        if out_dir:
+            os.makedirs(out_dir, exist_ok=True)
+            np.savez_compressed(os.path.join(out_dir, "eval_batched.npz"), cum_reward=cum, arrived_trains=arr, delays=delays,
+                                num_malfunctions=malf, seeds=seeds,
+                                arrived_mask=log["arrived_mask"][:, 0].copy(), arrived_mask_hi=log["arrived_mask_hi"][:, 0].copy())
+        return cum, arr, delays, malf, at_dest
+
     # ------------------------------------------------------------------ distr_q.py:400-490, on the host dict
     # The reference's per-decision learner methods, for code that drives the AEC protocol itself (env.agent_iter /
     # last / step) and keeps the learning rule on the host.  They work on ``self.q_table`` exactly like the reference
@@ -512,9 +566,7 @@ class DistrQLearning:
             pickle.dump(q, f)
 
     def load(self, filename: str):
-        with open(filename, "rb") as f:
-            q = pickle.load(f)
-        self.q_table = {tuple(int(x) for x in k): [float(x) for x in v] for k, v in q.items()}
+        self.q_table = read_q_table(filename)
         eng = self.env.engine
         if not eng.shared_q and len(self.q_table) >= eng.cfg.q_cap:
             raise ValueError(f"{filename}: {len(self.q_table)} rows do not fit the {eng.cfg.q_cap}-row Q tables of this env; "
@@ -525,6 +577,13 @@ class DistrQLearning:
             eng.import_q(i, self.q_table)
         self._table_dirty = True
         self._q_inited = False
+
+
+def read_q_table(filename: str) -> Dict[tuple, List[float]]:
+    """A pickled q_table (distr_q_model.pkl / checkpoint_N.pkl, distr_q.py:521-527) as the dict ``load()`` keeps."""
+    with open(filename, "rb") as f:
+        q = pickle.load(f)
+    return {tuple(int(x) for x in k): [float(x) for x in v] for k, v in q.items()}
 
 
 def learn_concurrently(models: Sequence[DistrQLearning], num_episodes: int, out_dirs: Optional[Sequence[Optional[str]]] = None,

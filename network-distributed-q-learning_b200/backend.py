@@ -18,7 +18,7 @@ from . import railmap
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "csrc", "libswitchfl_b200.so")
 
-ABI_VERSION = 9
+ABI_VERSION = 10
 MODE_LEARN, MODE_GREEDY, MODE_REPLAY, MODE_STEP = 0, 1, 2, 3
 RNG_PHILOX, RNG_REFERENCE = 0, 1
 RNG_NAMES = {"philox": RNG_PHILOX, "reference": RNG_REFERENCE}
@@ -46,19 +46,21 @@ class MapDesc(C.Structure):
 
 class Config(C.Structure):
     _fields_ = [(n, C.c_int32) for n in ("n_envs", "q_cap", "pend_cap", "max_steps", "dec_cap", "tick_cap", "ep_cap",
-                                         "act_cap", "ev_cap", "trace_sem", "shared_q", "rng", "malf_rng")]
+                                         "act_cap", "ev_cap", "trace_sem", "shared_q", "rng", "malf_rng", "eval_q")]
 
 
 class Sizes(C.Structure):
     _fields_ = [(n, C.c_uint64) for n in ("state_bytes", "env_stride", "hparams_bytes", "trace_dec_bytes", "trace_tick_bytes",
                                           "trace_sem_bytes", "ep_log_bytes", "ep_delay_bytes", "replay_act_bytes",
                                           "replay_ev_bytes", "counters_bytes", "step_out_bytes", "shared_q_bytes", "shared_d_bytes",
-                                          "shared_c_bytes")] + [("q_stride", C.c_int32), ("a_max", C.c_int32), ("rng_offset", C.c_uint64)]
+                                          "shared_c_bytes")] + [("q_stride", C.c_int32), ("a_max", C.c_int32), ("rng_offset", C.c_uint64),
+                                                                  ("eval_q_bytes", C.c_uint64)]
 
 
 class Buffers(C.Structure):
     _fields_ = [(n, C.c_void_p) for n in ("state", "hparams", "counters", "trace_dec", "trace_tick", "trace_sem", "ep_log",
-                                          "ep_delay", "replay_act", "replay_ev", "step_out", "shared_q", "shared_d", "shared_c")]
+                                          "ep_delay", "replay_act", "replay_ev", "step_out", "shared_q", "shared_d", "shared_c",
+                                          "eval_q")]
 
 
 HPARAMS_DT = np.dtype([("gamma", "f8"), ("epsilon", "f8"), ("epsilon_decay_rate", "f8"), ("lr", "f8"), ("lr_decay_rate", "f8"),
@@ -111,6 +113,7 @@ def load_library(path: Optional[str] = None) -> C.CDLL:
     lib.sfl_total_decisions.argtypes = [C.c_void_p, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64), C.c_void_p]
     lib.sfl_export_q.argtypes = [C.c_void_p, C.c_int, C.POINTER(C.c_uint32), C.POINTER(C.c_double), C.c_int, C.POINTER(C.c_int), C.c_void_p]
     lib.sfl_import_q.argtypes = [C.c_void_p, C.c_int, C.POINTER(C.c_uint32), C.POINTER(C.c_double), C.c_int, C.c_void_p]
+    lib.sfl_set_eval_table.argtypes = [C.c_void_p, C.POINTER(C.c_uint32), C.POINTER(C.c_double), C.c_int, C.c_void_p]
     lib.sfl_shared_q_apply.argtypes = [C.c_void_p, C.c_void_p]
     lib.sfl_shared_q_apply_to.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
     lib.sfl_kat_q_update.argtypes = [C.POINTER(C.c_double), C.c_int32, C.POINTER(C.c_double), C.c_int]
@@ -287,6 +290,45 @@ class RailMap:
         semb = sum(int(sem[k]) << k for k in range(P))
         return (((int(t.sw_port0[s]) + cur) * len(tr.targets) + tgt) * 16 + semb) * 3 + int(delay[cur])
 
+    def q_arrays(self, q: Dict[tuple, List[float]], a_max: int):
+        """The reference's dict as (uint32[n] state keys, float64[n, a_max] values, zero-padded): ``obs_to_key`` of every
+        observation, computed per group of equally long observations and rows with array operations."""
+        t, tr = self.tab, self.trains
+        NT = len(tr.targets)
+        n = len(q)
+        keys = np.zeros(max(n, 1), np.uint32)
+        vals = np.zeros((max(n, 1), a_max), np.float64)
+        if not n:
+            return keys, vals
+        # (row, col) -> switch and target cell -> target index: the first match, as list.index / np.where in obs_to_key
+        cell_sw = np.full(t.H * t.W, -1, np.int64)
+        for s in range(len(t.switch_cells) - 1, -1, -1):
+            r, c = t.switch_cells[s]
+            cell_sw[int(r) * t.W + int(c)] = s
+        cell_tgt = np.full(t.H * t.W, -1, np.int64)
+        targets = np.asarray(tr.targets, np.int64)
+        cell_tgt[targets[::-1]] = np.arange(NT - 1, -1, -1)
+        port0 = np.asarray(t.sw_port0, np.int64)
+        groups: Dict[tuple, List[int]] = {}
+        items = list(q.items())
+        for i, (obs, row) in enumerate(items):
+            groups.setdefault((len(obs), len(row)), []).append(i)
+        for (lo, lr), idx in groups.items():
+            P = (lo - 2) // 4
+            idx = np.asarray(idx)
+            o = np.array([items[i][0] for i in idx], np.int64).reshape(len(idx), lo)
+            vals[idx, :lr] = np.array([items[i][1] for i in idx], np.float64).reshape(len(idx), lr)
+            s = cell_sw[o[:, 0] * t.W + o[:, 1]]
+            delay = o[:, 2 + 3 * P:2 + 4 * P]
+            cur = np.argmax(delay >= 0, axis=1)
+            rows = np.arange(len(idx))
+            tgt = cell_tgt[o[rows, 2 + P + 2 * cur] * t.W + o[rows, 3 + P + 2 * cur]]
+            if (s < 0).any() or (tgt < 0).any() or not (delay >= 0).any(axis=1).all():
+                raise ValueError("an observation of the Q table is not one of this map's states")
+            semb = (o[:, 2:2 + P] << np.arange(P)).sum(axis=1)
+            keys[idx] = ((((port0[s] + cur) * NT + tgt) * 16 + semb) * 3 + delay[rows, cur]).astype(np.uint32)
+        return keys, vals
+
     def q_init_rows(self, default_q: float) -> Dict[tuple, List[float]]:
         """All rows __init_q_table creates (distr_q.py:81-181), as the reference's dict."""
         t, tr = self.tab, self.trains
@@ -314,8 +356,10 @@ class Engine:
                  max_steps: int = 100_000, dec_cap: int = 0, tick_cap: int = 0, ep_cap: int = 64, act_cap: int = 0,
                  ev_cap: int = 0, trace_sem: bool = False, lanes: Optional[int] = None, shared_q: bool = False,
                  cta_warps: Optional[int] = None, roomy: Optional[bool] = None, phase_clock: bool = False, bind: bool = True,
-                 rng: str = "philox", malfunction_rng: str = "philox"):
+                 rng: str = "philox", malfunction_rng: str = "philox", eval_q: bool = False):
         """``bind=False`` creates the context only (no device buffers): enough for ``describe_launch``.
+        ``eval_q``: an evaluation context -- greedy runs only, every environment reading ONE read-only Q table of ``q_cap``
+        rows (``set_eval_table``) instead of a private table; the environments keep no Q region.
         ``rng``: the epsilon-greedy stream of learn mode -- "philox" (the specialised learn kernels) or "reference" (numpy's
         PCG64 stream of the reference learner, seeded per environment from its seed at every reset that restarts the
         interaction counters: a seeded learn() makes the reference's decisions; runs on the full kernel).
@@ -338,8 +382,10 @@ class Engine:
         self.lib, self.device, dev_index = self._open(device)
         self.cfg = Config(n_envs=self.n_envs, q_cap=q_cap, pend_cap=pend_cap, max_steps=max_steps, dec_cap=dec_cap,
                           tick_cap=tick_cap, ep_cap=ep_cap, act_cap=act_cap, ev_cap=ev_cap, trace_sem=int(trace_sem),
-                          shared_q=int(shared_q), rng=RNG_NAMES[rng], malf_rng=MALF_NAMES[malfunction_rng])
+                          shared_q=int(shared_q), rng=RNG_NAMES[rng], malf_rng=MALF_NAMES[malfunction_rng], eval_q=int(eval_q))
         self.shared_q = bool(shared_q)
+        self.eval_q = bool(eval_q)
+        self.eval_rows = 0                                # rows of the evaluation table (set_eval_table)
         self.sizes = Sizes()
         self._ck(self.lib.sfl_query_sizes(C.byref(rail_map.desc), C.byref(self.cfg), C.byref(self.sizes)))
         self.ctx = C.c_void_p()
@@ -369,7 +415,7 @@ class Engine:
                     "trace_dec": z(s.trace_dec_bytes), "trace_tick": z(s.trace_tick_bytes), "trace_sem": z(s.trace_sem_bytes),
                     "ep_log": z(s.ep_log_bytes), "ep_delay": z(s.ep_delay_bytes), "replay_act": z(s.replay_act_bytes),
                     "replay_ev": z(s.replay_ev_bytes), "step_out": z(s.step_out_bytes), "shared_q": z(s.shared_q_bytes),
-                    "shared_d": z(s.shared_d_bytes), "shared_c": z(s.shared_c_bytes)}
+                    "shared_d": z(s.shared_d_bytes), "shared_c": z(s.shared_c_bytes), "eval_q": z(s.eval_q_bytes)}
         b = Buffers(**{k: v.data_ptr() for k, v in self.buf.items()})
         self._ck(self.lib.sfl_bind(self.ctx, C.byref(b)))
 
@@ -749,11 +795,17 @@ class Engine:
         return out
 
     def import_q(self, env: int, q: Dict[tuple, List[float]]):
-        a_max = self.sizes.a_max
-        keys = np.zeros(max(len(q), 1), np.uint32)
-        vals = np.zeros((max(len(q), 1), a_max), np.float64)
-        for i, (obs, row) in enumerate(q.items()):
-            keys[i] = self.map.obs_to_key(obs)
-            vals[i, :len(row)] = row
+        keys, vals = self.map.q_arrays(q, self.sizes.a_max)
         self._ck(self.lib.sfl_import_q(self.ctx, env, keys.ctypes.data_as(C.POINTER(C.c_uint32)),
                                        vals.ctypes.data_as(C.POINTER(C.c_double)), len(q), self._stream()))
+
+    def set_eval_table(self, q: Dict[tuple, List[float]]):
+        """``eval_q``: fill the evaluation table with the reference's dict (observation tuple -> list of A floats), hashed on
+        the host and uploaded once (``sfl_set_eval_table``).  Needs ``q_cap`` above the row count."""
+        if not self.eval_q:
+            raise RuntimeError("set_eval_table() needs Engine(eval_q=True)")
+        keys, vals = self.map.q_arrays(q, self.sizes.a_max)
+        self._ck(self.lib.sfl_set_eval_table(self.ctx, keys.ctypes.data_as(C.POINTER(C.c_uint32)),
+                                             vals.ctypes.data_as(C.POINTER(C.c_double)), len(q), self._stream()))
+        self.h2d_bytes += int(self.sizes.eval_q_bytes)
+        self.eval_rows = len(q)

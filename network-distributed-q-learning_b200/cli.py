@@ -3,6 +3,7 @@
     python -m switchfl_b200.cli -c config.ini                 # main.py:83-88, same INI schema
     launch_grid(hyperparams, random_seeds, out_dir, ...)      # hyperparam_tuning.py:42-91 without the process fan-out
     launch_eval(exp_dir_list)                                 # eval.py:31-97
+    python -m switchfl_b200.cli --eval EXP_DIR... [--num-evals N]
 
 ``config.ini`` keeps the reference's sections and keys (hyperparam_tuning.py:51-78): MISC{random_seed, out_dir,
 checkpoint_freq, exploit_freq}, ENV{width, height, max_num_cities, max_rails_between_cities, max_rail_pairs_in_city,
@@ -27,7 +28,7 @@ from typing import Dict, List, Optional, Sequence
 import numpy as np
 
 from . import mapgen, sharding
-from .api import ASyncSwitchEnv, DistrQLearning, MalfunctionParameters, ParamMalfunctionGen, RailEnv, learn_concurrently
+from .api import ASyncSwitchEnv, DistrQLearning, MalfunctionParameters, ParamMalfunctionGen, RailEnv, learn_concurrently, read_q_table
 
 
 def fixture_from_env_section(env: Dict[str, str], seed: int) -> dict:
@@ -148,10 +149,12 @@ def launch_grid(hyperparams: Dict[str, Sequence[float]], random_seeds: Sequence[
 
 
 def launch_eval(exp_dir_list: Sequence[str], distr_q_model_name: str = "distr_q_model.pkl", device: Optional[str] = None,
-                q_cap: Optional[int] = None, env_cls=ASyncSwitchEnv, _engine_kwargs=None) -> Dict[str, np.ndarray]:
+                q_cap: Optional[int] = None, env_cls=ASyncSwitchEnv, _engine_kwargs=None, num_evals: Optional[int] = None) -> Dict[str, np.ndarray]:
     """eval.py:31-97: for every experiment directory reload ``config.ini`` + the pickled Q-table and run the greedy
-    ``test()`` -- once, or ten times when the map has malfunctions (eval.py:88).  The evaluations are the environment
-    axis of one engine (environment i draws its malfunctions from seed + i) and go to ``eval_i/`` like the reference's."""
+    ``test()`` -- once, or ten times when the map has malfunctions (eval.py:88); ``num_evals`` runs instead when given.
+    The evaluations are the environments of one evaluation engine that reads the table once for all of them
+    (``DistrQLearning.evaluate``); environment i draws its malfunctions from seed + i.  The first ten go to ``eval_i/`` like
+    the reference's; with more than ten, ``eval_batched.npz`` holds every run."""
     out = {}
     device = device or default_device()
     for exp_dir in exp_dir_list:
@@ -161,16 +164,17 @@ def launch_eval(exp_dir_list: Sequence[str], distr_q_model_name: str = "distr_q_
         envs, mdl, seed = config["ENV"], config["MODEL"], int(config["MISC"]["random_seed"])
         rate = float(envs["malfunction_rate"])
         mf = ParamMalfunctionGen(MalfunctionParameters(rate, int(envs["min_duration"]), int(envs["max_duration"])))
-        num_evals = 10 if rate > 0 else 1
+        n = int(num_evals) if num_evals is not None else (10 if rate > 0 else 1)
         cap = q_cap if q_cap is not None else (int(config["MISC"]["q_cap"]) if config["MISC"].get("q_cap") else None)
+        # the learner's own engine only carries the map: one environment
         env = env_cls(RailEnv(fixture_from_env_section(dict(envs), seed), malfunction_generator=mf), render_mode=None,
-                      max_steps=100_000, n_envs=num_evals, device=device, q_cap=cap, _engine_kwargs=_engine_kwargs)
+                      max_steps=100_000, n_envs=1, device=device, q_cap=cap, _engine_kwargs=_engine_kwargs)
         model = DistrQLearning(env=env, gamma=float(mdl["gamma"]), epsilon=float(mdl["epsilon"]),
                                epsilon_decay_rate=float(mdl["epsilon_decay_rate"]), lr=float(mdl["lr"]),
                                lr_decay_rate=float(mdl["lr_decay_rate"]), default_q=float(mdl["default_q"]), seed=seed)
-        model.load(os.path.join(exp_dir, distr_q_model_name))
-        cum, arrived, delays = model.test(out_dir=None, plot=False, save_outputs=False, _batched=True)
-        for i in range(num_evals):
+        cum, arrived, delays, _, _ = model.evaluate(read_q_table(os.path.join(exp_dir, distr_q_model_name)), n_runs=n,
+                                                    out_dir=exp_dir if n > 10 else None)
+        for i in range(min(n, 10)):
             print(f"Eval {i+1}")
             d = os.path.join(exp_dir, f"eval_{i}")
             os.makedirs(d, exist_ok=True)
@@ -183,7 +187,11 @@ def launch_eval(exp_dir_list: Sequence[str], distr_q_model_name: str = "distr_q_
 
 def main(argv=None):
     ap = argparse.ArgumentParser()
-    ap.add_argument("-c", "--config", type=str, help="Config file path", required=True)
+    ap.add_argument("-c", "--config", type=str, help="Config file path (required unless --eval)")
+    ap.add_argument("--eval", nargs="+", metavar="EXP_DIR", default=None,
+                    help="evaluate the distr_q_model.pkl of these experiment directories (eval.py) instead of learning")
+    ap.add_argument("--num-evals", type=int, default=None,
+                    help="--eval: greedy runs per experiment, seeds random_seed + i (default: 10 on maps with malfunctions, else 1)")
     ap.add_argument("--device", default=None, help="default: cuda:<LOCAL_RANK>")
     ap.add_argument("--q-cap", type=int, default=None, help="Q hash rows per environment (default: MISC.q_cap, else sized from the map)")
     ap.add_argument("--rng", choices=("philox", "reference"), default=None,
@@ -191,6 +199,11 @@ def main(argv=None):
     ap.add_argument("--malfunction-rng", choices=("philox", "reference"), default=None,
                     help="malfunction draws: philox, or flatland's own numpy stream of the seed (default: MISC.malfunction_rng, else philox)")
     args = ap.parse_args(argv)
+    if args.eval:
+        launch_eval(args.eval, device=args.device, q_cap=args.q_cap, num_evals=args.num_evals)
+        return
+    if not args.config:
+        ap.error("the following arguments are required: -c/--config")
     launch_experiment(args.config, device=args.device, q_cap=args.q_cap, rng=args.rng, malfunction_rng=args.malfunction_rng)
 
 

@@ -73,7 +73,7 @@ struct DeviceGuard {
 #define SFL_SMEM_BUDGET (56u * 1024u)                  // per CTA, so that four CTAs share an SM
 
 // ------------------------------------------------------------------------------------------------ kernels
-struct InitArgs { Layout L; char *state; const sfl_hparams *hp; int n_envs, keep_q, keep_ninter, pad; };
+struct InitArgs { Layout L; char *state; const sfl_hparams *hp; int n_envs, keep_q, keep_ninter, no_q; };   // no_q: evaluation context
 
 struct InitEnv {          // the env block in HBM, no staging
   const Layout *L;
@@ -97,7 +97,7 @@ SFL_FN void env_init(const InitArgs &ia, int env_id, int lane, int lanes) {
     e.tra()[t] = make_int4(-1, 0, 0, 0); e.trb()[t] = make_int4(px, 0xFFFF, 0, 0);
   }
   if (!ia.keep_ninter) for (int s = lane; s < ia.L.S; s += lanes) { SwS z; z.ninter = 0; z.pad = 0; z.eps_pow = 1.0; e.sws()[s] = z; }
-  if (!ia.keep_q) {
+  if (!ia.keep_q && !ia.no_q) {
     size_t n = (size_t)ia.L.q_cap * ia.L.q_stride;
     for (size_t i = lane; i < n; i += lanes) e.q()[i] = 0.0;
   }
@@ -276,6 +276,16 @@ __global__ void k_kat_q_update(const double *in, int n, double *out) {
   if (i < n) out[i] = td_value(in[6 * i], in[6 * i + 1], in[6 * i + 2], in[6 * i + 3], in[6 * i + 4], in[6 * i + 5] != 0.0);
 }
 
+// Evaluation contexts (sfl_config.eval_q): the greedy kernel on the one read-only table (EVQ), compiled like the greedy
+// k_run instantiation it stands in for.  A kernel of its own, so that the names of the k_run instantiations stay as they were.
+template <int G, bool TH, bool ONE, int NW = 1>
+__global__ void __launch_bounds__(SFL_CTA_THREADS, NW > 1 ? SFL_MINB_WIDE : TH ? (G == 32 ? 7 : 4) : SFL_MINB_BIG)
+k_eval(const __grid_constant__ KArgs K) {
+  const int slot = threadIdx.x / G;
+  const int env_id = blockIdx.x * (blockDim.x / G) + slot;
+  env_run<G, K_GREEDY, TH, false, ONE, NW, true>(K, env_id, (unsigned)slot * K.ra.env_smem, nullptr);
+}
+
 typedef void (*run_kernel_t)(const KArgs);
 // `one`: every train has its own lane (T <= G): the production kernels have a single-pass variant for that; the full and
 // the shared-table kernels always run the general chunked loops.
@@ -296,6 +306,20 @@ template <int G> static run_kernel_t pick_kernel_g(int kind, int th, int sq, int
 template <int G> static run_kernel_t pick_wide_g(int kind) {
   return kind == K_FULL ? k_run<G, K_FULL, false, false, false, false, 2>
        : kind == K_GREEDY ? k_run<G, K_GREEDY, false, false, false, false, 2> : k_run<G, K_LEARN, false, false, false, false, 2>;
+}
+template <int G> static run_kernel_t pick_eval_g(int th, int one) {
+  return th ? (one ? k_eval<G, true, true> : k_eval<G, true, false>) : (one ? k_eval<G, false, true> : k_eval<G, false, false>);
+}
+static run_kernel_t pick_eval(int G, int th, int one, int nw) {
+  if (nw > 1) return G == 8 ? k_eval<8, false, false, 2> : G == 16 ? k_eval<16, false, false, 2> : k_eval<32, false, false, 2>;
+  switch (G) {
+    case 1: return pick_eval_g<1>(th, one);
+    case 2: return pick_eval_g<2>(th, one);
+    case 4: return pick_eval_g<4>(th, one);
+    case 8: return pick_eval_g<8>(th, one);
+    case 16: return pick_eval_g<16>(th, one);
+    default: return pick_eval_g<32>(th, one);
+  }
 }
 static run_kernel_t pick_kernel(int G, int kind, int th, int sq, int one, int roomy, int nw) {
   if (nw > 1) return G == 8 ? pick_wide_g<8>(kind) : G == 16 ? pick_wide_g<16>(kind) : pick_wide_g<32>(kind);
@@ -383,6 +407,7 @@ static int make_layout(const sfl_map_desc *map, const sfl_config *cfg, Layout *L
   if (cfg->rng != SFL_RNG_PHILOX && cfg->rng != SFL_RNG_REFERENCE) return fail(SFL_E_ARG, "rng must be SFL_RNG_PHILOX (0) or SFL_RNG_REFERENCE (1)%s");
   if (cfg->malf_rng != SFL_MALF_PHILOX && cfg->malf_rng != SFL_MALF_REFERENCE)
     return fail(SFL_E_ARG, "malf_rng must be SFL_MALF_PHILOX (0) or SFL_MALF_REFERENCE (1)%s");
+  if (cfg->eval_q != 0 && cfg->eval_q != 1) return fail(SFL_E_ARG, "eval_q must be 0 or 1%s");
   memset(L, 0, sizeof(*L));
   L->T = map->T; L->S = map->S; L->NP = map->NP; L->NT = map->NT; L->a_max = a_max; L->q_cap = cfg->q_cap;
   L->q_stride = 1 + a_max; L->pend_cap = cfg->pend_cap;
@@ -395,9 +420,36 @@ static int make_layout(const sfl_map_desc *map, const sfl_config *cfg, Layout *L
   PUT(off_sem, 16 * (unsigned)map->NP); PUT(off_rewards, 4 * (unsigned)map->S * T); PUT(off_sws, 16 * (unsigned)map->S);
 #undef PUT
   L->off_q = o;
-  L->env_stride = ((unsigned long long)o + (unsigned long long)cfg->q_cap * L->q_stride * 8ull + 127ull) / 128ull * 128ull;
+  // an evaluation context has no Q region: q_cap rows are the one table in sfl_buffers.eval_q
+  const unsigned long long q_bytes = cfg->eval_q ? 0ull : (unsigned long long)cfg->q_cap * L->q_stride * 8ull;
+  L->env_stride = ((unsigned long long)o + q_bytes + 127ull) / 128ull * 128ull;
   *a_max_out = a_max;
   return SFL_OK;
+}
+
+// The hash image of a Q table of L.q_cap rows (distr_q.py:510-527 load): row r at the slot the kernels' probe finds key r
+// at (q_row / eval_action: same hash, linear probing); a repeated key overwrites its row.  Returns the distinct keys.
+// n_rows < q_cap, so that an empty slot ends every probe.
+static int q_image(const Layout &L, const uint32_t *keys_host, const double *vals_host, int n_rows, std::vector<double> &img) {
+  img.assign((size_t)L.q_cap * L.q_stride, 0.0);
+  const unsigned mask = (unsigned)L.q_cap - 1u;
+  int distinct = 0;
+  for (int r = 0; r < n_rows; r++) {
+    unsigned key = keys_host[r];
+    unsigned i = (key * 2654435761u) >> 7;
+    for (;;) {
+      i &= mask;
+      unsigned long long k;
+      memcpy(&k, &img[(size_t)i * L.q_stride], 8);
+      if (k == 0) distinct++;
+      if (k == 0 || k == (unsigned long long)key + 1ull) break;
+      i++;
+    }
+    unsigned long long k = (unsigned long long)key + 1ull;
+    memcpy(&img[(size_t)i * L.q_stride], &k, 8);
+    for (int a = 0; a < L.a_max; a++) img[(size_t)i * L.q_stride + 1 + a] = vals_host[(size_t)r * L.a_max + a];
+  }
+  return distinct;
 }
 
 extern "C" {
@@ -561,6 +613,7 @@ int sfl_query_sizes(const sfl_map_desc *map, const sfl_config *cfg, sfl_sizes *o
   out->q_stride = L.q_stride;
   out->a_max = a_max;
   out->rng_offset = L.off_rng;
+  out->eval_q_bytes = cfg->eval_q ? (uint64_t)cfg->q_cap * L.q_stride * 8ull : 0;
   return SFL_OK;
 }
 
@@ -594,6 +647,10 @@ int sfl_create(const sfl_map_desc *map, const sfl_config *cfg, int device, void 
     return fail(SFL_E_ARG, "flatland's malfunction stream (SFL_MALF_REFERENCE) has no shared-table mode%s");
   if (cfg->malf_rng == SFL_MALF_REFERENCE && cfg->ev_cap < 1)
     return fail(SFL_E_ARG, "flatland's malfunction stream (SFL_MALF_REFERENCE) needs ev_cap >= 1: the schedule goes to replay_ev%s");
+  if (cfg->eval_q && cfg->shared_q)
+    return fail(SFL_E_ARG, "an evaluation context (eval_q) has no shared-table mode: shared-table mode is for learning%s");
+  if (cfg->eval_q && cfg->rng == SFL_RNG_REFERENCE)
+    return fail(SFL_E_ARG, "an evaluation context (eval_q) runs greedy rollouts only, which draw nothing from the reference's epsilon-greedy stream (SFL_RNG_REFERENCE)%s");
   const int H = map->H, W = map->W, Hp = H + 2, Wp = W + 2, T = map->T, NT = map->NT, S = map->S, NP = map->NP, NA = map->NA;
   // every transition must lead to a rail cell inside the grid (flatland maps are consistent); the device relies on it
   for (int r = 0; r < H; r++) for (int cc = 0; cc < W; cc++) {
@@ -713,6 +770,7 @@ int sfl_bind(void *ctx, const sfl_buffers *bufs) {
   if (c->cfg.dec_cap > 0 && !bufs->trace_dec) return fail(SFL_E_ARG, "dec_cap > 0 needs trace_dec%s");
   if (c->cfg.tick_cap > 0 && !bufs->trace_tick) return fail(SFL_E_ARG, "tick_cap > 0 needs trace_tick%s");
   if (c->cfg.shared_q && (!bufs->shared_q || !bufs->shared_d || !bufs->shared_c)) return fail(SFL_E_ARG, "shared_q needs the three shared buffers%s");
+  if (c->cfg.eval_q && !bufs->eval_q) return fail(SFL_E_ARG, "an evaluation context (eval_q) needs the eval_q buffer%s");
   c->bufs = *bufs;
   c->bound = 1;
   return SFL_OK;
@@ -749,6 +807,7 @@ int sfl_set_phase_clock(void *ctx, int on) {
   Ctx *c = (Ctx *)ctx;
   if (!c) return fail(SFL_E_ARG, "null ctx%s");
   if (on && c->cfg.shared_q) return fail(SFL_E_ARG, "shared-table mode has no instrumented kernel%s");
+  if (on && c->cfg.eval_q) return fail(SFL_E_ARG, "an evaluation context (eval_q) has no instrumented kernel%s");
   c->phase_clock = on ? 1 : 0;
   return SFL_OK;
 }
@@ -761,6 +820,12 @@ int sfl_describe_launch(void *ctx, int mode, int traced, char *buf, int cap) {
   const int kind = trace ? K_FULL : (mode == SFL_MODE_GREEDY ? K_GREEDY : K_LEARN);
   LaunchPlan lp;
   if (plan_launch(c, kind, &lp)) return SFL_E_ARG;
+  if (c->cfg.eval_q) {                                 // the only kernel of an evaluation context (sfl_run refuses the rest)
+    if (kind != K_GREEDY) return fail(SFL_E_ARG, "an evaluation context (eval_q) runs SFL_MODE_GREEDY only, without traces or the phase clock%s");
+    snprintf(buf, (size_t)cap, "k_eval<G=%d,KIND=greedy,TH=%d,SQ=0,ONE=%d,ROOMY=0%s,EVQ=1> grid=%d block=%d smem=%zu", lp.G, lp.th, lp.one,
+             lp.nw > 1 ? ",NW=2" : "", lp.grid, lp.threads, lp.smem);
+    return SFL_OK;
+  }
   static const char *kinds[] = {"learn", "greedy", "full"};
   snprintf(buf, (size_t)cap, "k_run<G=%d,KIND=%s,TH=%d,SQ=%d,ONE=%d,ROOMY=%d%s> grid=%d block=%d smem=%zu", lp.G, kinds[kind], lp.th,
            c->cfg.shared_q ? 1 : 0, lp.one, lp.roomy, lp.nw > 1 ? ",NW=2" : "", lp.grid, lp.threads, lp.smem);
@@ -777,7 +842,7 @@ int sfl_reset(void *ctx, int keep, void *stream) {
   if (!c) return fail(SFL_E_ARG, "null ctx%s");
   if (!c->bound) return fail(SFL_E_STATE, "sfl_bind first%s");
   DeviceGuard dg(c->device);
-  InitArgs ia; ia.L = c->L; ia.state = (char *)c->bufs.state; ia.hp = (const sfl_hparams *)c->bufs.hparams; ia.n_envs = c->cfg.n_envs; ia.keep_q = keep & 1; ia.keep_ninter = (keep >> 1) & 1; ia.pad = 0;
+  InitArgs ia; ia.L = c->L; ia.state = (char *)c->bufs.state; ia.hp = (const sfl_hparams *)c->bufs.hparams; ia.n_envs = c->cfg.n_envs; ia.keep_q = keep & 1; ia.keep_ninter = (keep >> 1) & 1; ia.no_q = c->cfg.eval_q;
   CK(dev_zero(c->bufs.counters, (size_t)c->cfg.n_envs * sizeof(sfl_env_counters), stream));
 #ifndef SFL_HOST_EMUL
   int grid = (c->cfg.n_envs + SFL_WARPS_PER_CTA - 1) / SFL_WARPS_PER_CTA;
@@ -794,6 +859,7 @@ int sfl_reapply_q_init(void *ctx, void *stream) {
   if (!c) return fail(SFL_E_ARG, "null ctx%s");
   if (!c->bound) return fail(SFL_E_STATE, "sfl_bind first%s");
   if (c->cfg.shared_q) return fail(SFL_E_STATE, "shared-table mode keeps no per-environment tables%s");
+  if (c->cfg.eval_q) return fail(SFL_E_STATE, "an evaluation context (eval_q) keeps no per-environment tables: put the optimistic rows into the evaluation table%s");
   DeviceGuard dg(c->device);
   ReinitArgs a;
   a.L = c->L; a.sw = c->m.sw; a.port = c->m.port; a.qinit = c->m.qinit; a.state = (char *)c->bufs.state;
@@ -823,6 +889,12 @@ int sfl_run(void *ctx, int mode, int max_ticks, void *stream) {
   if ((mode == SFL_MODE_REPLAY || mode == SFL_MODE_STEP) && (!c->bufs.replay_act || c->cfg.act_cap < 1))
     return fail(SFL_E_ARG, "replay / step mode needs replay_act (act_cap >= 1)%s");
   if (mode == SFL_MODE_STEP && !c->bufs.step_out) return fail(SFL_E_ARG, "step mode needs step_out%s");
+  if (c->cfg.eval_q) {
+    if (mode != SFL_MODE_GREEDY)
+      return fail(SFL_E_ARG, "an evaluation context (eval_q) runs SFL_MODE_GREEDY only: learn, replay and step mode need per-environment tables%s");
+    if (c->cfg.dec_cap > 0 || c->cfg.tick_cap > 0 || c->phase_clock)
+      return fail(SFL_E_ARG, "an evaluation context (eval_q) has no traced or instrumented kernel (dec_cap, tick_cap, phase clock)%s");
+  }
   DeviceGuard dg(c->device);
   KArgs K;
   memset(&K, 0, sizeof(K));
@@ -841,6 +913,7 @@ int sfl_run(void *ctx, int mode, int max_ticks, void *stream) {
   ra.replay_act = (const int8_t *)c->bufs.replay_act;
   ra.step_out = (sfl_step_rec *)c->bufs.step_out;
   if (c->cfg.shared_q) { ra.sq_q = (double *)c->bufs.shared_q; ra.sq_d = (long long *)c->bufs.shared_d; ra.sq_c = (int *)c->bufs.shared_c; }
+  if (c->cfg.eval_q) ra.eval_q = (const double *)c->bufs.eval_q;
   // recorded malfunction events replace the Philox draws in replay mode, and in greedy / step mode when a schedule was bound (ev_cap > 0)
   // -- and in learn mode with the reference's stream or flatland's malfunction schedule, whose learn runs use the full kernel
   const int ref_learn = mode == SFL_MODE_LEARN && (c->cfg.rng == SFL_RNG_REFERENCE || c->cfg.malf_rng == SFL_MALF_REFERENCE);
@@ -856,14 +929,17 @@ int sfl_run(void *ctx, int mode, int max_ticks, void *stream) {
   if (c->cfg.shared_q && trace) return fail(SFL_E_ARG, "shared-table mode has no trace / step variants%s");
   const int grid = lp.grid, threads = lp.threads;
   const size_t smem = lp.smem;
-  run_kernel_t k = pick_kernel(lp.G, kind, lp.th, c->cfg.shared_q, lp.one, lp.roomy, lp.nw);
+  run_kernel_t k = c->cfg.eval_q ? pick_eval(lp.G, lp.th, lp.one, lp.nw) : pick_kernel(lp.G, kind, lp.th, c->cfg.shared_q, lp.one, lp.roomy, lp.nw);
   CU(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   k<<<grid, threads, smem, (cudaStream_t)stream>>>(K);
   CU(cudaGetLastError());
 #else
   static thread_local char host_scratch[32 * SFL_MAX_T + 2 * SFL_MAX_T + 64];
   for (int i = 0; i < c->cfg.n_envs; i++) {
-    if (c->cfg.shared_q) {
+    if (c->cfg.eval_q) {
+      if (c->L.T > 64) env_run<1, K_GREEDY, true, false, false, 2, true>(K, i, 0u, host_scratch);
+      else env_run<1, K_GREEDY, true, false, false, 1, true>(K, i, 0u, host_scratch);
+    } else if (c->cfg.shared_q) {
       if (trace) return fail(SFL_E_ARG, "shared-table mode has no trace / step variants%s");
       if (kind == K_GREEDY) env_run<1, K_GREEDY, true, true, false>(K, i, 0u, host_scratch); else env_run<1, K_LEARN, true, true, false>(K, i, 0u, host_scratch);
     } else if (c->L.T > 64) {
@@ -966,6 +1042,7 @@ int sfl_export_q(void *ctx, int env, uint32_t *keys_host, double *vals_host, int
   Ctx *c = (Ctx *)ctx;
   if (!c || !c->bound) return fail(SFL_E_STATE, "sfl_bind first%s");
   DeviceGuard dg(c->device);
+  if (c->cfg.eval_q) return fail(SFL_E_STATE, "an evaluation context (eval_q) keeps no per-environment tables%s");
   if (env < 0 || env >= c->cfg.n_envs || !n_rows) return fail(SFL_E_ARG, "bad env / n_rows%s");
   const Layout &L = c->L;
   size_t n = (size_t)L.q_cap * L.q_stride;
@@ -990,31 +1067,34 @@ int sfl_import_q(void *ctx, int env, const uint32_t *keys_host, const double *va
   Ctx *c = (Ctx *)ctx;
   if (!c || !c->bound) return fail(SFL_E_STATE, "sfl_bind first%s");
   DeviceGuard dg(c->device);
+  if (c->cfg.eval_q) return fail(SFL_E_STATE, "an evaluation context (eval_q) keeps no per-environment tables: use sfl_set_eval_table%s");
   if (env < 0 || env >= c->cfg.n_envs || n_rows < 0 || n_rows >= c->cfg.q_cap) return fail(SFL_E_ARG, "bad env / n_rows%s");
   const Layout &L = c->L;
-  size_t n = (size_t)L.q_cap * L.q_stride;
-  std::vector<double> img(n, 0.0);
-  unsigned mask = (unsigned)L.q_cap - 1u;
-  int distinct = 0;
-  for (int r = 0; r < n_rows; r++) {
-    unsigned key = keys_host[r];
-    unsigned i = (key * 2654435761u) >> 7;
-    for (;;) {
-      i &= mask;
-      unsigned long long k;
-      memcpy(&k, &img[(size_t)i * L.q_stride], 8);
-      if (k == 0) distinct++;
-      if (k == 0 || k == (unsigned long long)key + 1ull) break;
-      i++;
-    }
-    unsigned long long k = (unsigned long long)key + 1ull;
-    memcpy(&img[(size_t)i * L.q_stride], &k, 8);
-    for (int a = 0; a < L.a_max; a++) img[(size_t)i * L.q_stride + 1 + a] = vals_host[(size_t)r * L.a_max + a];
-  }
+  std::vector<double> img;
+  int q_rows = q_image(L, keys_host, vals_host, n_rows, img);     // repeated keys overwrite their row
   char *base = (char *)c->bufs.state + (size_t)env * L.env_stride;
-  CK(h2d(base + L.off_q, img.data(), n * 8, stream));
-  int q_rows = distinct;                         // repeated keys overwrite their row
+  CK(h2d(base + L.off_q, img.data(), img.size() * 8, stream));
   CK(h2d(base + offsetof(EnvHdr, q_rows), &q_rows, 4, stream));
+#ifndef SFL_HOST_EMUL
+  CU(cudaStreamSynchronize((cudaStream_t)stream));
+#endif
+  return SFL_OK;
+}
+
+int sfl_set_eval_table(void *ctx, const uint32_t *keys_host, const double *vals_host, int n_rows, void *stream) {
+  Ctx *c = (Ctx *)ctx;
+  if (!c || !c->bound) return fail(SFL_E_STATE, "sfl_bind first%s");
+  if (!c->cfg.eval_q) return fail(SFL_E_STATE, "the context was not created as an evaluation context (eval_q)%s");
+  if (n_rows < 0 || (n_rows && (!keys_host || !vals_host))) return fail(SFL_E_ARG, "bad keys / values / n_rows%s");
+  if (n_rows >= c->cfg.q_cap) {
+    char detail[96];
+    snprintf(detail, sizeof(detail), "%d rows, q_cap is %d", n_rows, c->cfg.q_cap);
+    return fail(SFL_E_NOMEM, "the evaluation table needs q_cap above its row count (a power of two; an empty slot ends every probe): %s", detail);
+  }
+  DeviceGuard dg(c->device);
+  std::vector<double> img;
+  q_image(c->L, keys_host, vals_host, n_rows, img);
+  CK(h2d(c->bufs.eval_q, img.data(), img.size() * 8, stream));
 #ifndef SFL_HOST_EMUL
   CU(cudaStreamSynchronize((cudaStream_t)stream));
 #endif

@@ -9,7 +9,7 @@
 // their predicates (see Grp below).  The per-tick train phase is lane-parallel inside the group (lane = train, in
 // chunks of G when T > G); the per-decision phase is inherently serial inside an environment (every _apply_action
 // mutates the semaphores the next observe reads, switch_env.py:648) and runs on the group's first lane -- for all
-// groups of the warp at once.  What a launch cannot need is compiled out (kernel KIND, TH, SQ, ONE: DESIGN.md section 4).
+// groups of the warp at once.  What a launch cannot need is compiled out (kernel KIND, TH, SQ, ONE, EVQ: DESIGN.md section 4).
 //
 // The same source compiles for a single "lane" on the host: tests/emul builds it with g++ (-DSFL_HOST_EMUL) to
 // unit-test the logic on the CPU box that has no GPU.  That build is test infrastructure; the product library
@@ -212,6 +212,7 @@ struct RunArgs {           // per-launch arguments
   sfl_step_rec *step_out;
   double *sq_q; long long *sq_d; int *sq_c;           // shared-table mode (null otherwise): table, delta sums (2^-24), delta counts
   const int8_t *replay_act; const int *replay_ev;     // ev: [env][ev_cap][3] = (tick, train, duration), tick-sorted, tick<0 ends
+  const double *eval_q;                               // evaluation contexts (EVQ kernels): the one read-only table; null otherwise
 };
 
 // Map constants, env-block layout and launch arguments travel as ONE __grid_constant__ kernel parameter (constant bank,
@@ -237,6 +238,7 @@ SFL_FN char *hot_ptr(hot_t o) { return o; }
 // Q-row functions cost the private-table kernels 20-25 % on large maps (registers / code size at 72 registers)
 template <bool TH, bool SQ_ = false> struct EnvT {
   static const bool SQ = SQ_;
+  static const bool EVQ = false;           // EnvEval: greedy decisions read the evaluation table
   static const bool HOT_TAIL = TH;
   static const int NW = 1;                 // 64-bit words per train set (EnvW: 2)
   const KArgs *kp;         // the launch's parameter block (methods below read the layout through it)
@@ -270,8 +272,12 @@ template <bool TH, bool SQ_ = false> struct EnvT {
 // template argument of EnvT, so that the types -- and the out-of-line callees named after them -- of the one-word
 // kernels stay exactly what they were
 template <bool TH, bool SQ_ = false> struct EnvW : EnvT<TH, SQ_> { static const int NW = 2; };
-template <bool TH, bool SQ, int NW> struct EnvOf { typedef EnvT<TH, SQ> type; };
-template <bool TH, bool SQ> struct EnvOf<TH, SQ, 2> { typedef EnvW<TH, SQ> type; };
+// EVQ ("evaluation table"): the environment of an evaluation context (sfl_config.eval_q), which has no Q region of its own;
+// its greedy decisions probe the one read-only table of the launch (eval_action).  A wrapper type, for the same reason as EnvW
+template <class Base> struct EnvEval : Base { static const bool EVQ = true; };
+template <bool TH, bool SQ, int NW, bool EVQ = false> struct EnvOf { typedef EnvT<TH, SQ> type; };
+template <bool TH, bool SQ> struct EnvOf<TH, SQ, 2, false> { typedef EnvW<TH, SQ> type; };
+template <bool TH, int NW> struct EnvOf<TH, false, NW, true> { typedef EnvEval<typename EnvOf<TH, false, NW>::type> type; };
 
 // the header's train sets as TSet<Env::NW>
 template <class Env> SFL_FN TSet<Env::NW> tset(const Env &e, int m) {
@@ -689,8 +695,8 @@ SFL_NI void q_update(SFL_K, Env e, const Hp hp, unsigned key, int action, double
   row[action] = nq;
 }
 
-// distr_q.py:468-490 max_action
-SFL_FN int max_action(const double *row, int A, int mask) {
+// distr_q.py:468-490 max_action (Row: a plain pointer, or RO<double> for the evaluation table)
+template <class Row> SFL_FN int max_action_of(const Row row, int A, int mask) {
   int best = 0, b2 = -1;                       // first maximum over all actions / over the allowed ones (np.argmax)
   double bv = row[0], b2v = 0.0;
   if (mask & 1) { b2 = 0; b2v = bv; }
@@ -701,6 +707,27 @@ SFL_FN int max_action(const double *row, int A, int mask) {
     if (((mask >> a) & 1) && (b2 < 0 || v > b2v)) { b2v = v; b2 = a; }
   }
   return ((mask >> best) & 1) ? best : b2;
+}
+SFL_FN int max_action(const double *row, int A, int mask) { return max_action_of(row, A, mask); }
+
+// EVQ: the greedy decision on the evaluation table -- the probe of q_row (same hash, linear probing) on the launch's one
+// read-only table, loaded through the non-coherent path; nothing is inserted.  A missing row reads as the default row
+// (default_q x A): max_action of A equal values is the lowest allowed action, the decision test() makes after inserting
+// that row (distr_q.py:482 -> :56-57).  The table always has an empty slot (sfl_set_eval_table: rows < q_cap).
+SFL_FN int eval_action(SFL_K, unsigned key, int A, int mask) {
+  const unsigned qmask = (unsigned)c_L.q_cap - 1u;
+  const unsigned long long want = (unsigned long long)key + 1ull;
+  unsigned i = (key * 2654435761u) >> 7;
+  SFL_NU
+  for (int probe = 0; probe < c_L.q_cap; probe++) {
+    i &= qmask;
+    const double *row = c_ra.eval_q + (size_t)i * c_L.q_stride;
+    const unsigned long long k = ldg((const unsigned long long *)row);
+    if (k == want) { RO<double> r; r.p = row + 1; return max_action_of(r, A, mask); }
+    if (k == 0ull) break;
+    i++;
+  }
+  return ffs64((unsigned long long)((unsigned)mask & ((1u << A) - 1u)));
 }
 
 // ------------------------------------------------------------------------------------------------ E3
@@ -979,8 +1006,11 @@ SFL_FN void decide(SFL_K, Env e, const Hp hp, int env_id, int t, const int semb_
     }
   }
   if (action < 0) {                                        // exploit (distr_q.py:318-319) / test() (:211)
-    my_row = q_row(K, e, hp, key);
-    action = max_action(my_row, A, mask);
+    if (Env::EVQ) action = eval_action(K, key, A, mask);
+    else {
+      my_row = q_row(K, e, hp, key);
+      action = max_action(my_row, A, mask);
+    }
   }
   SFL_PHASE_MARK(h, PH_ACT);
   // ---- apply (switch_env.py:203-294, switch_agents.py:136-168)
@@ -1460,7 +1490,7 @@ SFL_FN void step_report(SFL_K, Env e, int env_id, int t) {
   o->arrived_hi = Env::NW > 1 ? *e.hw1(HM_DONE) : 0ull;
 }
 
-template <int G, int KIND, bool TH, bool SQ, bool ONE, int NW = 1>
+template <int G, int KIND, bool TH, bool SQ, bool ONE, int NW = 1, bool EVQ = false>
 SFL_FN void env_run(SFL_K, int env_id, unsigned stage, char *host_scratch) {
   const bool TRACE = KIND == K_FULL;
   const Grp<G> g;
@@ -1468,7 +1498,7 @@ SFL_FN void env_run(SFL_K, int env_id, unsigned stage, char *host_scratch) {
   if (!valid) env_id = 0;
   char *gbase = c_ra.state + (size_t)env_id * c_L.env_stride;
   const unsigned hot_bytes = valid ? c_ra.hot_bytes : 0u;
-  typename EnvOf<TH, SQ, NW>::type e;
+  typename EnvOf<TH, SQ, NW, EVQ>::type e;
   Hp hp;
   Scratch sc;
   e.kp = &K; sc.kp = &K;
