@@ -191,12 +191,12 @@ struct EnvHdr {
 
 // Per-train records (16 bytes each, one vector load per phase):
 //   TrA {pos, dir | state<<8 | saved<<16 | prev_act<<24, plan (4 bits per entry, head lowest) | plan_len<<16, malf (u16) | next_port<<16}
-//   TrB {prev_port (u16) | source_port<<16 (0xFFFF = none), act_switch (u16) | pend_n<<16, last_delay, 0}
+//   TrB {prev_port (u16) | source_port<<16 (0xFFFF = none), act_switch (u16) | pend_n<<16, last_delay, stop_tick}
+//   stop_tick: the last tick of the episode the train ended STOPPED or MALFUNCTION (SFL_NO_STOP: none yet; see t0_eff)
 // Per-switch record SwS {interactions, 0, eps_pow (f64) = epsilon_decay_rate ** interactions}.
 // Pending update (distr_q.py:340-342): {key, next_sw | prev_sw<<12 | action<<24}; part of the tail (decision phase only).
 // Semaphore record (rail_network.py:133 [train, in/out, dir, t0, t1]): {t0, t1 - t0, train (-1 = absent), type} -- start
-// and LENGTH of the window, so that extend_semaphores (rail_network.py:229-244: slide the window to start now, keep its
-// length) is one 4-byte store per record and needs no load.
+// as written and LENGTH of the window; the window starts at t0_eff, the start with extend_semaphores applied.
 struct SwS { int ninter, pad; double eps_pow; };
 enum { HM_ACTIVE = 0, HM_MALF = 1, HM_DEST = 2, HM_DONE = 3 };   // the header's train sets: active, malf_prev, at_dest, done
 
@@ -261,6 +261,7 @@ template <bool TH, bool SQ_ = false> struct EnvT {
   SFL_FN int owner(int p) const { return TH ? sem()[p].z : (int)(int8_t)own_ptr()[p]; }
   SFL_FN void sem_put(int p, int4 r) const { sem()[p] = r; if (!TH) own_ptr()[p] = (uint8_t)r.z; }
   SFL_FN void sem_drop(int p) const { sem()[p].z = -1; if (!TH) own_ptr()[p] = 0xFFu; }
+  SFL_FN int stop_tick(int t) const { return trb()[t].w; }
   // header train set m (HM_*): word 0 in EnvHdr, word 1 (EnvW) right after it
   SFL_FN unsigned long long &hw0(int m) const {
     EnvHdr *x = h();
@@ -574,6 +575,15 @@ SFL_FN Mv check_action(SFL_K, int action, int cell, int dir) { return mv_apply(K
 SFL_FN int is_moving(int a) { return a >= A_LEFT && a <= A_RIGHT; }
 
 // ------------------------------------------------------------------------------------------------ E4
+// extend_semaphores (rail_network.py:229-244) slides every record held by a train that ends a tick STOPPED or MALFUNCTION
+// to start at that tick, keeping its length.  The kernel stores only the tick, in the holder's TrB.stop_tick, and every
+// reader of a window start takes the later of the two.  Exact, because every writer of a record sets t0 to the current
+// tick (transition_semaphore: now; the departure booking: ed - 2 == now; the MALFUNCTION booking: now) and no stamp is
+// later than the current tick: a record written after its holder's last stop has t0 >= stop_tick, one written before it
+// was slid to exactly that tick.  The reset bookings' t0 = ed - 2 precedes every stop of their holder, and may be
+// negative (ed < 2), so the stamp of a train that has not stopped this episode is SFL_NO_STOP, below every t0.
+#define SFL_NO_STOP (-0x7FFFFFFF - 1)
+SFL_FN int t0_eff(int t0, int stop_tick) { return t0 > stop_tick ? t0 : stop_tick; }
 // observer.py:44-151 check_port_blocked.  Every writer of a semaphore record stores dir == map_direction(port)
 // (rail_network.py:243,327,337,372,382,396,408; switch_env.py:382,566), so the eight clauses reduce to:
 //   rule_next: 'out' -> blocked, 'in' -> blocked iff holder MALFUNCTION;  rule_out: 'in' -> blocked, 'out' -> iff MALFUNCTION.
@@ -582,15 +592,18 @@ SFL_FN int tr_state(Env e, int t) { return (e.tra()[t].y >> 8) & 0xFF; }
 template <class Env>
 SFL_FN int rule_port(Env e, int port, int me, int now, int blocking_type) {
   int4 r;
+  int stamp;
   if (Env::HOT_TAIL) {                                                        // staged table: one shared-memory load
     r = e.sem()[port];
-    if (r.z < 0 || r.z == me || r.x > now || r.x + r.y < now) return 0;
+    if (r.z < 0 || r.z == me) return 0;
+    stamp = e.stop_tick(r.z);
   } else {                                                              // table in HBM: ask the holder mirror first
     const int holder = e.owner(port);
     if (holder < 0 || holder == me) return 0;
     r = e.sem()[port];
-    if (r.x > now || r.x + r.y < now) return 0;
+    stamp = e.stop_tick(holder);                                        // shared memory: in flight with the record's load
   }
+  if (r.x > now || t0_eff(r.x, stamp) + r.y < now) return 0;           // t0_eff > now iff t0 > now: no stamp is later than now
   if (r.w == blocking_type) return 1;
   return tr_state(e, r.z) == ST_MALF;
 }
@@ -741,7 +754,8 @@ SFL_FN void sem_delete_owned(SFL_K, Env e, int port, int h) {
   }
 }
 
-// rail_network.py:303-416 transition_semaphore, step by step
+// rail_network.py:303-416 transition_semaphore, step by step.  Its window-start tests `t0 > now` read the stored t0: no stop
+// stamp is later than now, so t0_eff(r) > now exactly when t0 > now.
 template <class Env>
 SFL_FN void transition_semaphore(SFL_K, Env e, int source, int out_port, int target, int h, int now, int st, int old_next, int old_prev) {
   if (st != ST_MALF) {                                                  // :315-323
@@ -851,7 +865,11 @@ SFL_FN void finish_decision(SFL_K, Env e, const Hp hp, int env_id) {
       if (c_ra.trace_sem_buf) {
         int4 *dst = c_ra.trace_sem_buf + ((size_t)env_id * c_ra.dec_cap + h->cur_dec) * c_L.NP;
         SFL_NU
-        for (int p = 0; p < c_L.NP; p++) { int4 r = e.sem()[p]; r.y += r.x; dst[p] = r; }      // traced as {t0, t1, train, type}
+        for (int p = 0; p < c_L.NP; p++) {                                                       // traced as {t0, t1, train, type}
+          int4 r = e.sem()[p];
+          if (r.z >= 0) r.x = t0_eff(r.x, e.stop_tick(r.z));
+          r.y += r.x; dst[p] = r;
+        }
       }
     }
     h->cur_dec = -1;
@@ -1124,7 +1142,7 @@ SFL_RARE void env_reset(SFL_K, Env e, const Grp<G> &g, int on) {
     e.tra()[t] = make_int4(-1, tr0.y | (ST_WAITING << 8) | (0 << 16) | (A_NONE << 24), 0, (int)((unsigned)tr1.z << 16));
     int4 b = e.trb()[t];
     // prev_port / source_port are NOT cleared: RailNetwork.reset (rail_network.py:135-149) keeps them
-    e.trb()[t] = make_int4(b.x, 0xFFFF, c_m.init_delay[t], 0);
+    e.trb()[t] = make_int4(b.x, 0xFFFF, c_m.init_delay[t], SFL_NO_STOP);
   }
   SFL_NU
   for (int p = g.gl; p < NP; p += G) e.sem_put(p, make_int4(0, 0, -1, 0));
@@ -1288,12 +1306,12 @@ SFL_FN void env_tick(SFL_K, Env e, Scratch sc, const Hp hp, int env_id, const Gr
   }
   // ---- phase C: state machine + position update (Appendix B steps 4-5), held-back trains (switch_env.py:353-367),
   //      and _check_active_switch (switch_env.py:427-485), which reads only the train's own new state
-  TSet<Env::NW> done_bits, malf_bits, stopped_bits, depart_bits, active;
-  done_bits.clear(); malf_bits.clear(); stopped_bits.clear(); depart_bits.clear(); active.clear();
+  TSet<Env::NW> done_bits, malf_bits, broken_bits, depart_bits, active;      // broken: ended the tick in state MALFUNCTION
+  done_bits.clear(); malf_bits.clear(); broken_bits.clear(); depart_bits.clear(); active.clear();
   SFL_NU
   for (int base = 0; base < (ONE ? 1 : Tw); base += (ONE ? 1 : G)) {
     const int t = base + g.gl;
-    int f_done = 0, f_malf = 0, f_stop = 0, f_dep = 0, f_act = 0;
+    int f_done = 0, f_malf = 0, f_broken = 0, f_dep = 0, f_act = 0;
     if (t < T) {
       int4 ta = e.tra()[t];
       const int4 m = sc.tmp()[t];
@@ -1328,7 +1346,8 @@ SFL_FN void env_tick(SFL_K, Env e, Scratch sc, const Hp hp, int env_id, const Gr
       if (nxt == ST_DONE) p = -1;
       if (mc > 0) mc--;
       if (p >= 0) saved = 0;
-      f_done = nxt == ST_DONE; f_malf = mc != 0; f_stop = nxt == ST_STOPPED || nxt == ST_MALF; f_dep = now == ed - 2;
+      f_done = nxt == ST_DONE; f_malf = mc != 0; f_broken = nxt == ST_MALF; f_dep = now == ed - 2;
+      if (nxt == ST_STOPPED || nxt == ST_MALF) e.trb()[t].w = now;        // extend_semaphores (rail_network.py:229-244): t0_eff
       if (TRACE) {
         if (c_ra.trace_tick && h->n_tick_logged < c_ra.tick_cap) {
           sfl_tick_rec *rec = c_ra.trace_tick + ((size_t)env_id * c_ra.tick_cap + h->n_tick_logged) * T + t;
@@ -1366,7 +1385,7 @@ SFL_FN void env_tick(SFL_K, Env e, Scratch sc, const Hp hp, int env_id, const Gr
     }
     done_bits.or_ballot(g.ballot(f_done), base);
     malf_bits.or_ballot(g.ballot(f_malf), base);
-    stopped_bits.or_ballot(g.ballot(f_stop), base);
+    broken_bits.or_ballot(g.ballot(f_broken), base);
     depart_bits.or_ballot(g.ballot(f_dep), base);
     active.or_ballot(g.ballot(f_act), base);
   }
@@ -1382,10 +1401,11 @@ SFL_FN void env_tick(SFL_K, Env e, Scratch sc, const Hp hp, int env_id, const Gr
       if (tr >= 0 && (ended || done_bits.test(tr))) e.sem_drop(p);
     }
   }
-  // ---- phase D3: departure bookings (switch_env.py:379-384), train order
-  if (g.wany(depart_bits.any())) {
+  // ---- phase D3: departure bookings (switch_env.py:379-384), then the bookings of extend_semaphores for trains in
+  //      MALFUNCTION (rail_network.py:229-244; the slide of the stopped trains' windows is their stop_tick), train order
+  if (g.wany(depart_bits.any() || broken_bits.any())) {
     g.sync();
-    if (depart_bits.any() && g.gl == 0) {
+    if (g.gl == 0) {
       TSet<Env::NW> b = depart_bits;
       SFL_NU
       while (b.any()) {
@@ -1393,33 +1413,12 @@ SFL_FN void env_tick(SFL_K, Env e, Scratch sc, const Hp hp, int env_id, const Gr
         int4 tr1 = c_m.train1[t];
         e.sem_put((int)((unsigned)e.tra()[t].w >> 16), make_int4(tr1.x - 2, tr1.w + 2, t, SEM_IN));
       }
-    }
-  }
-  // ---- phase D4: extend_semaphores (rail_network.py:229-244)
-  if (g.wany(stopped_bits.any())) {
-    g.sync();
-    const int NP = stopped_bits.any() ? c_L.NP : 0;
-    SFL_NU
-    for (int p = g.gl; p < NP; p += G) {
-      if (Env::HOT_TAIL) {
-        int4 r = e.sem()[p];
-        if (r.z >= 0 && stopped_bits.test(r.z)) e.sem()[p].x = now;
-      } else {
-        const int holder = e.owner(p);                                   // only the records of stopped trains leave shared memory
-        if (holder >= 0 && stopped_bits.test(holder)) e.sem()[p].x = now;      // a 4-byte store, no load
-      }
-    }
-    g.sync();
-    if (stopped_bits.any() && g.gl == 0) {
-      TSet<Env::NW> b = stopped_bits;
+      b = broken_bits;
       SFL_NU
       while (b.any()) {
         int t = b.pop();
-        int4 ta = e.tra()[t];
-        if (((ta.y >> 8) & 0xFF) == ST_MALF) {
-          int port = (int)((unsigned)ta.w >> 16);
-          if (e.owner(port) < 0) e.sem_put(port, make_int4(now, c_m.train1[t].w, t, SEM_IN));
-        }
+        int port = (int)((unsigned)e.tra()[t].w >> 16);
+        if (e.owner(port) < 0) e.sem_put(port, make_int4(now, c_m.train1[t].w, t, SEM_IN));
       }
     }
   }
