@@ -329,6 +329,17 @@ int sfl_total_decisions(void *ctx, uint64_t *decisions, uint64_t *ticks, void *s
 
 /* Q-table export for distr_q_model.pkl (distr_q.py:492-523): rows of env `env` as (key, A_max values) */
 int sfl_export_q(void *ctx, int env, uint32_t *keys_host, double *vals_host, int cap_rows, int *n_rows, void *stream);
+/* Q-table export of environments env_lo .. env_hi - 1 at once, on the device (the checkpoints of distr_q.py:288-294 for every
+ * learner of a batch).  DEVICE pointers: row_offsets[env_hi - env_lo + 1], the caller's exclusive scan of the environments'
+ * q_rows (sfl_env_counters after the last sfl_run); keys[cap_rows], vals[cap_rows * a_max]; rows_found[env_hi - env_lo].
+ * Environment env_lo + j's rows go to rows row_offsets[j] .. row_offsets[j + 1] - 1, in the slot order of sfl_export_q,
+ * as (key, a_max values); rows_found[j] = the occupied slots the table holds.  A count that differs from q_rows means a
+ * corrupted table: the rows past the environment's range are not written, and the caller should raise.  Deterministic
+ * (no atomics).  Reads row_offsets[env_hi - env_lo] back first (8 bytes, waits for `stream`) and fails with SFL_E_NOMEM
+ * when it exceeds cap_rows; the compaction itself is only enqueued on `stream`, so the caller can overlap the copy-out.
+ * SFL_E_ARG for a range outside 0 <= env_lo <= env_hi <= n_envs; refused by evaluation contexts like sfl_export_q.     */
+int sfl_export_q_batch(void *ctx, int env_lo, int env_hi, const uint64_t *row_offsets, uint32_t *keys, double *vals,
+                       uint64_t cap_rows, int32_t *rows_found, void *stream);
 /* Q-table import (distr_q.py:510-527 load) */
 int sfl_import_q(void *ctx, int env, const uint32_t *keys_host, const double *vals_host, int n_rows, void *stream);
 /* sfl_config.eval_q: fill the bound evaluation table with n_rows (key, A_max values) rows -- the hash image sfl_import_q

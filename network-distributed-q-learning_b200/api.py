@@ -16,8 +16,10 @@ from __future__ import annotations
 
 import os
 import pickle
+import queue
+import threading
 import time
-from typing import Dict, List, Optional, Sequence
+from typing import Dict, Iterator, List, Optional, Sequence
 
 import numpy as np
 
@@ -230,8 +232,76 @@ class ASyncSwitchEnv:
         pass
 
 
+class _CheckpointWriter:
+    """The thread that writes learn()'s checkpoint files while the next episodes run.  Each checkpoint fills one of two host
+    staging buffers (``staging()`` waits while both are still being written) and hands the writer a job that reads it.
+    ``overlap``: True runs the jobs on the thread, False in the caller at ``submit`` (a run that waits at every checkpoint),
+    None: no checkpoints.  Leaving the ``with`` block waits for the jobs and re-raises the first exception of one; when the
+    block itself raises (an error of learn(), KeyboardInterrupt), the jobs not yet started are dropped instead of written."""
+
+    def __init__(self, overlap: Optional[bool]):
+        self.free: "queue.Queue[dict]" = queue.Queue()
+        for _ in range(2):
+            self.free.put({})
+        self.jobs: "queue.Queue" = queue.Queue()
+        self.errors: List[BaseException] = []
+        self.cancelled = False
+        self.thread = threading.Thread(target=self._work, daemon=True) if overlap else None
+        if self.thread is not None:
+            self.thread.start()
+
+    def staging(self) -> dict:
+        return self.free.get()
+
+    def submit(self, job, staging: dict):
+        if self.errors:
+            raise self.errors[0]
+        if self.thread is not None:
+            self.jobs.put((job, staging))
+            return
+        try:
+            job()
+        finally:
+            self.free.put(staging)
+
+    def _work(self):
+        while True:
+            item = self.jobs.get()
+            if item is None:
+                return
+            job, staging = item
+            try:
+                if not self.errors and not self.cancelled:
+                    job()
+            except BaseException as ex:                # re-raised by submit() / __exit__ in learn()'s thread
+                self.errors.append(ex)
+            finally:
+                self.free.put(staging)
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, exc_type, exc, tb):
+        self.cancelled = exc_type is not None
+        if self.thread is not None:
+            self.jobs.put(None)
+            self.thread.join()
+        if exc_type is None and self.errors:
+            raise self.errors[0]
+        return False
+
+
+def _dump_q(q: Dict[tuple, List[float]], filename: str):
+    """distr_q.py:521-523: pickle the table with np.int64 key elements (observer.py:306)."""
+    q = {tuple(np.int64(x) for x in k): list(v) for k, v in q.items()}
+    with open(filename, "wb") as f:
+        pickle.dump(q, f)
+
+
 class DistrQLearning:
     """Batched counterpart of distr_q.py:11-527."""
+
+    _overlap_checkpoints = True              # False: learn() writes each checkpoint before it goes on (same files)
 
     def __init__(self, env: ASyncSwitchEnv, gamma=1.0, epsilon=0.4, epsilon_decay_rate=0.0, lr=0.4, lr_decay_rate=0.0,
                  default_q=0.0, seed=450565, seeds: Optional[Sequence[int]] = None, dist=None):
@@ -342,12 +412,21 @@ class DistrQLearning:
         return eng.counters()
 
     # ------------------------------------------------------------------ distr_q.py:244-379
-    def learn(self, num_episodes: int, out_dir: Optional[str], checkpoint_freq: int, exploit_freq: Optional[int] = None):
+    def learn(self, num_episodes: int, out_dir: Optional[str], checkpoint_freq: int, exploit_freq: Optional[int] = None,
+              env_out_dirs: Optional[Sequence[str]] = None):
+        """distr_q.py:244-379 for every environment at once.  ``out_dir`` gets the primary environment's files, as the
+        reference's.  ``env_out_dirs``: one directory per environment, each of which also gets its environment's checkpoint
+        files (checkpoint_N.pkl and the five *_checkpoint_N.npz of distr_q.py:288-294).  The checkpoints are written on a
+        thread of their own from one device-side compaction of every table while the next episodes run; learn() waits for
+        them before it returns and re-raises what failed there."""
         eng, env = self.env.engine, self.env
         B, T = env.n_envs, env.rail_map.trains.T
         p = self.primary_env
-        if out_dir:
-            os.makedirs(out_dir, exist_ok=True)
+        if env_out_dirs is not None and len(env_out_dirs) != B:
+            raise ValueError(f"env_out_dirs has {len(env_out_dirs)} directories for {B} environments")
+        targets = ([(p, out_dir)] if out_dir else []) + [(i, d) for i, d in enumerate(env_out_dirs or [])]
+        for _, d in targets:
+            os.makedirs(d, exist_ok=True)
         cum_reward = np.zeros((B, num_episodes))
         arrived = np.zeros((B, num_episodes), np.int32)
         delays = np.zeros((B, num_episodes, T))
@@ -359,44 +438,39 @@ class DistrQLearning:
                          if (exploit_freq and (t + 1) % exploit_freq == 0) or (checkpoint_freq and (t + 1) % checkpoint_freq == 0)}
                         | {num_episodes})
         done, first = 0, True
-        for cut in pauses:
-            while done < cut:                                   # run episodes [done, cut) in ep_cap-sized launches
-                seg = min(cut - done, eng.cfg.ep_cap)
-                self._hparams(seg, episode_base=done)
-                if first:
-                    t0 = time.time()
-                    eng.reset(keep_q=self._table_dirty, keep_interactions=False)     # agent_num_interactions is per learn() (:263)
-                    self._begin_tables(self._table_dirty)
-                    if self._table_dirty:
-                        self._apply_q_init_to_existing_rows()
-                    eng.enable_q_init(True)                                           # distr_q.py:299-300
-                    self._q_inited = True
-                    first = False
-                    env.reset_total_time += time.time() - t0
-                else:
-                    eng.reset(keep_q=True, keep_interactions=True)
-                self._run_until_halted(MODE_LEARN)
-                _, log, dl = eng.episode_log()
-                cum_reward[:, done:done + seg] = log["cum_reward"][:, :seg]
-                arrived[:, done:done + seg] = log["arrived"][:, :seg]
-                num_malf[:, done:done + seg] = log["num_malfunctions"][:, :seg]
-                last_mask = log[["arrived_mask", "arrived_mask_hi"]][:, seg - 1].copy()
-                delays[:, done:done + seg] = dl[:, :seg]
-                done += seg
-            if cut >= num_episodes:
-                break
-            if exploit_freq and (cut + 1) % exploit_freq == 0:
-                r, a, _ = self.test(out_dir=None, plot=False, save_outputs=False, _batched=True)
-                cum_reward_exploit.append(r)
-                arrived_exploit.append(a)
-            if checkpoint_freq and (cut + 1) % checkpoint_freq == 0 and out_dir:
-                self._q_stale = True
-                self.save(os.path.join(out_dir, f"checkpoint_{cut + 1}.pkl"))
-                np.savez_compressed(os.path.join(out_dir, f"cum_reward_checkpoint_{cut + 1}.npz"), x=cum_reward[p])
-                np.savez_compressed(os.path.join(out_dir, f"arrived_trains_checkpoint_{cut + 1}.npz"), x=arrived[p, :cut])
-                np.savez_compressed(os.path.join(out_dir, f"delays_checkpoint_{cut + 1}.npz"), x=delays[p, :cut])
-                np.savez_compressed(os.path.join(out_dir, f"trains_at_dest_checkpoint_{cut + 1}.npz"), x=[])   # SURVEY App. A #14
-                np.savez_compressed(os.path.join(out_dir, f"num_malfunctions_checkpoint_{cut + 1}.npz"), x=num_malf[p, :cut])
+        with _CheckpointWriter(self._overlap_checkpoints if targets and checkpoint_freq else None) as writer:
+            for cut in pauses:
+                while done < cut:                                   # run episodes [done, cut) in ep_cap-sized launches
+                    seg = min(cut - done, eng.cfg.ep_cap)
+                    self._hparams(seg, episode_base=done)
+                    if first:
+                        t0 = time.time()
+                        eng.reset(keep_q=self._table_dirty, keep_interactions=False)     # agent_num_interactions is per learn() (:263)
+                        self._begin_tables(self._table_dirty)
+                        if self._table_dirty:
+                            self._apply_q_init_to_existing_rows()
+                        eng.enable_q_init(True)                                           # distr_q.py:299-300
+                        self._q_inited = True
+                        first = False
+                        env.reset_total_time += time.time() - t0
+                    else:
+                        eng.reset(keep_q=True, keep_interactions=True)
+                    self._run_until_halted(MODE_LEARN)
+                    _, log, dl = eng.episode_log()
+                    cum_reward[:, done:done + seg] = log["cum_reward"][:, :seg]
+                    arrived[:, done:done + seg] = log["arrived"][:, :seg]
+                    num_malf[:, done:done + seg] = log["num_malfunctions"][:, :seg]
+                    last_mask = log[["arrived_mask", "arrived_mask_hi"]][:, seg - 1].copy()
+                    delays[:, done:done + seg] = dl[:, :seg]
+                    done += seg
+                if cut >= num_episodes:
+                    break
+                if exploit_freq and (cut + 1) % exploit_freq == 0:
+                    r, a, _ = self.test(out_dir=None, plot=False, save_outputs=False, _batched=True)
+                    cum_reward_exploit.append(r)
+                    arrived_exploit.append(a)
+                if checkpoint_freq and (cut + 1) % checkpoint_freq == 0 and targets:
+                    self._checkpoint(writer, targets, cut, cum_reward, arrived, delays, num_malf)
         self._table_dirty = True
         self._q_stale = True                 # q_table is read back from the device when it is next used
         at_dest = [train_set(mk["arrived_mask"], mk["arrived_mask_hi"], T) for mk in last_mask] if num_episodes else [[] for _ in range(B)]
@@ -412,12 +486,64 @@ class DistrQLearning:
             env.train_to_last_node = {h: (None, float(delays[p, -1, h])) for h in range(T)}
         env.close()
 
+    def _checkpoint(self, writer: _CheckpointWriter, targets, cut: int, cum_reward, arrived, delays, num_malf):
+        """distr_q.py:288-294 before episode ``cut`` for every (environment, directory) of ``targets``: the tables are
+        compacted on the device and copied out behind the launches already queued; the writer turns them into the files.
+        The metric rows [:cut] are final here, and cum_reward is zero from ``cut`` on, so the job reads them in place."""
+        eng = self.env.engine
+        envs = sorted({i for i, _ in targets})
+        include_init, dq = self._q_inited, {i: self._default_q_of(i) for i in envs}
+        staging = writer.staging()
+        if eng.shared_q:
+            shared = dict(zip(envs, eng.export_q_batch(envs, include_init, [dq[i] for i in envs])))
+        else:
+            snap = eng.compact_q(envs[0], envs[-1] + 1, staging)
+        n_ep = cum_reward.shape[1]
+
+        def job():
+            init = {}
+            if not eng.shared_q:
+                snap.wait()
+            # one table in memory at a time; the primary environment's is kept for its second directory only
+            uses = {i: sum(1 for j, _ in targets if j == i) for i in envs}
+            kept: Dict[int, Dict[tuple, List[float]]] = {}
+            for i, d in targets:
+                q = kept.pop(i, None)
+                if q is None and eng.shared_q:
+                    q = shared[i]
+                elif q is None:
+                    if include_init and dq[i] not in init:
+                        init[dq[i]] = self.env.rail_map.q_init_rows(dq[i])
+                    q = snap.table(i, init[dq[i]] if include_init else None)
+                uses[i] -= 1
+                if uses[i]:
+                    kept[i] = q
+                _dump_q(q, os.path.join(d, f"checkpoint_{cut + 1}.pkl"))
+                del q
+                np.savez_compressed(os.path.join(d, f"cum_reward_checkpoint_{cut + 1}.npz"),
+                                    x=np.concatenate([cum_reward[i, :cut], np.zeros(n_ep - cut)]))
+                np.savez_compressed(os.path.join(d, f"arrived_trains_checkpoint_{cut + 1}.npz"), x=arrived[i, :cut])
+                np.savez_compressed(os.path.join(d, f"delays_checkpoint_{cut + 1}.npz"), x=delays[i, :cut])
+                np.savez_compressed(os.path.join(d, f"trains_at_dest_checkpoint_{cut + 1}.npz"), x=[])   # SURVEY App. A #14
+                np.savez_compressed(os.path.join(d, f"num_malfunctions_checkpoint_{cut + 1}.npz"), x=num_malf[i, :cut])
+
+        writer.submit(job, staging)
+
+    def env_q_tables(self, envs: Optional[Sequence[int]] = None) -> Iterator[Dict[tuple, List[float]]]:
+        """The ``q_table`` of every environment of ``envs`` (consecutive indices, default all) -- the dicts ``save()``
+        pickles for that environment -- from one compaction of their tables on the device, built one at a time in the
+        order of ``envs`` (``Engine.iter_q_batch``), so that a caller writing them holds one table at a time."""
+        envs = list(range(self.env.n_envs) if envs is None else envs)
+        return self.env.engine.iter_q_batch(envs, include_init=self._q_inited, default_q=[self._default_q_of(i) for i in envs])
+
     def _default_q_of(self, i: int) -> float:
         d = np.asarray(self.default_q, np.float64).reshape(-1)
         return float(d[i % d.size])
 
-    def write_outputs(self, env_index: int, out_dir: str, exploit: bool = True, pkl: bool = True):
-        """The reference's end-of-learn files (distr_q.py:368-375, main.py:66) for environment ``env_index``."""
+    def write_outputs(self, env_index: int, out_dir: str, exploit: bool = True, pkl: bool = True,
+                      q_table: Optional[Dict[tuple, List[float]]] = None):
+        """The reference's end-of-learn files (distr_q.py:368-375, main.py:66) for environment ``env_index``.  ``q_table``:
+        the environment's table when the caller has it already (``env_q_tables``), else it is exported here."""
         m, i = self.metrics, env_index
         os.makedirs(out_dir, exist_ok=True)
         np.savez_compressed(os.path.join(out_dir, "cum_reward.npz"), x=m["cum_reward"][i])
@@ -428,7 +554,9 @@ class DistrQLearning:
         if exploit:
             np.savez_compressed(os.path.join(out_dir, "cum_reward_exploit.npz"), x=[r[i] for r in m["cum_reward_exploit"]])
             np.savez_compressed(os.path.join(out_dir, "arrived_trains_exploit.npz"), x=[a[i] for a in m["arrived_trains_exploit"]])
-        if pkl:
+        if pkl and q_table is not None:
+            _dump_q(q_table, os.path.join(out_dir, "distr_q_model.pkl"))
+        elif pkl:
             keep = self.q_table
             self.q_table = self.env.engine.export_q(i, include_init=self._q_inited, default_q=self._default_q_of(i))
             self.save(os.path.join(out_dir, "distr_q_model.pkl"))
@@ -561,9 +689,7 @@ class DistrQLearning:
     def save(self, filename: str, mode: str = "pickle"):
         if mode != "pickle":
             raise AttributeError("only mode='pickle' exists in the reference (distr_q.py:505-508 dispatch to undefined methods)")
-        q = {tuple(np.int64(x) for x in k): list(v) for k, v in self.q_table.items()}   # np.int64 key elements (observer.py:306)
-        with open(filename, "wb") as f:
-            pickle.dump(q, f)
+        _dump_q(self.q_table, filename)
 
     def load(self, filename: str):
         self.q_table = read_q_table(filename)
@@ -587,32 +713,33 @@ def read_q_table(filename: str) -> Dict[tuple, List[float]]:
 
 
 def learn_concurrently(models: Sequence[DistrQLearning], num_episodes: int, out_dirs: Optional[Sequence[Optional[str]]] = None,
-                       checkpoint_freq: int = 0, exploit_freq: Optional[int] = None) -> None:
+                       checkpoint_freq: int = 0, exploit_freq: Optional[int] = None,
+                       env_out_dirs: Optional[Sequence[Optional[Sequence[str]]]] = None) -> None:
     """``learn()`` of several independent learners (different maps / seeds) at the same time on one GPU: one host thread and
     one CUDA stream per learner, so that their kernel launches overlap.  This is hyperparam_tuning.py:85-91 -- every
     (point, seed) run started at once, no communication -- with streams in place of OS processes; the results are those of
-    calling ``learn()`` on each model in turn."""
-    import threading
+    calling ``learn()`` on each model in turn.  ``env_out_dirs``: one ``learn(env_out_dirs=...)`` list per model."""
     import torch
     out_dirs = list(out_dirs) if out_dirs is not None else [None] * len(models)
+    env_out_dirs = list(env_out_dirs) if env_out_dirs is not None else [None] * len(models)
     if torch.cuda.is_available():
         torch.cuda.synchronize()                       # buffers were created on the default stream
     errors: List[BaseException] = []
 
-    def work(m: DistrQLearning, out_dir: Optional[str]):
+    def work(m: DistrQLearning, out_dir: Optional[str], dirs: Optional[Sequence[str]]):
         try:
             dev = m.env.engine.device
             if dev.type == "cuda":
                 stream = torch.cuda.Stream(device=dev)
                 with torch.cuda.device(dev), torch.cuda.stream(stream):
-                    m.learn(num_episodes, out_dir, checkpoint_freq, exploit_freq)
+                    m.learn(num_episodes, out_dir, checkpoint_freq, exploit_freq, env_out_dirs=dirs)
                     stream.synchronize()
             else:
-                m.learn(num_episodes, out_dir, checkpoint_freq, exploit_freq)
+                m.learn(num_episodes, out_dir, checkpoint_freq, exploit_freq, env_out_dirs=dirs)
         except BaseException as ex:                    # re-raised in the caller's thread
             errors.append(ex)
 
-    threads = [threading.Thread(target=work, args=(m, d)) for m, d in zip(models, out_dirs)]
+    threads = [threading.Thread(target=work, args=(m, d, e)) for m, d, e in zip(models, out_dirs, env_out_dirs)]
     for t in threads:
         t.start()
     for t in threads:

@@ -112,6 +112,7 @@ def load_library(path: Optional[str] = None) -> C.CDLL:
     lib.sfl_run.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_void_p]
     lib.sfl_total_decisions.argtypes = [C.c_void_p, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64), C.c_void_p]
     lib.sfl_export_q.argtypes = [C.c_void_p, C.c_int, C.POINTER(C.c_uint32), C.POINTER(C.c_double), C.c_int, C.POINTER(C.c_int), C.c_void_p]
+    lib.sfl_export_q_batch.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p]
     lib.sfl_import_q.argtypes = [C.c_void_p, C.c_int, C.POINTER(C.c_uint32), C.POINTER(C.c_double), C.c_int, C.c_void_p]
     lib.sfl_set_eval_table.argtypes = [C.c_void_p, C.POINTER(C.c_uint32), C.POINTER(C.c_double), C.c_int, C.c_void_p]
     lib.sfl_shared_q_apply.argtypes = [C.c_void_p, C.c_void_p]
@@ -329,6 +330,44 @@ class RailMap:
             keys[idx] = ((((port0[s] + cur) * NT + tgt) * 16 + semb) * 3 + delay[rows, cur]).astype(np.uint32)
         return keys, vals
 
+    def q_dict(self, keys: np.ndarray, vals: np.ndarray, out: Optional[Dict[tuple, List[float]]] = None) -> Dict[tuple, List[float]]:
+        """The inverse of ``q_arrays``: (uint32[n] state keys, float64[n, >= A] values) as the reference's dict -- ``key_to_obs``
+        of every key with the first A values of its row -- computed per switch size with array operations.  The rows are
+        added to ``out`` (a new dict when None) in the order of ``keys``; ``out`` is returned."""
+        out = {} if out is None else out
+        n = len(keys)
+        if not n:
+            return out
+        t, tr = self.tab, self.trains
+        NT = len(tr.targets)
+        port, rem = np.divmod(np.asarray(keys, np.int64), NT * 48)
+        tgt, rem = np.divmod(rem, 48)
+        semb, level = np.divmod(rem, 3)
+        s = np.asarray(t.port_switch, np.int64)[port]
+        P, A = np.asarray(t.sw_P, np.int64)[s], np.asarray(t.sw_A, np.int64)[s]
+        cur = port - np.asarray(t.sw_port0, np.int64)[s]
+        cell = np.asarray(t.switch_cells, np.int64).reshape(-1, 2)[s]
+        tcell = np.asarray(tr.targets, np.int64)[tgt]
+        obs: List[tuple] = [()] * n
+        rows: List[List[float]] = [[]] * n
+        for p in np.unique(P).tolist():
+            idx = np.nonzero(P == p)[0]
+            r, c = np.arange(len(idx)), cur[idx]
+            o = np.full((len(idx), 2 + 4 * p), -1, np.int64)
+            o[:, :2] = cell[idx]
+            o[:, 2:2 + p] = (semb[idx, None] >> np.arange(p)) & 1
+            o[r, 2 + p + 2 * c] = tcell[idx] // t.W
+            o[r, 3 + p + 2 * c] = tcell[idx] % t.W
+            o[r, 2 + 3 * p + c] = level[idx]
+            for i, ob in zip(idx.tolist(), o.tolist()):
+                obs[i] = tuple(ob)
+        for a in np.unique(A).tolist():
+            idx = np.nonzero(A == a)[0]
+            for i, v in zip(idx.tolist(), np.asarray(vals)[idx, :a].tolist()):
+                rows[i] = v
+        out.update(zip(obs, rows))
+        return out
+
     def q_init_rows(self, default_q: float) -> Dict[tuple, List[float]]:
         """All rows __init_q_table creates (distr_q.py:81-181), as the reference's dict."""
         t, tr = self.tab, self.trains
@@ -347,6 +386,37 @@ class RailMap:
                         row[a] = float(tr.qinit_val[port, tgt])
                         out[self.key_to_obs(((port * NT + tgt) * 16 + semb) * 3 + level)] = row
         return out
+
+
+class QSnapshot:
+    """The packed Q rows of environments [lo, hi) on their way to the host (``Engine.compact_q``): environment lo + j's rows
+    are rows off[j] .. off[j + 1] - 1 of the staging buffers, in slot order."""
+
+    def __init__(self, rail_map: RailMap, lo: int, off: np.ndarray, q_rows: np.ndarray, a_max: int, host: dict, event):
+        self.map, self.lo, self.off, self.q_rows, self.a_max, self.host, self.event = rail_map, lo, off, q_rows, a_max, host, event
+
+    def wait(self):
+        """Wait for the copy, then check every table's row count against its q_rows."""
+        if self.event is not None:
+            self.event.synchronize()
+        found = self.host["found"][:len(self.q_rows)].numpy()
+        bad = np.nonzero(found != self.q_rows)[0]
+        if len(bad):
+            j = int(bad[0])
+            raise RuntimeError(f"env {self.lo + j}: its Q table holds {int(found[j])} rows but counts {int(self.q_rows[j])}: the table "
+                               f"is corrupted ({len(bad)} env(s) disagree)")
+
+    def rows(self, env: int):
+        """(uint32[n] state keys, float64[n, a_max] values) of environment ``env``: views of the staging buffers."""
+        a, b = int(self.off[env - self.lo]), int(self.off[env - self.lo + 1])
+        keys = self.host["keys"][a:b].numpy().view(np.uint32)
+        return keys, self.host["vals"][a * self.a_max:b * self.a_max].numpy().reshape(b - a, self.a_max)
+
+    def table(self, env: int, init: Optional[Dict[tuple, List[float]]] = None) -> Dict[tuple, List[float]]:
+        """Environment ``env``'s rows as the reference's dict, after a copy of ``init`` (the optimistic rows) when given:
+        what ``Engine.export_q`` returns."""
+        out = {k: list(v) for k, v in init.items()} if init else {}
+        return self.map.q_dict(*self.rows(env), out)
 
 
 class Engine:
@@ -405,6 +475,7 @@ class Engine:
         self.max_malfunction_events = 0                   # events of the longest generated schedule
         self._pinned = {}
         self._pinned_ev = {}
+        self._qc = {}                                     # device buffers of compact_q, grown as needed
         self.buf = {}
         self.reset_io_counters()
         if not bind:
@@ -793,6 +864,82 @@ class Engine:
             A = int(t.sw_A[t.port_switch[int(k) // (NT * 48)]])
             out[self.map.key_to_obs(int(k))] = [float(x) for x in v[:A]]
         return out
+
+    def compact_q(self, lo: int, hi: int, staging: Optional[dict] = None) -> "QSnapshot":
+        """Enqueue, on the current stream, the compaction of environments [lo, hi)'s tables into one packed buffer on the
+        device (``sfl_export_q_batch``) and its copy into host staging (pinned on a CUDA device); returns without waiting for
+        either.  The row counts are the tables' q_rows as the last launch reported them (``counters()``), so call it after a
+        run.  ``staging``: a dict of host buffers to copy into, reused and grown as needed (default: new ones); it must not
+        be reused before the returned snapshot has been read."""
+        lo, hi = int(lo), int(hi)
+        if not 0 <= lo <= hi <= self.n_envs:
+            raise ValueError(f"environments [{lo}, {hi}) are not a range of this engine's {self.n_envs}")
+        torch, a_max = self.torch, self.sizes.a_max
+        q_rows = self.counters()["q_rows"][lo:hi].astype(np.int64)
+        off = np.zeros(hi - lo + 1, np.int64)
+        np.cumsum(q_rows, out=off[1:])
+        total = int(off[-1])
+        need = {"off": (hi - lo + 1, torch.int64), "keys": (total, torch.int32), "vals": (total * a_max, torch.float64),
+                "found": (hi - lo, torch.int32)}
+        dev = self._qc
+        for name, (n, dt) in need.items():
+            if name not in dev or dev[name].numel() < n:
+                dev[name] = torch.empty(max(n, 1), dtype=dt, device=self.device)
+        dev["off"][:hi - lo + 1].copy_(torch.from_numpy(off))
+        ptr = lambda name: C.c_void_p(dev[name].data_ptr())
+        self._ck(self.lib.sfl_export_q_batch(self.ctx, lo, hi, ptr("off"), ptr("keys"), ptr("vals"), C.c_uint64(max(total, 1)),
+                                             ptr("found"), self._stream()))
+        pinned = self.device.type == "cuda"
+        host = {} if staging is None else staging
+        for name in ("keys", "vals", "found"):
+            n = need[name][0]
+            if name not in host or host[name].numel() < n:
+                host[name] = torch.empty(max(n, 1), dtype=need[name][1], pin_memory=pinned)
+            host[name][:n].copy_(dev[name][:n], non_blocking=pinned)
+            self.d2h_bytes += n * host[name].element_size()
+        event = None
+        if pinned:
+            event = torch.cuda.Event()
+            event.record(torch.cuda.current_stream(self.device))
+        return QSnapshot(self.map, lo, off, q_rows, a_max, host, event)
+
+    def export_q_batch(self, envs: Optional[Sequence[int]] = None, include_init: bool = False,
+                       default_q=None) -> List[Dict[tuple, List[float]]]:
+        """``export_q(i, include_init, default_q_i)`` of every environment i of ``envs`` (consecutive indices, default all):
+        the same dicts in the same insertion order, so that ``DistrQLearning.save`` writes the same bytes, from one
+        compaction of all their tables on the device and one copy to the host (``compact_q``).  ``default_q``: one value,
+        one per environment of ``envs``, or None (the hparams' default_q).  The optimistic rows are built once per distinct
+        default_q.  Shared-table mode: every environment gets the one table ``export_shared_q`` gives."""
+        return list(self.iter_q_batch(envs, include_init, default_q))
+
+    def iter_q_batch(self, envs: Optional[Sequence[int]] = None, include_init: bool = False, default_q=None):
+        """``export_q_batch`` one dict at a time: the compaction and the copy happen at once (they raise here, before the
+        first dict), and each environment's dict is built when the iteration reaches it."""
+        envs = list(range(self.n_envs) if envs is None else envs)
+        if envs and envs != list(range(envs[0], envs[0] + len(envs))):
+            raise ValueError("export_q_batch() takes consecutive environment indices")
+        if default_q is None:
+            dq = [float(self.hparams["default_q"][i]) for i in envs]
+        else:
+            dq = np.broadcast_to(np.asarray(default_q, np.float64), (len(envs),)).tolist()
+        if not envs:
+            return iter(())
+        if self.shared_q:
+            shared: Dict[float, Dict[tuple, List[float]]] = {}
+            for d in dq:
+                if d not in shared:
+                    shared[d] = self.export_shared_q(d)
+            return ({k: list(v) for k, v in shared[d].items()} for d in dq)
+        snap = self.compact_q(envs[0], envs[-1] + 1)
+        snap.wait()
+        init: Dict[float, Dict[tuple, List[float]]] = {}
+
+        def tables():
+            for i, d in zip(envs, dq):
+                if include_init and d not in init:
+                    init[d] = self.map.q_init_rows(d)
+                yield snap.table(i, init[d] if include_init else None)
+        return tables()
 
     def import_q(self, env: int, q: Dict[tuple, List[float]]):
         keys, vals = self.map.q_arrays(q, self.sizes.a_max)

@@ -124,11 +124,15 @@ def launch_grid(hyperparams: Dict[str, Sequence[float]], random_seeds: Sequence[
                                lr=col("lr", 0.4), lr_decay_rate=col("lr_decay_rate", 0.0), default_q=default_q,
                                seeds=np.full(len(points), seed, np.uint64))          # same seed for every point, as the reference
         runs.append((rdx, seed, model))
-    # hyperparam_tuning.py:85-91 starts every run at once; here the seeds of this rank learn concurrently, one stream each
-    learn_concurrently([m for _, _, m in runs], num_episodes, None, checkpoint_freq, exploit_freq)
+    exp_dirs = {rdx: [os.path.join(out_dir, f"exp_{idx}", f"seed_{rdx}") for idx in range(len(points))] for rdx, _, _ in runs}
+    # hyperparam_tuning.py:85-91 starts every run at once; here the seeds of this rank learn concurrently, one stream each.
+    # Every environment's checkpoints go to its exp_i/seed_j, where main.py writes them (distr_q.py:288-294).
+    learn_concurrently([m for _, _, m in runs], num_episodes, None, checkpoint_freq, exploit_freq,
+                       env_out_dirs=[exp_dirs[rdx] for rdx, _, _ in runs])
     for rdx, seed, model in runs:
-        for idx, params in enumerate(points):
-            exp_dir = os.path.join(out_dir, f"exp_{idx}", f"seed_{rdx}")
+        tables = model.env_q_tables()                # every environment's final table from one compaction, built one at a time
+        for (idx, params), q in zip(enumerate(points), tables):
+            exp_dir = exp_dirs[rdx][idx]
             os.makedirs(exp_dir, exist_ok=True)
             config = configparser.ConfigParser()
             config["MISC"] = {"random_seed": str(seed), "out_dir": exp_dir, "checkpoint_freq": str(checkpoint_freq),
@@ -142,7 +146,7 @@ def launch_grid(hyperparams: Dict[str, Sequence[float]], random_seeds: Sequence[
                                "num_episodes": str(num_episodes)}
             with open(os.path.join(exp_dir, "config.ini"), "w") as f:
                 config.write(f)
-            model.write_outputs(idx, exp_dir, exploit=exploit_freq is not None)
+            model.write_outputs(idx, exp_dir, exploit=exploit_freq is not None, q_table=q)
             written.append(exp_dir)
         model.env.engine.close()
     return written

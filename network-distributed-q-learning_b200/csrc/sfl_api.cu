@@ -133,6 +133,44 @@ SFL_FN void q_reinit_slot(const ReinitArgs &a, int env, int slot) {
   row[1 + (qi & 15)] = (qi & 16) ? 1000.0 : 500.0;
 }
 
+// Checkpoint export of many tables at once (sfl_export_q_batch): the occupied rows of environment env_lo + j go to rows
+// off[j] .. off[j + 1] - 1 of (keys, vals), in slot order -- the order sfl_export_q gives.  A group walks the table G slots
+// at a time: a ballot over the key words marks the occupied slots, and a row's place is the running count plus the popcount
+// of the ballot bits below its lane.  No atomics, so the output does not depend on scheduling.  Only key words are read to
+// find the rows; values are read for occupied rows only.  Rows past off[j + 1] or cap_rows are counted but not written, so
+// a table whose row count disagrees with its q_rows cannot write outside its range: found[j] reports it to the host.
+struct CompactArgs { Layout L; const char *state; const unsigned long long *off; uint32_t *keys; double *vals; int *found;
+                     unsigned long long cap_rows; int env_lo, n; };
+#define SFL_COMPACT_UNROLL 4                           // key loads in flight per lane
+template <int G> SFL_FN void q_compact_env(const CompactArgs &a, int j, const Grp<G> &g) {
+  const Layout &L = a.L;
+  const double *q = (const double *)(a.state + (size_t)(a.env_lo + j) * L.env_stride + L.off_q);
+  const unsigned long long row0 = a.off[j], end = a.off[j + 1] < a.cap_rows ? a.off[j + 1] : a.cap_rows;
+  const unsigned below = (1u << g.gl) - 1u;
+  unsigned long long n = 0;
+  SFL_NU
+  for (int base = 0; base < L.q_cap; base += G * SFL_COMPACT_UNROLL) {
+    unsigned long long k[SFL_COMPACT_UNROLL];
+    SFL_UA
+    for (int u = 0; u < SFL_COMPACT_UNROLL; u++) {
+      const int slot = base + u * G + g.gl;
+      k[u] = slot < L.q_cap ? *(const unsigned long long *)(q + (size_t)slot * L.q_stride) : 0ull;
+    }
+    SFL_UA
+    for (int u = 0; u < SFL_COMPACT_UNROLL; u++) {
+      const unsigned b = g.ballot(k[u] != 0ull);
+      const unsigned long long row = row0 + n + (unsigned)popc32(b & below);
+      if (k[u] && row < end) {
+        const double *src = q + (size_t)(base + u * G + g.gl) * L.q_stride + 1;
+        a.keys[row] = (uint32_t)(k[u] - 1ull);
+        for (int x = 0; x < L.a_max; x++) a.vals[row * (unsigned)L.a_max + x] = src[x];
+      }
+      n += (unsigned)popc32(b);
+    }
+  }
+  if (g.gl == 0) a.found[j] = (int)n;
+}
+
 // known-answer hooks of the reference's stream: the kernel's own PCG64 / SeedSequence / epsilon functions on caller operands
 SFL_FN void pcg_words(const Pcg &g, uint64_t *o) { o[0] = g.s_hi; o[1] = g.s_lo; o[2] = g.i_hi; o[3] = g.i_lo; o[4] = g.has32; o[5] = g.u32; }
 SFL_FN void kat_pcg64_one(const uint64_t *gen, const uint64_t *codes, int n_codes, uint64_t *out) {
@@ -191,6 +229,11 @@ __global__ void __launch_bounds__(256) k_q_reinit(const __grid_constant__ Reinit
   const size_t n = (size_t)a.n_envs * a.L.q_cap;
   for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x)
     q_reinit_slot(a, (int)(i / a.L.q_cap), (int)(i % a.L.q_cap));
+}
+
+// one warp per environment, one warp per CTA: a checkpoint of a few hundred learners still spreads over every SM
+__global__ void __launch_bounds__(32) k_q_compact(const __grid_constant__ CompactArgs a) {
+  if ((int)blockIdx.x < a.n) q_compact_env(a, (int)blockIdx.x, Grp<32>());
 }
 
 __global__ void __launch_bounds__(SFL_CTA_THREADS) k_init(const __grid_constant__ InitArgs ia) {
@@ -1061,6 +1104,35 @@ int sfl_export_q(void *ctx, int env, uint32_t *keys_host, double *vals_host, int
   }
   *n_rows = rows;
   return rows > cap_rows && keys_host ? fail(SFL_E_NOMEM, "export buffer too small%s") : SFL_OK;
+}
+
+int sfl_export_q_batch(void *ctx, int env_lo, int env_hi, const uint64_t *row_offsets, uint32_t *keys, double *vals, uint64_t cap_rows,
+                       int32_t *rows_found, void *stream) {
+  Ctx *c = (Ctx *)ctx;
+  if (!c || !c->bound) return fail(SFL_E_STATE, "sfl_bind first%s");
+  DeviceGuard dg(c->device);
+  if (c->cfg.eval_q) return fail(SFL_E_STATE, "an evaluation context (eval_q) keeps no per-environment tables%s");
+  if (env_lo < 0 || env_hi > c->cfg.n_envs || env_lo > env_hi) return fail(SFL_E_ARG, "bad environment range: need 0 <= env_lo <= env_hi <= n_envs%s");
+  if (!row_offsets || !keys || !vals || !rows_found) return fail(SFL_E_ARG, "null argument%s");
+  const int n = env_hi - env_lo;
+  uint64_t last = 0;
+  CK(d2h(&last, row_offsets + n, 8, stream));
+  if (last > cap_rows) {
+    char detail[96];
+    snprintf(detail, sizeof(detail), "%llu rows, cap_rows is %llu", (unsigned long long)last, (unsigned long long)cap_rows);
+    return fail(SFL_E_NOMEM, "the export buffers are smaller than the last row offset: %s", detail);
+  }
+  if (!n) return SFL_OK;
+  CompactArgs a;
+  a.L = c->L; a.state = (const char *)c->bufs.state; a.off = (const unsigned long long *)row_offsets; a.keys = keys; a.vals = vals;
+  a.found = rows_found; a.cap_rows = cap_rows; a.env_lo = env_lo; a.n = n;
+#ifndef SFL_HOST_EMUL
+  k_q_compact<<<n, 32, 0, (cudaStream_t)stream>>>(a);
+  CU(cudaGetLastError());
+#else
+  for (int j = 0; j < n; j++) q_compact_env(a, j, Grp<1>());
+#endif
+  return SFL_OK;
 }
 
 int sfl_import_q(void *ctx, int env, const uint32_t *keys_host, const double *vals_host, int n_rows, void *stream) {
